@@ -153,6 +153,33 @@ def pinned(n):
     return t, t.numpy()
 
 
+DUMP_SAMPLE = 1 << 21      # solution entries kept by --dump-outputs: with their indices 32 MB, inside the 64 MB the dump may take
+
+
+def dump_outputs(d, s, hist, corr, rel):
+    """--dump-outputs: what the last timed solve handed back, as d/<name>.npy (float64), so that two builds can be compared
+    output for output on the same inputs.  Synchronous solvers: the relative residual history; asynchronous ones: the
+    corrections per level and the final relative residual.  The solution whole when it has at most DUMP_SAMPLE entries, else
+    a fixed sample of it (seed 0, ascending rows) and the sampled row indices."""
+    os.makedirs(d, exist_ok=True)
+    out = {}
+    if hist is not None:
+        out["relres_history"] = np.asarray(hist, dtype=np.float64)
+    else:
+        out["corrections_per_level"] = np.asarray(corr, dtype=np.float64)
+        out["final_relres"] = np.asarray([rel], dtype=np.float64)
+    u = s.get_solution()
+    if u.size <= DUMP_SAMPLE:
+        out["solution"] = u
+    else:
+        rows = np.sort(np.random.default_rng(0).choice(u.size, DUMP_SAMPLE, replace=False))
+        out["solution_sample"] = u[rows]
+        out["solution_sample_rows"] = rows.astype(np.float64)
+    for name, a in out.items():
+        np.save(os.path.join(d, name + ".npy"), a)
+    log("[bench] outputs of the last timed step written to %s: %s" % (d, ", ".join("%s%s" % (k, v.shape) for k, v in out.items())))
+
+
 # ------------------------------------------------------------------------------------------------
 def run_b200(args):
     import torch
@@ -164,6 +191,8 @@ def run_b200(args):
     if not torch.cuda.is_available():
         raise SystemExit("bench.py: no CUDA device -- the B200 path has no CPU fallback")
     if world > 1:
+        if args.dump_outputs:
+            raise SystemExit("bench.py: --dump-outputs covers the single-GPU solve only")
         from async_multigrid_b200 import dist_bench
         if args.solver == "async_multadd":
             return dist_bench.run_async(args, rank, world, local)     # BASELINE.json configs[4]: asynchronous across GPUs
@@ -234,6 +263,8 @@ def run_b200(args):
     torch.cuda.synchronize()
     launches = s.launch_count() - launches0
     solve_s = float(np.mean(secs_list))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, s, hist, corr, rel)
 
     # end to end through the drop-in call with host buffers
     one_solve_e2e()
@@ -696,7 +727,14 @@ def main():
     ap.add_argument("--cpu-port", action="store_true", help="time the oracle port instead of oracle/_ref")
     ap.add_argument("--cpu-sample-cycles", type=int, default=3)
     ap.add_argument("--cpu-threads", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (residual history or correction counts, the "
+                         "solution or a fixed sample of it) to DIR/<name>.npy; single-GPU b200 arm only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm's timed solve")
     if args.warmup < 3 and args.impl == "b200":
         log("[bench] note: fewer than 3 warm-up steps requested")
     if args.impl == "reference":
