@@ -86,7 +86,11 @@ __device__ __forceinline__ void cta_slice_rows(const DevCSR &M, int slice_ctas, 
    else { *r0 = (int)u0; *r1 = (int)u1; }
 }
 
-template <bool HEAVY>
+// EXT: the instantiation of the asynchronous implicit extended-system solver (extended.cu): the AOP_EXT_* operations, a
+// per-CTA omega / loc_iters, and an L1 invalidation after the barrier of a one-CTA group too (its reads of other groups'
+// u_j / e_j must never be served by a line cached before the barrier).  HEAVY = false / EXT = false and HEAVY = true are the
+// asynchronous additive solver's instantiations; the EXT branches compile out of them.
+template <bool HEAVY, bool EXT = false>
 __global__ void __launch_bounds__(kABlock, HEAVY ? 3 : 6) k_async_amg(const AsyncParams *__restrict__ pp)
 {
    const AsyncParams &p = *pp;
@@ -111,6 +115,8 @@ __global__ void __launch_bounds__(kABlock, HEAVY ? 3 : 6) k_async_amg(const Asyn
    const unsigned long long t_begin = global_ns();
    int stop = 0;
    unsigned long long seq = 0;            // exchange steps of this group so far (row-partitioned solve)
+   double omega = 2.0;                    // EXT: the group's Chebyshev omega, advanced identically by every CTA of the group
+   int loc_iters = 1;                     // EXT: the group's loc_iters (every CTA keeps the same count)
 
    while (!stop) {
       for (int i = 0; i < nops; i++) {
@@ -120,15 +126,60 @@ __global__ void __launch_bounds__(kABlock, HEAVY ? 3 : 6) k_async_amg(const Asyn
          __syncthreads();
          const AsyncOp &op = sv.op;
          const int type = op.type;
-         if (type == AOP_SPMV) {
+         if (type == AOP_SPMV || (EXT && type == AOP_EXT_RESID)) {
             if (threadIdx.x == 0)
                make_view(sv, op.mat_kind == AMGB_MAT_A ? p.A[op.mat_level] : (op.mat_kind == AMGB_MAT_P ? p.P[op.mat_level] : (op.mat_kind == AMGB_MAT_R ? p.R[op.mat_level] : p.Ainv)), p.slice_ctas);
             __syncthreads();
             const DevCSR &M = sv.M;
             const int t0 = op.range ? (int)threadIdx.x : tm.tid, ts = op.range ? kABlock : tm.size;
-            if (M.sell_slices > 0 && M.su_desc) sell_rows_team<false, false, 4>(M, op.x, op.y, op.e, t0, ts, false);
-            else if (M.sell_slices > 0) sell_rows_team<false, false>(M, op.x, op.y, op.e, t0, ts, false);
-            else if (M.nrows > 0) csr_rows_dispatch<false, false>(M, op.x, op.y, op.e, t0, ts, false);
+            const bool ss = EXT && type == AOP_EXT_RESID;
+            double part = 0.0;
+            if (M.sell_slices > 0 && M.su_desc) part = sell_rows_team<false, false, 4>(M, op.x, op.y, op.e, t0, ts, ss);
+            else if (M.sell_slices > 0) part = sell_rows_team<false, false>(M, op.x, op.y, op.e, t0, ts, ss);
+            else if (M.nrows > 0) part = csr_rows_dispatch<false, false>(M, op.x, op.y, op.e, t0, ts, ss);
+            if (ss) {
+               part = block_sum(part);
+               if (threadIdx.x == 0) *((volatile double *)(p.ext.cta_ss + blockIdx.x)) = part;
+            }
+         } else if (EXT && type == AOP_EXT_CHEBY) {
+            // u_k <- y_k + omega (delta rs o r_k + u_k - y_k), y_k <- old u_k (k_cheby's arithmetic).  u_k is read by the other
+            // groups while this runs: stored through L2
+            const int n = p.A[op.level].nrows;
+            const double dl = p.ext.delta;
+            for (int k = tm.tid; k < n; k += tm.size) {
+               const double uo = ld_cg(op.y + k), yo = ld_cg(op.e.c + k);
+               const double s = __ldg(op.e.rs + k) * ld_cg(op.x + k);
+               st_cg(op.y + k, yo + omega * (dl * s + uo - yo));
+               st_cg(const_cast<double *>(op.e.c) + k, uo);
+            }
+            omega = 1.0 / (1.0 - omega / p.ext.mu22);
+         } else if (EXT && type == AOP_EXT_STOP) {
+            // the stop rule of SMEM_ExtendedSystemSolve's asynchronous branch (src/SMEM_ExtendedSystem.cpp:636-652); the previous
+            // operation's barrier made every CTA's residual slot visible
+            if (tm.tid == 0) {
+               double s = 0.0;
+               for (int t = p.cta_begin[q]; t < p.cta_begin[q + 1]; t++) s += *((volatile double *)(p.ext.cta_ss + t));
+               if (loc_iters > 1) p.ext.contrib[q] = s;         // check_resnorm_flag && loc_iters > 1, before the increment
+               __threadfence();
+               if (q == 0 && *p.converge_flag == 0) {           // the reference's thread 0: sum of the (possibly stale) contributions
+                  double tot = 0.0;
+                  for (int l = 0; l < L; l++) tot += p.ext.contrib[l];
+                  if (sqrt(tot) / p.ext.r0_ext < p.ext.tol) { *p.converge_flag = 1; __threadfence(); }
+               }
+               if (loc_iters + 1 == p.num_cycles) { atomicAdd(p.ext.done, 1); __threadfence(); }
+               const int st = *p.converge_flag != 0 || *((volatile int *)p.ext.done) >= L;
+               *((volatile int *)(p.group_stop + q)) = st;
+               if (tm.nctas == 1) s_stop = st;
+            }
+            loc_iters++;
+            // every CTA takes the group root's decision
+            if (tm.nctas > 1) {
+               group_barrier(tm);
+               if (threadIdx.x == 0) s_stop = *((volatile int *)(p.group_stop + q));
+            }
+            __syncthreads();
+            stop = s_stop;
+            __syncthreads();
          } else if (type == AOP_SCALE) {
             // y = rs o x (zero-guess Jacobi, src/SMEM_Smooth.cpp:381-389), optionally reduced into the shared u
             int r0 = 0, r1 = p.A[op.level].nrows, step = tm.size, first = tm.tid;
@@ -253,9 +304,15 @@ __global__ void __launch_bounds__(kABlock, HEAVY ? 3 : 6) k_async_amg(const Asyn
             async_gs_team<false>(p.A[op.level], op.x, op.y, p.jgs_block_rows, op.sweeps, tm.tid, tm.size);
          }
          if (op.barrier && type != AOP_WAIT) group_barrier(tm);
+         if (EXT && op.barrier && tm.nctas == 1) {
+            // (a one-CTA group's barrier has no fence of its own: drop what this SM's L1 holds of the other groups' vectors)
+            if (threadIdx.x == 0) __threadfence();
+            __syncthreads();
+         }
       }
    }
    if (tm.tid == 0) p.group_ns[q] = global_ns() - t_begin;
+   if (EXT && tm.tid == 0) p.ext.loc_iters[q] = loc_iters;
 }
 
 constexpr size_t kHeavySmem = (size_t)(kABlock / 4) * AMGB_JGS_BMAX * sizeof(double);
@@ -292,6 +349,38 @@ int launch_async(cudaStream_t st, const AsyncParams *params_dev, int grid, int b
    cfg.attrs = attrs;
    cfg.numAttrs = na;
    cudaError_t e = heavy ? cudaLaunchKernelEx(&cfg, k_async_amg<true>, params_dev) : cudaLaunchKernelEx(&cfg, k_async_amg<false>, params_dev);
+   return e == cudaSuccess ? 1 : -(int)e;
+}
+
+int async_max_grid_ext(int block)
+{
+   int dev = 0, sms = 0, per_sm = 0;
+   cudaGetDevice(&dev);
+   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+   cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_async_amg<false, true>, block, 0);
+   return sms * per_sm;
+}
+
+int launch_async_ext(cudaStream_t st, const AsyncParams *params_dev, int grid, int block, const cudaAccessPolicyWindow *window)
+{
+   cudaLaunchConfig_t cfg = {};
+   cfg.gridDim = dim3(grid);
+   cfg.blockDim = dim3(block);
+   cfg.dynamicSmemBytes = 0;
+   cfg.stream = st;
+   cudaLaunchAttribute attrs[2];
+   int na = 0;
+   attrs[na].id = cudaLaunchAttributeCooperative;
+   attrs[na].val.cooperative = 1;
+   na++;
+   if (window && window->num_bytes > 0) {
+      attrs[na].id = cudaLaunchAttributeAccessPolicyWindow;
+      attrs[na].val.accessPolicyWindow = *window;
+      na++;
+   }
+   cfg.attrs = attrs;
+   cfg.numAttrs = na;
+   const cudaError_t e = cudaLaunchKernelEx(&cfg, k_async_amg<false, true>, params_dev);
    return e == cudaSuccess ? 1 : -(int)e;
 }
 
@@ -485,6 +574,46 @@ int async_build_program(const amgb_options &o, int L, bool symmetric, bool fact0
    return AMGB_OK;
 }
 
+// The program of group q of the asynchronous implicit extended-system solver (SMEM_ExtendedSystemSolve with
+// IMPLICIT_EXTENDED_SYSTEM_BPX and async_flag = 1, src/SMEM_ExtendedSystem.cpp:305,365,474-479,636-652): the reference's thread
+// group of level q rebuilds both chains it needs from whatever the other groups have written so far --
+//   z1_{L-1} = u_{L-1},  z1_j = P_j z1_{j+1} + u_j  (j = L-2 .. q);   z2_0 = 0,  z2_{j+1} = R_j (z2_j + e_j)  (j = 0 .. q-1)
+//   r_q = f_q - z2_q - A_q z1_q;  u_q <- y_q + omega (delta rs o r_q + u_q - y_q), y_q <- old u_q;  e_q = A_q u_q;  count / stop
+// It writes u_q, y_q, e_q and its own chain vectors only; it reads u_j (j >= q) and e_j (j < q).
+int async_build_ext_program(const amgb_options &o, int L, int q, std::vector<AsyncOpSym> &ops)
+{
+   if (o.smoother != AMGB_SMOOTH_JACOBI && o.smoother != AMGB_SMOOTH_L1_JACOBI) return AMGB_EINVAL;
+   if (L < 1 || L > AMGB_MAX_LEVELS || q < 0 || q >= L) return AMGB_EINVAL;
+   ProgBuilder B{o, L, true, false, ops};
+   // ---- prolongation chain; the last one needs no barrier of its own when the restriction chain follows (it does not read z1)
+   int z1 = AV_ID(AV_XU, L - 1);
+   for (int j = L - 2; j >= q; j--) {
+      B.spmv(AMGB_MAT_P, j, 0, z1, AV_ID(AV_XZ1, j), 1.0, 1.0, AV_ID(AV_XU, j)).barrier = (j == q && q > 0) ? 0 : 1;
+      z1 = AV_ID(AV_XZ1, j);
+   }
+   // ---- restriction chain: on the levels it passes, the SpMV's epilogue adds e_{j+1} (z2_{j+1} alone is never read there)
+   int z2 = AV_ID(AV_XE, 0);
+   for (int j = 0; j < q; j++) {
+      const bool last = j + 1 == q;
+      B.spmv(AMGB_MAT_R, j, 0, z2, AV_ID(AV_XZ2, j + 1), 1.0, last ? 0.0 : 1.0, last ? AV_NONE : AV_ID(AV_XE, j + 1));
+      z2 = AV_ID(AV_XZ2, j + 1);
+   }
+   // ---- residual and its sum of squares, Chebyshev update, e_q (no group reads e_{L-1})
+   {
+      AsyncOpSym &r = B.spmv(AMGB_MAT_A, q, 0, z1, AV_ID(AV_XR, q), -1.0, 1.0, AV_ID(AV_XF, q));
+      r.type = AOP_EXT_RESID;
+      if (q > 0) { r.b2 = z2; r.beta2 = -1.0; }
+   }
+   {
+      AsyncOpSym &c = B.vec(AOP_EXT_CHEBY, q, AV_ID(AV_XR, q), AV_ID(AV_XU, q));
+      c.c = AV_ID(AV_XY, q);
+      c.rs = B.rs_id(q);
+   }
+   if (q < L - 1) B.spmv(AMGB_MAT_A, q, 0, AV_ID(AV_XU, q), AV_ID(AV_XE, q), 1.0, 0.0, AV_NONE);
+   B.vec(AOP_EXT_STOP, q, AV_NONE, AV_NONE).barrier = 0;      // (it ends with the group's decision, a barrier of its own)
+   return AMGB_OK;
+}
+
 // ---- host side: build the parameter block once, run ---------------------------------------------
 static bool async_heavy(const amgb_options &o)
 {
@@ -660,6 +789,14 @@ void async_assign_groups(amgb_ctx *c, const std::vector<double> &work)
 {
    AsyncParams &hp = *c->async_host;
    const int L = c->L, first = c->async_first, grid = c->async_grid;
+   async_deal_ctas(work, L, first, grid, hp.cta_begin);
+   hp.slice_ctas = std::max(1, L > 1 ? hp.cta_begin[L - 1] : hp.cta_begin[L]);      // CTAs of the working groups
+   c->async_cta_begin.assign(hp.cta_begin, hp.cta_begin + L + 1);
+   c->async_grid_used = hp.cta_begin[L];
+}
+
+void async_deal_ctas(const std::vector<double> &work, int L, int first, int grid, int *cta_begin)
+{
    double tot = 0.0;
    for (int q = first; q < L; q++) tot += work[q];
    std::vector<int> ctas(L, 0);
@@ -687,11 +824,8 @@ void async_assign_groups(amgb_ctx *c, const std::vector<double> &work)
          ctas[best]++; left--;
       }
    }
-   for (int q = 0; q <= first; q++) hp.cta_begin[q] = 0;
-   for (int q = first; q < L; q++) hp.cta_begin[q + 1] = hp.cta_begin[q] + ctas[q];
-   hp.slice_ctas = std::max(1, L > 1 ? hp.cta_begin[L - 1] : hp.cta_begin[L]);      // CTAs of the working groups
-   c->async_cta_begin.assign(hp.cta_begin, hp.cta_begin + L + 1);
-   c->async_grid_used = hp.cta_begin[L];
+   for (int q = 0; q <= first; q++) cta_begin[q] = 0;
+   for (int q = first; q < L; q++) cta_begin[q + 1] = cta_begin[q] + ctas[q];
 }
 
 void amgb_async_teardown(amgb_ctx *c)
@@ -834,6 +968,22 @@ extern "C" int amgb_async_program(const amgb_options *o, int num_levels, int sym
       op_begin[q] = (int)sym.size();
       if (q < first) continue;
       int rc = async_build_program(*o, num_levels, symmetric != 0, fact0 != 0, q, sym);
+      if (rc) return rc;
+   }
+   op_begin[num_levels] = (int)sym.size();
+   if ((int)sym.size() > max_ops) return AMGB_ENOMEM;
+   memcpy(ops, sym.data(), sizeof(AsyncOpSym) * sym.size());
+   return AMGB_OK;
+}
+
+// Host-only probe: the programs of amgb_solve_extended_implicit_async for these options and this number of levels.
+extern "C" int amgb_ext_async_program(const amgb_options *o, int num_levels, void *ops, int max_ops, int *op_begin)
+{
+   if (!o || !ops || !op_begin || num_levels < 1 || num_levels > AMGB_MAX_LEVELS) return AMGB_EINVAL;
+   std::vector<AsyncOpSym> sym;
+   for (int q = 0; q < num_levels; q++) {
+      op_begin[q] = (int)sym.size();
+      const int rc = async_build_ext_program(*o, num_levels, q, sym);
       if (rc) return rc;
    }
    op_begin[num_levels] = (int)sym.size();

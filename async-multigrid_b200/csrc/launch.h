@@ -79,11 +79,19 @@ enum { AOP_SPMV = 0, AOP_SCALE = 1, AOP_COPY = 2, AOP_ZERO = 3, AOP_UPDATE = 4, 
        AOP_JGS = 8, AOP_ASYNC_GS = 9,
        // row-partitioned solve (dist_async.cu): PUSH = boundary / owned entries of a vector into a peer GPU's ghost slots;
        // SIGNAL = "this group's stores of exchange step s are in place" into a peer's flag word; WAIT = until a peer's flag says s
-       AOP_PUSH = 10, AOP_SIGNAL = 11, AOP_WAIT = 12 };
+       AOP_PUSH = 10, AOP_SIGNAL = 11, AOP_WAIT = 12,
+       // asynchronous implicit extended-system BPX (extended.cu; the EXT instantiation of the kernel only):
+       // EXT_RESID = an SpMV like AOP_SPMV whose rows' sum of squares goes into this CTA's slot AsyncExtParams::cta_ss;
+       // EXT_CHEBY = y <- c + omega (delta rs o x + y - c), c <- old y over level `level` (x = r_k, y = u_k, c = y_k), then
+       //             omega <- 1 / (1 - omega / (2 mu)^2) in every CTA of the group; EXT_STOP = the group's count / stop rule
+       AOP_EXT_RESID = 13, AOP_EXT_CHEBY = 14, AOP_EXT_STOP = 15 };
 // vectors a program names: id = kind * 64 + level (group-private unless said otherwise)
 enum { AV_NONE = -1, AV_F = 0 /* shared f */, AV_U = 1 /* shared u */, AV_RS = 2 /* shared residual (GLOBAL / READ_RES) */,
        AV_R = 3, AV_E = 4, AV_T = 5, AV_W = 6, AV_UL = 7 /* private copy of u */, AV_T0 = 8 /* level-0 scratch */,
-       AV_FACC = 9 /* accumulated corrections (READ_RES) */, AV_WS = 10 /* w/d (read-only) */, AV_INVL1 = 11 /* 1/l1 (read-only) */ };
+       AV_FACC = 9 /* accumulated corrections (READ_RES) */, AV_WS = 10 /* w/d (read-only) */, AV_INVL1 = 11 /* 1/l1 (read-only) */,
+       // extended-system programs: the shared per-level vectors f_l, u_l, y_l, e_l (ExtState), and the group-private chain
+       // vectors z1_l (prolongation chain), z2_l (restriction chain; z2_l + e_l on the levels the chain passes) and r_l
+       AV_XF = 12, AV_XU = 13, AV_XY = 14, AV_XE = 15, AV_XZ1 = 16, AV_XZ2 = 17, AV_XR = 18 };
 #define AV_ID(kind, level) ((kind) * 64 + (level))
 #define AMAT_AINV 3                // AsyncOp::mat_kind beside AMGB_MAT_A / P / R: the dense inverse of the coarsest operator (coarse_solve)
 struct AsyncOpSym {                // one operation, symbolic (what the CPU tests interpret)
@@ -130,12 +138,29 @@ struct AsyncParams {
    volatile int *converge_flag;             // thread.converge_flag
    int *lock;                               // SEMI_ASYNC: the omp lock around "u += e; u_k = u"
    unsigned long long *group_ns;            // [L] nanoseconds every group spent in the kernel (CTA-group balancing)
+   // asynchronous implicit extended-system BPX only (the EXT instantiation reads these; the others never do)
+   struct AsyncExtParams {
+      double delta, mu22;                   // Chebyshev: delta, (2 mu)^2
+      double tol, r0_ext;                   // stop when sqrt(sum of the published contributions) / r0_ext < tol
+      double *cta_ss;                       // [grid] sum of r^2 over this CTA's rows of its group's last residual
+      volatile double *contrib;             // [L] published sum r_k^2 of every group (1e300 = not measured yet)
+      int *loc_iters;                       // [L] every group's loc_iters at exit
+      int *done;                            // groups whose loc_iters reached num_cycles
+   } ext;
 };
 // heavy: the instantiation that carries the Gauss-Seidel-type smoothers (more registers, fewer CTAs per SM)
 int launch_async(cudaStream_t st, const AsyncParams *params_dev, int grid, int block, bool heavy, const cudaAccessPolicyWindow *window);
 int async_max_grid(int block, bool heavy);
+// the instantiation that carries the extended-system operations (AOP_EXT_*)
+int launch_async_ext(cudaStream_t st, const AsyncParams *params_dev, int grid, int block, const cudaAccessPolicyWindow *window);
+int async_max_grid_ext(int block);
 // host-only: the program of group q (appended to `ops`); returns AMGB_OK or AMGB_EINVAL for an unsupported combination
 int async_build_program(const amgb_options &o, int L, bool symmetric, bool fact0, int q, std::vector<AsyncOpSym> &ops, bool partitioned = false);
+// host-only: the program of group q of the asynchronous implicit extended-system solver (appended to `ops`); AMGB_EINVAL for
+// smoothers other than weighted / L1 Jacobi
+int async_build_ext_program(const amgb_options &o, int L, int q, std::vector<AsyncOpSym> &ops);
+// CTA groups in proportion to `work` (at least one CTA per group from `first` on): cta_begin[L + 1]
+void async_deal_ctas(const std::vector<double> &work, int L, int first, int grid, int *cta_begin);
 
 // ---- row-partitioned asynchronous solve (dist_async.cu): the same programs on every GPU's row blocks, with AOP_PUSH
 // operations after every operation whose result a later SpMV reads with ghosts.  Pure host planning, shared by the device

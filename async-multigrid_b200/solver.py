@@ -26,6 +26,7 @@ ABI_SYMBOLS = [
     "amgb_spgemv", "amgb_spgemv_transpose", "amgb_smooth", "amgb_set_jgs_blocks", "amgb_norm2", "amgb_cycle", "amgb_eigs_power", "amgb_solve_sync", "amgb_solve_async",
     "amgb_async_groups", "amgb_solve_extended", "amgb_solve_extended_async", "amgb_smooth_transfer", "amgb_host_csr_free", "amgb_smem_solve", "amgb_time_residual", "amgb_level_storage", "amgb_time_spmv", "amgb_stream_stats", "amgb_l2_arena_bytes", "amgb_sellu_stats",
     "amgb_sellu_encode_host", "amgb_host_free", "amgb_async_program", "amgb_async_group_times",
+    "amgb_solve_extended_implicit_async", "amgb_ext_async_program",
     "amgb_dist_unique_id", "amgb_dist_init", "amgb_dist_set_level", "amgb_dist_setup", "amgb_dist_set_rhs",
     "amgb_dist_get_solution", "amgb_dist_solve_sync", "amgb_dist_solve_sync_accel", "amgb_dist_stats", "amgb_dist_eigs_power",
     "amgb_dist_solve_async", "amgb_dist_async_groups", "amgb_dist_async_plan",
@@ -89,6 +90,8 @@ def load_library():
     L.amgb_solve_async.argtypes = [C.c_void_p, C.c_int, C.c_int, IP, DP, DP]
     L.amgb_solve_extended.argtypes = [C.c_void_p, C.c_double, C.c_int, C.c_double, C.c_double, DP, IP, DP, DP, DP]
     L.amgb_solve_extended_async.argtypes = [C.c_void_p, C.c_double, C.c_int, C.c_double, C.c_double, IP, IP, DP, DP]
+    L.amgb_solve_extended_implicit_async.argtypes = [C.c_void_p, C.c_double, C.c_int, C.c_double, C.c_double, IP, DP, DP, DP, DP]
+    L.amgb_ext_async_program.argtypes = [C.POINTER(Options), C.c_int, C.c_void_p, C.c_int, IP]
     L.amgb_smooth_transfer.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_int, IP, IP, DP, C.c_int, IP, IP, DP,
                                        C.POINTER(HostCSR), C.POINTER(HostCSR)]
     L.amgb_host_csr_free.argtypes = [C.POINTER(HostCSR)]
@@ -290,6 +293,18 @@ class Solver:
         return dict(x=self.get_solution(), iters=it.value, ext_hist=hist[:it.value], ext_relres=er.value, relres=rr.value,
                     seconds=secs.value)
 
+    def SMEM_ExtendedSystemSolve_async(self, f, tol=1e-9, num_cycles=100, mu=1.0, delta=1.0):
+        """`-solver async_iebpx` (amgb_solve_extended_implicit_async): the implicit form with every level's group iterating
+        asynchronously in one persistent kernel.  -> dict(x, iters (every group's loc_iters), ext_relres, relres,
+        group_seconds, seconds)"""
+        self.set_rhs(f)
+        it = np.zeros(self.h.num_levels, dtype=np.int32)
+        gs = np.zeros(self.h.num_levels)
+        er, rr, secs = C.c_double(0), C.c_double(0), C.c_double(0)
+        self._ck(self.L.amgb_solve_extended_implicit_async(self.ctx, tol, int(num_cycles), mu, delta, _ip(it), C.byref(er), C.byref(rr),
+                                                           _dp(gs), C.byref(secs)))
+        return dict(x=self.get_solution(), iters=it, ext_relres=er.value, relres=rr.value, group_seconds=gs, seconds=secs.value)
+
     def ChebySetup(self, iters=20):
         """EigsPower + ChebySetup (src/SMEM_Cheby.cpp:28-60,410-518): returns (mu, delta, alpha, beta)"""
         a, b = C.c_double(0), C.c_double(0)
@@ -420,6 +435,22 @@ def async_program(num_levels, solver, smoother=H.JACOBI, symmetric=True, factor_
     rc = L.amgb_async_program(C.byref(o), num_levels, int(symmetric), int(factor_level0), ops, 4096, _ip(ob))
     if rc != 0:
         raise AmgError("amgb_async_program failed (%d): unsupported combination of asynchronous options" % rc)
+    return [[ops[i] for i in range(ob[q], ob[q + 1])] for q in range(num_levels)]
+
+
+def ext_async_program(num_levels, smoother=H.JACOBI):
+    """the programs of the asynchronous implicit extended-system solver (amgb_ext_async_program; host-only, no GPU needed):
+    list over the level groups of lists of AsyncOpSym"""
+    L = load_library()
+    o = Options()
+    L.amgb_default_options(C.byref(o))
+    o.solver, o.smoother = H.IMPLICIT_EXTENDED_SYSTEM_BPX, smoother
+    ops = (AsyncOpSym * 4096)()
+    ob = np.zeros(max(num_levels, 0) + 1, dtype=np.int32)
+    rc = L.amgb_ext_async_program(C.byref(o), num_levels, ops, 4096, _ip(ob))
+    if rc != 0:
+        raise AmgError("amgb_ext_async_program failed (%d): the asynchronous extended-system solver runs with weighted or L1 "
+                       "Jacobi on at most 32 levels" % rc)
     return [[ops[i] for i in range(ob[q], ob[q + 1])] for q in range(num_levels)]
 
 

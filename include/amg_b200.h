@@ -191,6 +191,26 @@ int amgb_solve_extended(amgb_ctx *ctx, double tol, int num_cycles, double mu, do
 int amgb_solve_extended_async(amgb_ctx *ctx, double tol, int num_cycles, double mu, double delta, int *iters_min, int *iters_max,
                               double *ext_relres, double *solve_seconds);
 
+/* The IMPLICIT form run ASYNCHRONOUSLY (`-solver async_iebpx`: SMEM_ExtendedSystemSolve with IMPLICIT_EXTENDED_SYSTEM_BPX and
+ * async_flag = 1, src/SMEM_Main.cpp:309, async branches of src/SMEM_ExtendedSystem.cpp:305,365,474-479,636-652) on the resident
+ * f, hierarchy as for amgb_solve_extended (solver BPX or IEBPX, weighted or L1 Jacobi, one GPU).  Set-up and finish are those
+ * of amgb_solve_extended; in between, one launch of the persistent kernel in which every level k owns a CTA group (the
+ * reference's thread group of level k) that rebuilds the z1 / z2 chains from the other groups' latest u_j (j >= k) and
+ * e_j (j < k), forms r_k, takes its own Chebyshev step (its own omega recurrence from 2) and refreshes e_k, with no barrier
+ * between groups.  Stop rule (:636-652): no iteration at all for num_cycles <= 1; a group publishes its sum r_k^2 from its
+ * second iteration on; group 0 raises the converge flag once the sum of the published (possibly stale) contributions is below
+ * tol * r0_ext; a group whose loc_iters reaches num_cycles counts itself done, and groups keep iterating until the flag is up
+ * or every group is done.  iters[num_levels] = every group's final loc_iters; ext_relres / relres = final relative residuals
+ * of the extended system and of A x = f; group_seconds[num_levels] (may be NULL) = time every group spent in the launch; the
+ * solution x = sum_l P^{0<-l} u_l is left in u (amgb_get_solution).  AMGB_EINVAL, before any launch, on a distributed
+ * context, for other smoothers or solvers, and when one cooperative wave holds fewer CTAs than levels. */
+int amgb_solve_extended_implicit_async(amgb_ctx *ctx, double tol, int num_cycles, double mu, double delta, int *iters,
+                                       double *ext_relres, double *relres, double *group_seconds, double *solve_seconds);
+/* Host-only (no CUDA call): the per-group programs amgb_solve_extended_implicit_async hands the persistent kernel for these
+ * options on num_levels levels (csrc/launch.h AsyncOpSym records; ops: caller's array of max_ops; op_begin[num_levels + 1]).
+ * AMGB_EINVAL for smoothers other than weighted / L1 Jacobi and for more than 32 levels. */
+int amgb_ext_async_program(const amgb_options *opt, int num_levels, void *ops, int max_ops, int *op_begin);
+
 /* Drop-in for one whole SMEM_Solve call with HOST buffers (what SMEM_Main's run loop would call,
  * src/SMEM_Main.cpp:694-757): uploads f, zeroes u (InitSolve), runs the sync or async solve named
  * by opt.solver, downloads u. */

@@ -1,5 +1,6 @@
 """Times the implicit extended-system BPX solver (amgb_solve_extended) next to Chebyshev-accelerated BPX (amgb_solve_sync)
-on the same hierarchy and bounds:  python tools/iebpx_time.py --n 128"""
+on the same hierarchy and bounds:  python tools/iebpx_time.py --n 128
+--async adds the asynchronous implicit form (amgb_solve_extended_implicit_async) on the same hierarchy and bounds."""
 import argparse
 import json
 import os
@@ -18,6 +19,8 @@ def main():
     ap.add_argument("--eig-iters", type=int, default=60, help="power-iteration steps (the reference's default 20 underestimates "
                     "the largest eigenvalue at 128^3 and the Chebyshev iteration then diverges -- in the reference's own loop too)")
     ap.add_argument("--eig-inflate", type=float, default=1.1, help="safety factor on the largest eigenvalue estimate")
+    ap.add_argument("--async", dest="run_async", action="store_true", help="also time the asynchronous implicit form")
+    ap.add_argument("--async-cap", type=int, default=20000, help="num_cycles of the asynchronous form")
     a = ap.parse_args()
     t0 = time.time()
     A = H.laplacian("7pt", a.n)
@@ -40,10 +43,17 @@ def main():
         s.set_solution(None)
         hist, secs = s.solve_sync(1e-9, 1000, cheby=(mu, delta))
         bpx = dict(cycles=len(hist) - 1, seconds=secs, relres=float(hist[-1]))
-    print(json.dumps({"n": a.n, "rows": h.n, "levels": h.num_levels, "host_setup_s": round(setup_s, 1), "eig": [lo, hi],
-                      "iebpx": {"iters": out["iters"], "seconds": out["seconds"], "ms_per_iter": 1e3 * out["seconds"] / max(out["iters"] - 1, 1),
-                                "ext_relres": out["ext_relres"], "relres": out["relres"], "launches": launches},
-                      "bpx_cheby": bpx}))
+    res = {"n": a.n, "rows": h.n, "levels": h.num_levels, "host_setup_s": round(setup_s, 1), "eig": [lo, hi],
+           "iebpx": {"iters": out["iters"], "seconds": out["seconds"], "ms_per_iter": 1e3 * out["seconds"] / max(out["iters"] - 1, 1),
+                     "ext_relres": out["ext_relres"], "relres": out["relres"], "launches": launches},
+           "bpx_cheby": bpx}
+    if a.run_async:
+        runs = [s.SMEM_ExtendedSystemSolve_async(b, 1e-9, a.async_cap, mu, delta) for _ in range(3)]
+        ao = runs[-1]
+        res["async_iebpx"] = {"seconds": ao["seconds"], "iters": [int(k) for k in ao["iters"]],
+                              "group_seconds": [float(t) for t in ao["group_seconds"]], "ext_relres": ao["ext_relres"],
+                              "relres": ao["relres"], "seconds_all_runs": [r["seconds"] for r in runs]}
+    print(json.dumps(res))
     s.close()
 
 
