@@ -153,6 +153,7 @@ int amgb_destroy(amgb_ctx *c)
    for (double *p : c->peer_u) cudaIpcCloseMemHandle(p);
    amgb_async_teardown(c);
    amgb_ext_teardown(c);
+   amgb_pcg_teardown(c);
    if (c->graph_exec) cudaGraphExecDestroy(c->graph_exec);
    for (void *p : c->allocs) cudaFree(p);
    if (c->h_scalars) cudaFreeHost(c->h_scalars);
@@ -845,6 +846,24 @@ void enq_spmv(amgb_ctx *c, const DevCSR &M, bool sval, const double *x, double *
    if (norm) c->launches += launch_reduce_partials(c->stream, c->partials, grid, c->d_scalars);
 }
 
+// the same with the fused sum_i y_i w_i reduced into *dot_out (w == nullptr: plain enq_spmv, no reduction)
+void enq_spmv_dot(amgb_ctx *c, const DevCSR &M, bool sval, const double *x, double *y, const SpmvEpilogue &e, const double *w, double *dot_out)
+{
+   if (!w) { enq_spmv(c, M, sval, x, y, e, false); return; }
+   int grid = 0;
+   c->launches += launch_spmv(c->cfg, c->stream, M, sval, x, y, e, c->partials, &grid, w);
+   c->launches += launch_reduce_partials(c->stream, c->partials, grid, dot_out);
+}
+
+// *out = sum_i x_i w_i (nothing when w == nullptr)
+static void enq_dot(amgb_ctx *c, int n, const double *x, const double *w, double *out)
+{
+   if (!w) return;
+   int grid = 0;
+   c->launches += launch_dot(c->cfg, c->stream, n, x, w, c->partials, &grid);
+   c->launches += launch_reduce_partials(c->stream, c->partials, grid, out);
+}
+
 // r0 = f - A0 u, d_scalars[0] = ||r||^2     (SMEM_Sync_Residual + norm, src/SMEM_Solve.cpp:192-203)
 void enq_residual(amgb_ctx *c)
 {
@@ -909,8 +928,10 @@ void enq_smooth_zero(amgb_ctx *c, int l, const double *f, double *e, int sweeps,
    (void)s2;
 }
 
-// One additive cycle on residual r[0]:  target = gamma*target + B r.
-void enq_cycle(amgb_ctx *c, double *target, bool accumulate)
+// One additive cycle on residual r[0]:  target = gamma*target + B r.  r[0] is read and never written (the factorised level-0
+// path included): the preconditioned conjugate-gradient solve (pcg.cu) keeps its residual there across the cycle.
+// dot_w != nullptr: sum_i target_i dot_w_i is reduced into *dot_out, fused into the cycle's last launch when that is an SpMV.
+void enq_cycle(amgb_ctx *c, double *target, bool accumulate, const double *dot_w, double *dot_out)
 {
    const int L = c->L;
    const amgb_options &o = c->opt;
@@ -926,6 +947,7 @@ void enq_cycle(amgb_ctx *c, double *target, bool accumulate)
          if (accumulate) c->launches += launch_add(c->cfg, c->stream, n0, c->e[0], target);
          else cudaMemcpyAsync(target, c->e[0], sizeof(double) * n0, cudaMemcpyDeviceToDevice, c->stream);
       } else if (!accumulate) cudaMemsetAsync(target, 0, sizeof(double) * n0, c->stream);
+      enq_dot(c, n0, target, dot_w, dot_out);
       return;
    }
    // restriction chain, shared by all levels (the reference repeats it per level group,
@@ -971,13 +993,14 @@ void enq_cycle(amgb_ctx *c, double *target, bool accumulate)
       SpmvEpilogue fe = epi(-1.0, 1.0, c->r[0], 1.0, accumulate ? target : nullptr, rs0);
       fe.b2 = c->t[0]; fe.beta2 = 1.0;
       fe.xs = c->w[0]; fe.xself = 1.0;
-      enq_spmv(c, c->A[0], false, c->w[0], target, fe, false);
+      enq_spmv_dot(c, c->A[0], false, c->w[0], target, fe, dot_w, dot_out);
    } else if (top >= 2) {
       // target = [target +] e_0 + P_0 e_1   (u += e fused into the last prolongation)
-      enq_spmv(c, c->P[0], false, c->e[1], target, epi(1.0, 1.0, c->e[0], 1.0, accumulate ? target : nullptr), false);
+      enq_spmv_dot(c, c->P[0], false, c->e[1], target, epi(1.0, 1.0, c->e[0], 1.0, accumulate ? target : nullptr), dot_w, dot_out);
    } else {
       if (accumulate) c->launches += launch_add(c->cfg, c->stream, n0, c->e[0], target);
       else cudaMemcpyAsync(target, c->e[0], sizeof(double) * n0, cudaMemcpyDeviceToDevice, c->stream);
+      enq_dot(c, n0, target, dot_w, dot_out);
    }
 }
 
@@ -1059,6 +1082,7 @@ int amgb_set_jgs_blocks(amgb_ctx *c, int level, int nblocks, const int *bounds)
    c->jgs_bounds[level] = dev;
    c->jgs_nb[level] = nblocks;
    if (c->graph_exec) { cudaGraphExecDestroy(c->graph_exec); c->graph_exec = nullptr; }     // the captured cycle held the old launches
+   if (c->pcg_graph) { cudaGraphExecDestroy(c->pcg_graph); c->pcg_graph = nullptr; }
    return AMGB_OK;
 }
 

@@ -38,6 +38,10 @@ struct amgb_ctx {
    double r0_norm = 0.0;
    cudaGraphExec_t graph_exec = nullptr;
    long long graph_kernels = 0;
+   // preconditioned conjugate gradients (pcg.cu): direction p, A p, the device scalars (PCG_* slots), one iteration's graph
+   double *pcg_p = nullptr, *pcg_q = nullptr, *pcg_s = nullptr;
+   cudaGraphExec_t pcg_graph = nullptr;
+   long long pcg_graph_kernels = 0;
    long long launches = 0;
    size_t bytes_allocated = 0;
    int host_threads = 1;   // threads for the upload-time layout conversions (set in amgb_create)
@@ -76,6 +80,7 @@ int amgb_fail(amgb_ctx *c, int code, const char *fmt, ...);
 bool amgb_dist_owned_cols(const amgb_ctx *c, int kind, int level, int *c0, int *c1);
 void amgb_dist_teardown(amgb_ctx *c);
 void amgb_ext_teardown(amgb_ctx *c);
+void amgb_pcg_teardown(amgb_ctx *c);      // frees the conjugate-gradient vectors and graph
 void amgb_async_teardown(amgb_ctx *c);   // frees the host copy of the persistent kernel's parameter block
 // persistent kernel, host side (async.cu), shared with the row-partitioned solve (dist_async.cu)
 double async_op_cost(const DevCSR &M, long sell_entries);                      // cost-model seed of the CTA groups
@@ -102,5 +107,6 @@ int amgb_dev_alloc_bytes(amgb_ctx *c, void **p, size_t bytes, bool zero);
 int amgb_build_sellu(amgb_ctx *c, DevCSR &M);   // SELL-U encoding of a sliced-ELL matrix whose scaled values are final
 void enq_spmv(amgb_ctx *c, const DevCSR &M, bool sval, const double *x, double *y, const SpmvEpilogue &e, bool norm);
 void enq_residual(amgb_ctx *c);
-void enq_cycle(amgb_ctx *c, double *target, bool accumulate);
+void enq_spmv_dot(amgb_ctx *c, const DevCSR &M, bool sval, const double *x, double *y, const SpmvEpilogue &e, const double *w, double *dot_out);
+void enq_cycle(amgb_ctx *c, double *target, bool accumulate, const double *dot_w = nullptr, double *dot_out = nullptr);
 int amgb_fetch_scalar(amgb_ctx *c, double *out);

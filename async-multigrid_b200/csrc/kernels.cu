@@ -14,29 +14,32 @@ constexpr int kBlock = 256;
 
 // One kernel per storage scheme (separate register budgets): MODE 0 = vector-per-row CSR, 1 = sliced ELL,
 // 2 (3, 4: other register budgets) = sliced ELL with the SELL-U encoding (stencil levels); the CSR-stream kernel (row blocks through shared memory) is k_spmv_stream.
-template <int MODE, bool SVAL>
-__global__ void __launch_bounds__(kBlock, MODE == 2 ? 5 : (MODE == 3 ? 4 : (MODE == 4 ? 6 : (MODE == 5 ? 4 : 1)))) k_spmv(DevCSR M, const double *x, double *y, SpmvEpilogue e, double *partials)
+// DOT: the fused per-CTA partial is sum_i y_i * w_i instead of sum_i y_i^2 (a separate instantiation, so that the others keep
+// their registers)
+template <int MODE, bool SVAL, bool DOT = false>
+__global__ void __launch_bounds__(kBlock, MODE == 2 ? 5 : (MODE == 3 ? 4 : (MODE == 4 ? 6 : (MODE == 5 ? 4 : 1)))) k_spmv(DevCSR M, const double *x, double *y, SpmvEpilogue e, double *partials,
+                                                                                                                                          const double *w)
 {
    const int tid = blockIdx.x * kBlock + threadIdx.x;
    const int tsz = gridDim.x * kBlock;
    const bool norm = partials != nullptr;
    double ss;
-   if (MODE == 5) ss = sell_rows_team<true, SVAL, 8, false>(M, x, y, e, tid, tsz, norm);  // the generic batch-of-8 loop ("v2", 56 registers)
-   else if (MODE >= 2) ss = sell_rows_team<true, SVAL, 4, true>(M, x, y, e, tid, tsz, norm);   // (2 / 3 / 4: the cached-delta path at 5 / 4 / 6 CTAs per SM)
-   else if (MODE == 1) ss = sell_rows_team<true, SVAL>(M, x, y, e, tid, tsz, norm);
-   else ss = csr_rows_dispatch<true, SVAL>(M, x, y, e, tid, tsz, norm);
+   if (MODE == 5) ss = sell_rows_team<true, SVAL, 8, false, DOT>(M, x, y, e, tid, tsz, norm, w);  // the generic batch-of-8 loop ("v2", 56 registers)
+   else if (MODE >= 2) ss = sell_rows_team<true, SVAL, 4, true, DOT>(M, x, y, e, tid, tsz, norm, w);   // (2 / 3 / 4: the cached-delta path at 5 / 4 / 6 CTAs per SM)
+   else if (MODE == 1) ss = sell_rows_team<true, SVAL, 0, false, DOT>(M, x, y, e, tid, tsz, norm, w);
+   else ss = csr_rows_dispatch<true, SVAL, DOT>(M, x, y, e, tid, tsz, norm, w);
    if (norm) {
       ss = block_sum(ss);
       if (threadIdx.x == 0) partials[blockIdx.x] = ss;
    }
 }
 
-template <int NT, int CAP, int XCAP, int ST, bool SVAL>
-__global__ void __launch_bounds__(NT) k_spmv_stream(DevCSR M, const double *x, double *y, SpmvEpilogue e, double *partials)
+template <int NT, int CAP, int XCAP, int ST, bool SVAL, bool DOT = false>
+__global__ void __launch_bounds__(NT) k_spmv_stream(DevCSR M, const double *x, double *y, SpmvEpilogue e, double *partials, const double *w)
 {
    extern __shared__ __align__(128) unsigned char dyn_smem[];
    const bool norm = partials != nullptr;
-   double ss = stream_rows_team<true, SVAL, NT, CAP, XCAP, ST>(M, x, y, e, blockIdx.x, gridDim.x, dyn_smem, norm, M.blk, M.nblk);
+   double ss = stream_rows_team<true, SVAL, NT, CAP, XCAP, ST, DOT>(M, x, y, e, blockIdx.x, gridDim.x, dyn_smem, norm, M.blk, M.nblk, w);
    if (norm) {
       ss = block_sum(ss);
       if (threadIdx.x == 0) partials[blockIdx.x] = ss;
@@ -97,6 +100,45 @@ __global__ void __launch_bounds__(kBlock) k_dot(int n, const double *__restrict_
    for (int i = blockIdx.x * kBlock + threadIdx.x; i < n; i += gridDim.x * kBlock) s += x[i] * y[i];
    s = block_sum(s);
    if (threadIdx.x == 0) partials[blockIdx.x] = s;
+}
+
+// preconditioned conjugate gradients (csrc/pcg.cu): every CTA reads the scalars the previous reductions left in s[PCG_*]
+// (no host round trip).  p = z + beta p, beta = rho / rho_old, and p = z outright on the first iteration (0 * p would keep a
+// NaN an earlier solve left in p).
+__global__ void __launch_bounds__(kBlock) k_pcg_dir(int n, const double *__restrict__ z, double *__restrict__ p, const double *s)
+{
+   const bool first = s[PCG_DONE] == 0.0;
+   const double beta = first ? 0.0 : s[PCG_RHO] / s[PCG_RHO_OLD];
+   for (int i = blockIdx.x * kBlock + threadIdx.x; i < n; i += gridDim.x * kBlock) p[i] = first ? z[i] : z[i] + beta * p[i];
+}
+
+// alpha = rho / sigma; u += alpha p; r -= alpha q; partial sums of r_i^2.  On a breakdown (rho or sigma not positive and
+// finite) u and r are left as they are, so that they hold the completed iterations.  CTA 0 then records rho as rho_old and
+// counts the iteration (the other CTAs never read those two slots in this launch).
+__global__ void __launch_bounds__(kBlock) k_pcg_update(int n, const double *__restrict__ p, const double *__restrict__ q,
+                                                       double *__restrict__ u, double *__restrict__ r, double *s, double *partials)
+{
+   const double rho = s[PCG_RHO], sigma = s[PCG_SIGMA];
+   const bool ok = isfinite(rho) && rho > 0.0 && isfinite(sigma) && sigma > 0.0;
+   const double alpha = rho / sigma;
+   double ss = 0.0;
+   for (int i = blockIdx.x * kBlock + threadIdx.x; i < n; i += gridDim.x * kBlock) {
+      double ri = r[i];
+      if (ok) {
+         u[i] += alpha * p[i];
+         ri -= alpha * q[i];
+         r[i] = ri;
+      }
+      ss += ri * ri;
+   }
+   ss = block_sum(ss);
+   if (threadIdx.x == 0) {
+      partials[blockIdx.x] = ss;
+      if (blockIdx.x == 0 && ok) {
+         s[PCG_RHO_OLD] = rho;
+         s[PCG_DONE] += 1.0;
+      }
+   }
 }
 
 // u += e on this GPU and on every peer GPU (their u mapped through CUDA IPC): the `#pragma omp atomic` of
@@ -212,14 +254,14 @@ inline int grid_for(const LaunchCfg &cfg, long work_threads)
 
 }  // namespace
 
-template <int EPT, bool SVAL, bool SORTED>
-__global__ void __launch_bounds__(kBlock) k_spmv_wstream(DevCSR M, const double *x, double *y, SpmvEpilogue e, double *partials)
+template <int EPT, bool SVAL, bool SORTED, bool DOT = false>
+__global__ void __launch_bounds__(kBlock) k_spmv_wstream(DevCSR M, const double *x, double *y, SpmvEpilogue e, double *partials, const double *w)
 {
    __shared__ __align__(16) double swarp[(kBlock / 32) * EPT * 32];
    const bool norm = partials != nullptr;
    const int warp = threadIdx.x >> 5;
-   double ss = warp_stream_rows_team<true, SVAL, EPT, SORTED>(M, x, y, e, blockIdx.x * (kBlock / 32) + warp, gridDim.x * (kBlock / 32),
-                                                              swarp + warp * EPT * 32, norm);
+   double ss = warp_stream_rows_team<true, SVAL, EPT, SORTED, DOT>(M, x, y, e, blockIdx.x * (kBlock / 32) + warp, gridDim.x * (kBlock / 32),
+                                                              swarp + warp * EPT * 32, norm, w);
    if (norm) {
       ss = block_sum(ss);
       if (threadIdx.x == 0) partials[blockIdx.x] = ss;
@@ -240,75 +282,97 @@ static int resident_ctas(K kernel, int block, size_t dyn, int num_sms, int *cach
    return num_sms * *cache;
 }
 
+// (per instantiation: a function template has one set of statics per instantiation)
+template <int MODE, bool SVAL, bool DOT>
+static int spmv_mode_go(const LaunchCfg &cfg, cudaStream_t st, const DevCSR &M, const double *x, double *y, const SpmvEpilogue &e,
+                        double *partials, long ctas_of_work, const double *w)
+{
+   static int occ = 0;
+   const int cap = resident_ctas(k_spmv<MODE, SVAL, DOT>, kBlock, 0, cfg.num_sms, &occ);
+   const int grid = (int)std::max(1L, std::min(ctas_of_work, (long)cap));
+   k_spmv<MODE, SVAL, DOT><<<grid, kBlock, 0, st>>>(M, x, y, e, partials, w);
+   return grid;
+}
 template <int MODE>
 static int launch_spmv_mode(const LaunchCfg &cfg, cudaStream_t st, const DevCSR &M, bool use_sval, const double *x, double *y,
-                            const SpmvEpilogue &e, double *partials, long ctas_of_work)
+                            const SpmvEpilogue &e, double *partials, long ctas_of_work, const double *w)
 {
-   static int occ[2] = {0, 0};   // (per MODE: a function template has one set of statics per instantiation)
-   const int cap = use_sval ? resident_ctas(k_spmv<MODE, true>, kBlock, 0, cfg.num_sms, &occ[1])
-                            : resident_ctas(k_spmv<MODE, false>, kBlock, 0, cfg.num_sms, &occ[0]);
-   const int grid = (int)std::max(1L, std::min(ctas_of_work, (long)cap));
-   if (use_sval) k_spmv<MODE, true><<<grid, kBlock, 0, st>>>(M, x, y, e, partials);
-   else k_spmv<MODE, false><<<grid, kBlock, 0, st>>>(M, x, y, e, partials);
-   return grid;
+   if (w) return use_sval ? spmv_mode_go<MODE, true, true>(cfg, st, M, x, y, e, partials, ctas_of_work, w)
+                          : spmv_mode_go<MODE, false, true>(cfg, st, M, x, y, e, partials, ctas_of_work, w);
+   return use_sval ? spmv_mode_go<MODE, true, false>(cfg, st, M, x, y, e, partials, ctas_of_work, nullptr)
+                   : spmv_mode_go<MODE, false, false>(cfg, st, M, x, y, e, partials, ctas_of_work, nullptr);
 }
 
+template <int NT, int CAP, int XCAP, int ST, bool SVAL, bool DOT>
+static int stream_go(const LaunchCfg &cfg, cudaStream_t st, const DevCSR &M, const double *x, double *y, const SpmvEpilogue &e,
+                     double *partials, const double *w)
+{
+   static int occ = 0;
+   constexpr size_t dyn = stream_smem_bytes(CAP, XCAP, ST);
+   const int cap = resident_ctas(k_spmv_stream<NT, CAP, XCAP, ST, SVAL, DOT>, NT, dyn, cfg.num_sms, &occ);
+   const int grid = (int)std::max(1L, std::min((long)M.nblk, (long)cap));
+   k_spmv_stream<NT, CAP, XCAP, ST, SVAL, DOT><<<grid, NT, dyn, st>>>(M, x, y, e, partials, w);
+   return grid;
+}
 template <int NT, int CAP, int XCAP, int ST>
 static int launch_stream_variant(const LaunchCfg &cfg, cudaStream_t st, const DevCSR &M, bool use_sval, const double *x, double *y,
-                                 const SpmvEpilogue &e, double *partials)
+                                 const SpmvEpilogue &e, double *partials, const double *w)
 {
-   static int occ[2] = {0, 0};
-   constexpr size_t dyn = stream_smem_bytes(CAP, XCAP, ST);
-   const int cap = use_sval ? resident_ctas(k_spmv_stream<NT, CAP, XCAP, ST, true>, NT, dyn, cfg.num_sms, &occ[1])
-                            : resident_ctas(k_spmv_stream<NT, CAP, XCAP, ST, false>, NT, dyn, cfg.num_sms, &occ[0]);
-   const int grid = (int)std::max(1L, std::min((long)M.nblk, (long)cap));
-   if (use_sval) k_spmv_stream<NT, CAP, XCAP, ST, true><<<grid, NT, dyn, st>>>(M, x, y, e, partials);
-   else k_spmv_stream<NT, CAP, XCAP, ST, false><<<grid, NT, dyn, st>>>(M, x, y, e, partials);
-   return grid;
+   if (w) return use_sval ? stream_go<NT, CAP, XCAP, ST, true, true>(cfg, st, M, x, y, e, partials, w)
+                          : stream_go<NT, CAP, XCAP, ST, false, true>(cfg, st, M, x, y, e, partials, w);
+   return use_sval ? stream_go<NT, CAP, XCAP, ST, true, false>(cfg, st, M, x, y, e, partials, nullptr)
+                   : stream_go<NT, CAP, XCAP, ST, false, false>(cfg, st, M, x, y, e, partials, nullptr);
 }
 
-template <int EPT, bool SORTED>
-static int launch_wstream(const LaunchCfg &cfg, cudaStream_t st, const DevCSR &M, bool use_sval, const double *x, double *y,
-                          const SpmvEpilogue &e, double *partials)
+template <int EPT, bool SORTED, bool SVAL, bool DOT>
+static int wstream_go(const LaunchCfg &cfg, cudaStream_t st, const DevCSR &M, const double *x, double *y, const SpmvEpilogue &e,
+                      double *partials, const double *w)
 {
-   static int occ[2] = {0, 0};
-   const int cap = use_sval ? resident_ctas(k_spmv_wstream<EPT, true, SORTED>, kBlock, 0, cfg.num_sms, &occ[1])
-                            : resident_ctas(k_spmv_wstream<EPT, false, SORTED>, kBlock, 0, cfg.num_sms, &occ[0]);
+   static int occ = 0;
+   const int cap = resident_ctas(k_spmv_wstream<EPT, SVAL, SORTED, DOT>, kBlock, 0, cfg.num_sms, &occ);
    const long want = ((long)M.nblk + kBlock / 32 - 1) / (kBlock / 32);
    const int grid = (int)std::max(1L, std::min(want, (long)cap));
-   if (use_sval) k_spmv_wstream<EPT, true, SORTED><<<grid, kBlock, 0, st>>>(M, x, y, e, partials);
-   else k_spmv_wstream<EPT, false, SORTED><<<grid, kBlock, 0, st>>>(M, x, y, e, partials);
+   k_spmv_wstream<EPT, SVAL, SORTED, DOT><<<grid, kBlock, 0, st>>>(M, x, y, e, partials, w);
    return grid;
+}
+template <int EPT, bool SORTED>
+static int launch_wstream(const LaunchCfg &cfg, cudaStream_t st, const DevCSR &M, bool use_sval, const double *x, double *y,
+                          const SpmvEpilogue &e, double *partials, const double *w)
+{
+   if (w) return use_sval ? wstream_go<EPT, SORTED, true, true>(cfg, st, M, x, y, e, partials, w)
+                          : wstream_go<EPT, SORTED, false, true>(cfg, st, M, x, y, e, partials, w);
+   return use_sval ? wstream_go<EPT, SORTED, true, false>(cfg, st, M, x, y, e, partials, nullptr)
+                   : wstream_go<EPT, SORTED, false, false>(cfg, st, M, x, y, e, partials, nullptr);
 }
 
 int launch_spmv(const LaunchCfg &cfg, cudaStream_t st, const DevCSR &M, bool use_sval, const double *x, double *y,
-                const SpmvEpilogue &e, double *partials, int *grid_out)
+                const SpmvEpilogue &e, double *partials, int *grid_out, const double *dot_w)
 {
    int grid;
-   if (M.sell_slices > 0 && M.su_desc && cfg.sellu_ctas == 4) grid = launch_spmv_mode<3>(cfg, st, M, use_sval, x, y, e, partials, ((long)M.sell_slices * 32 + kBlock - 1) / kBlock);
-   else if (M.sell_slices > 0 && M.su_desc && cfg.sellu_ctas == 6) grid = launch_spmv_mode<4>(cfg, st, M, use_sval, x, y, e, partials, ((long)M.sell_slices * 32 + kBlock - 1) / kBlock);
-   else if (M.sell_slices > 0 && M.su_desc && cfg.sellu_ctas == 8) grid = launch_spmv_mode<5>(cfg, st, M, use_sval, x, y, e, partials, ((long)M.sell_slices * 32 + kBlock - 1) / kBlock);
-   else if (M.sell_slices > 0 && M.su_desc) grid = launch_spmv_mode<2>(cfg, st, M, use_sval, x, y, e, partials, ((long)M.sell_slices * 32 + kBlock - 1) / kBlock);
-   else if (M.sell_slices > 0) grid = launch_spmv_mode<1>(cfg, st, M, use_sval, x, y, e, partials, ((long)M.sell_slices * 32 + kBlock - 1) / kBlock);
+   if (M.sell_slices > 0 && M.su_desc && cfg.sellu_ctas == 4) grid = launch_spmv_mode<3>(cfg, st, M, use_sval, x, y, e, partials, ((long)M.sell_slices * 32 + kBlock - 1) / kBlock, dot_w);
+   else if (M.sell_slices > 0 && M.su_desc && cfg.sellu_ctas == 6) grid = launch_spmv_mode<4>(cfg, st, M, use_sval, x, y, e, partials, ((long)M.sell_slices * 32 + kBlock - 1) / kBlock, dot_w);
+   else if (M.sell_slices > 0 && M.su_desc && cfg.sellu_ctas == 8) grid = launch_spmv_mode<5>(cfg, st, M, use_sval, x, y, e, partials, ((long)M.sell_slices * 32 + kBlock - 1) / kBlock, dot_w);
+   else if (M.sell_slices > 0 && M.su_desc) grid = launch_spmv_mode<2>(cfg, st, M, use_sval, x, y, e, partials, ((long)M.sell_slices * 32 + kBlock - 1) / kBlock, dot_w);
+   else if (M.sell_slices > 0) grid = launch_spmv_mode<1>(cfg, st, M, use_sval, x, y, e, partials, ((long)M.sell_slices * 32 + kBlock - 1) / kBlock, dot_w);
    else if (M.nblk > 0 && M.wept > 0) {
       if (M.pos) {
-         if (M.wept <= 4) grid = launch_wstream<4, true>(cfg, st, M, use_sval, x, y, e, partials);
-         else grid = launch_wstream<8, true>(cfg, st, M, use_sval, x, y, e, partials);
-      } else if (M.wept <= 4) grid = launch_wstream<4, false>(cfg, st, M, use_sval, x, y, e, partials);
-      else if (M.wept <= 8) grid = launch_wstream<8, false>(cfg, st, M, use_sval, x, y, e, partials);
-      else grid = launch_wstream<16, false>(cfg, st, M, use_sval, x, y, e, partials);
+         if (M.wept <= 4) grid = launch_wstream<4, true>(cfg, st, M, use_sval, x, y, e, partials, dot_w);
+         else grid = launch_wstream<8, true>(cfg, st, M, use_sval, x, y, e, partials, dot_w);
+      } else if (M.wept <= 4) grid = launch_wstream<4, false>(cfg, st, M, use_sval, x, y, e, partials, dot_w);
+      else if (M.wept <= 8) grid = launch_wstream<8, false>(cfg, st, M, use_sval, x, y, e, partials, dot_w);
+      else grid = launch_wstream<16, false>(cfg, st, M, use_sval, x, y, e, partials, dot_w);
    } else if (M.nblk > 0) {
       switch (cfg.stream_variant) {   // keep in step with kStreamVariants (launch.h)
-         case 1: grid = launch_stream_variant<128, 1024, 0, 2>(cfg, st, M, use_sval, x, y, e, partials); break;
-         case 2: grid = launch_stream_variant<128, 1024, 0, 3>(cfg, st, M, use_sval, x, y, e, partials); break;
-         case 3: grid = launch_stream_variant<256, 2048, 1536, 2>(cfg, st, M, use_sval, x, y, e, partials); break;
-         case 4: grid = launch_stream_variant<128, 1024, 1024, 2>(cfg, st, M, use_sval, x, y, e, partials); break;
-         case 5: grid = launch_stream_variant<256, 1024, 0, 2>(cfg, st, M, use_sval, x, y, e, partials); break;
-         case 6: grid = launch_stream_variant<128, 1024, 1024, 3>(cfg, st, M, use_sval, x, y, e, partials); break;
-         case 7: grid = launch_stream_variant<128, 2048, 0, 2>(cfg, st, M, use_sval, x, y, e, partials); break;
-         default: grid = launch_stream_variant<256, 2048, 0, 3>(cfg, st, M, use_sval, x, y, e, partials); break;
+         case 1: grid = launch_stream_variant<128, 1024, 0, 2>(cfg, st, M, use_sval, x, y, e, partials, dot_w); break;
+         case 2: grid = launch_stream_variant<128, 1024, 0, 3>(cfg, st, M, use_sval, x, y, e, partials, dot_w); break;
+         case 3: grid = launch_stream_variant<256, 2048, 1536, 2>(cfg, st, M, use_sval, x, y, e, partials, dot_w); break;
+         case 4: grid = launch_stream_variant<128, 1024, 1024, 2>(cfg, st, M, use_sval, x, y, e, partials, dot_w); break;
+         case 5: grid = launch_stream_variant<256, 1024, 0, 2>(cfg, st, M, use_sval, x, y, e, partials, dot_w); break;
+         case 6: grid = launch_stream_variant<128, 1024, 1024, 3>(cfg, st, M, use_sval, x, y, e, partials, dot_w); break;
+         case 7: grid = launch_stream_variant<128, 2048, 0, 2>(cfg, st, M, use_sval, x, y, e, partials, dot_w); break;
+         default: grid = launch_stream_variant<256, 2048, 0, 3>(cfg, st, M, use_sval, x, y, e, partials, dot_w); break;
       }
-   } else grid = launch_spmv_mode<0>(cfg, st, M, use_sval, x, y, e, partials, ((long)M.nrows * M.lpr + kBlock - 1) / kBlock);
+   } else grid = launch_spmv_mode<0>(cfg, st, M, use_sval, x, y, e, partials, ((long)M.nrows * M.lpr + kBlock - 1) / kBlock, dot_w);
    if (grid_out) *grid_out = grid;
    return 1;
 }
@@ -317,7 +381,7 @@ int spmv_units(const DevCSR &M) { return M.sell_slices > 0 ? M.sell_slices : (M.
 
 // the same product restricted to launch units [u0, u1) (slices / chunks / rows, whichever the storage uses)
 int launch_spmv_units(const LaunchCfg &cfg, cudaStream_t st, const DevCSR &M, int u0, int u1, bool use_sval, const double *x,
-                      double *y, const SpmvEpilogue &e, double *partials, int *grid_out)
+                      double *y, const SpmvEpilogue &e, double *partials, int *grid_out, const double *dot_w)
 {
    if (grid_out) *grid_out = 0;
    if (u1 <= u0) return 0;
@@ -333,8 +397,9 @@ int launch_spmv_units(const LaunchCfg &cfg, cudaStream_t st, const DevCSR &M, in
       if (ev.rs) ev.rs += u0;
       if (ev.b2) ev.b2 += u0;
       if (ev.xs) ev.xs += u0;
+      if (dot_w) dot_w += u0;
    }
-   return launch_spmv(cfg, st, V, use_sval, x, yv, ev, partials, grid_out);
+   return launch_spmv(cfg, st, V, use_sval, x, yv, ev, partials, grid_out, dot_w);
 }
 
 int launch_reduce_partials(cudaStream_t st, const double *partials, int n, double *out)
@@ -373,6 +438,21 @@ int launch_dot(const LaunchCfg &cfg, cudaStream_t st, int n, const double *x, co
    int grid = grid_for(cfg, n);
    if (grid_out) *grid_out = grid;
    k_dot<<<grid, kBlock, 0, st>>>(n, x, y, partials);
+   return 1;
+}
+
+int launch_pcg_dir(const LaunchCfg &cfg, cudaStream_t st, int n, const double *z, double *p, const double *s)
+{
+   k_pcg_dir<<<grid_for(cfg, n), kBlock, 0, st>>>(n, z, p, s);
+   return 1;
+}
+
+int launch_pcg_update(const LaunchCfg &cfg, cudaStream_t st, int n, const double *p, const double *q, double *u, double *r,
+                      double *s, double *partials, int *grid_out)
+{
+   const int grid = grid_for(cfg, n);
+   if (grid_out) *grid_out = grid;
+   k_pcg_update<<<grid, kBlock, 0, st>>>(n, p, q, u, r, s, partials);
    return 1;
 }
 

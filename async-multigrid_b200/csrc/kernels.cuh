@@ -18,12 +18,17 @@ __device__ __forceinline__ double ld_x(const double *p)
    return ld_ca(p);
 }
 
+// DOT (stand-alone kernels): the fused per-CTA sum of a launch that wants one is sum_i y_i * dw_i instead of sum_i y_i^2 (the
+// dot products of the conjugate-gradient solve, pcg.cu).  It is written inline at every row store: routed through a helper
+// or a field of SpmvEpilogue, it changed the persistent kernel's spills although that kernel never takes the DOT path.
+
 // ---- CSR, LPR lanes per row (vector-per-row; LPR = 32 is warp-per-row) --------------------------
 // reference loop: src/SMEM_MatVec.cpp:316-322 (+ the epilogues listed in common.cuh)
-template <int LPR, bool RO, bool SVAL>
+template <int LPR, bool RO, bool SVAL, bool DOT = false>
 __device__ __forceinline__ double csr_rows_team(const DevCSR &M, const double *__restrict__ x,
                                                 double *y, const SpmvEpilogue &e,
-                                                int team_tid, int team_size, bool want_sumsq)
+                                                int team_tid, int team_size, bool want_sumsq,
+                                                const double *dw = nullptr)
 {
    const int lane = team_tid & (LPR - 1);
    constexpr int RPW = 32 / LPR;                       // rows per warp and iteration
@@ -41,7 +46,7 @@ __device__ __forceinline__ double csr_rows_team(const DevCSR &M, const double *_
       if (lane == 0 && ok) {
          double v = epilogue_apply<RO>(e, row, acc);
          epilogue_store<RO>(e, y, row, v);
-         if (want_sumsq) sumsq += v * v;
+         if (want_sumsq) sumsq += DOT ? v * __ldg(dw + row) : v * v;
       }
    }
    return sumsq;
@@ -59,10 +64,10 @@ __device__ __forceinline__ double csr_rows_team(const DevCSR &M, const double *_
 //          (profiles/README.md R2.3): it is bound by instruction issue and by the number of resident warps, not by HBM --
 //          a variant with every value and the epilogue operands held in registers (80 registers, 3 CTAs/SM) was SLOWER
 //          (0.226 ms against 0.19) than the generic loop at 56 registers; so this path is written for <= 40 registers.
-template <bool RO, bool SVAL, int SU = 0, bool FAST = false>
+template <bool RO, bool SVAL, int SU = 0, bool FAST = false, bool DOT = false>
 __device__ __forceinline__ double sell_rows_team(const DevCSR &M, const double *__restrict__ x,
                                                  double *y, const SpmvEpilogue &e,
-                                                 int team_tid, int team_size, bool want_sumsq)
+                                                 int team_tid, int team_size, bool want_sumsq, const double *dw = nullptr)
 {
    const int lane = team_tid & 31;
    const int nwarp = team_size >> 5;
@@ -104,7 +109,7 @@ __device__ __forceinline__ double sell_rows_team(const DevCSR &M, const double *
             if (k < ccount) acc += __ldg(gv + k) * xv[k];
          const double v = epilogue_apply<RO>(e, row, acc);
          epilogue_store<RO>(e, y, row, v);
-         if (want_sumsq) sumsq += v * v;
+         if (want_sumsq) sumsq += DOT ? v * __ldg(dw + row) : v * v;
       } else if (SU > 0 && dsc.y > 0) {
          const double *__restrict__ gv = SVAL ? M.su_sval : M.su_va;
          const bool ok = row < M.nrows;
@@ -130,7 +135,7 @@ __device__ __forceinline__ double sell_rows_team(const DevCSR &M, const double *
          if (ok) {
             const double v = PRELOAD ? epilogue_finish(e, ops, acc) : epilogue_apply<RO>(e, row, acc);
             epilogue_store<RO>(e, y, row, v);
-            if (want_sumsq) sumsq += v * v;
+            if (want_sumsq) sumsq += DOT ? v * __ldg(dw + row) : v * v;
          }
       } else {
          const int off = __ldg(M.sell_off + sl);
@@ -142,7 +147,7 @@ __device__ __forceinline__ double sell_rows_team(const DevCSR &M, const double *
          if (row >= 0 && row < M.nrows) {
             double v = epilogue_apply<RO>(e, row, acc);
             epilogue_store<RO>(e, y, row, v);
-            if (want_sumsq) sumsq += v * v;
+            if (want_sumsq) sumsq += DOT ? v * __ldg(dw + row) : v * v;
          }
       }
       dsc = dnext;
@@ -164,10 +169,11 @@ __device__ __forceinline__ double sell_rows_team(const DevCSR &M, const double *
 __host__ __device__ constexpr int stream_stage_bytes(int cap, int xcap) { return cap * 12 + xcap * 8; }
 __host__ __device__ constexpr int stream_smem_bytes(int cap, int xcap, int st) { return st * stream_stage_bytes(cap, xcap) + 64; }
 
-template <bool RO, bool SVAL, int NT, int CAP, int XCAP, int ST>
+template <bool RO, bool SVAL, int NT, int CAP, int XCAP, int ST, bool DOT = false>
 __device__ __forceinline__ double stream_rows_team(const DevCSR &M, const double *__restrict__ x, double *y,
                                                    const SpmvEpilogue &e, int team_cta, int team_nctas,
-                                                   unsigned char *smem, bool want_sumsq, const int4 *blk, int nblk)
+                                                   unsigned char *smem, bool want_sumsq, const int4 *blk, int nblk,
+                                                   const double *dw = nullptr)
 {
    constexpr int SB = stream_stage_bytes(CAP, XCAP);
    constexpr int EPT = CAP / NT;                      // entries per thread
@@ -252,7 +258,7 @@ __device__ __forceinline__ double stream_rows_team(const DevCSR &M, const double
          if (tid == 0) {
             const double v = epilogue_apply<RO>(e, r0, acc);
             y[r0] = v;
-            if (want_sumsq) sumsq += v * v;
+            if (want_sumsq) sumsq += DOT ? v * __ldg(dw + r0) : v * v;
          }
          __syncthreads();
       } else {
@@ -309,7 +315,7 @@ __device__ __forceinline__ double stream_rows_team(const DevCSR &M, const double
             if (lane == 0 && ok_a) {
                const double v = epilogue_finish(e, o_a, acc);
                y[row_a] = v;
-               if (want_sumsq) sumsq += v * v;
+               if (want_sumsq) sumsq += DOT ? v * __ldg(dw + row_a) : v * v;
             }
          }
          for (int base = rows_per_pass; base < nr; base += rows_per_pass) {   // only when lpr == 1
@@ -320,7 +326,7 @@ __device__ __forceinline__ double stream_rows_team(const DevCSR &M, const double
                for (int q = s1; q < t1; q++) acc += vs[q];
                const double v = epilogue_apply<RO>(e, row, acc);
                y[row] = v;
-               if (want_sumsq) sumsq += v * v;
+               if (want_sumsq) sumsq += DOT ? v * __ldg(dw + row) : v * v;
             }
          }
          __syncthreads();                              // the stage is free again
@@ -347,10 +353,10 @@ __device__ __forceinline__ double stream_rows_team(const DevCSR &M, const double
 // for each other, so the load / gather / reduce phases of the 32-64 resident warps of an SM overlap
 // freely -- the CTA-synchronous variant above spends ~20 % of its issue slots in barrier stalls and ~45 %
 // waiting on gathers with only 3-5 CTAs to hide them (profiles/).  swarp: EPT*32 doubles per warp.
-template <bool RO, bool SVAL, int EPT, bool SORTED = false>
+template <bool RO, bool SVAL, int EPT, bool SORTED = false, bool DOT = false>
 __device__ __forceinline__ double warp_stream_rows_team(const DevCSR &M, const double *__restrict__ x, double *y,
                                                         const SpmvEpilogue &e, int team_warp, int team_nwarps,
-                                                        double *swarp, bool want_sumsq)
+                                                        double *swarp, bool want_sumsq, const double *dw = nullptr)
 {
    constexpr int CAP = EPT * 32;
    const int lane = threadIdx.x & 31;
@@ -368,7 +374,7 @@ __device__ __forceinline__ double warp_stream_rows_team(const DevCSR &M, const d
          if (lane == 0) {
             const double v = epilogue_apply<RO>(e, r0, acc);
             y[r0] = v;
-            if (want_sumsq) sumsq += v * v;
+            if (want_sumsq) sumsq += DOT ? v * __ldg(dw + r0) : v * v;
          }
          continue;
       }
@@ -419,7 +425,7 @@ __device__ __forceinline__ double warp_stream_rows_team(const DevCSR &M, const d
          if (sub == 0 && ok_a) {
             const double v = epilogue_finish(e, o_a, acc);
             y[row_a] = v;
-            if (want_sumsq) sumsq += v * v;
+            if (want_sumsq) sumsq += DOT ? v * __ldg(dw + row_a) : v * v;
          }
       }
       for (int base = 32; base < nr; base += 32) {     // only when lpr == 1
@@ -430,7 +436,7 @@ __device__ __forceinline__ double warp_stream_rows_team(const DevCSR &M, const d
             for (int q = s1; q < t1; q++) acc += swarp[q];
             const double v = epilogue_apply<RO>(e, row, acc);
             y[row] = v;
-            if (want_sumsq) sumsq += v * v;
+            if (want_sumsq) sumsq += DOT ? v * __ldg(dw + row) : v * v;
          }
       }
    }
@@ -438,16 +444,16 @@ __device__ __forceinline__ double warp_stream_rows_team(const DevCSR &M, const d
 }
 
 // vector-per-row CSR with the lanes-per-row chosen at upload time
-template <bool RO, bool SVAL>
+template <bool RO, bool SVAL, bool DOT = false>
 __device__ __forceinline__ double csr_rows_dispatch(const DevCSR &M, const double *x, double *y, const SpmvEpilogue &e,
-                                                    int team_tid, int team_size, bool want_sumsq)
+                                                    int team_tid, int team_size, bool want_sumsq, const double *dw = nullptr)
 {
    switch (M.lpr) {
-      case 2: return csr_rows_team<2, RO, SVAL>(M, x, y, e, team_tid, team_size, want_sumsq);
-      case 4: return csr_rows_team<4, RO, SVAL>(M, x, y, e, team_tid, team_size, want_sumsq);
-      case 8: return csr_rows_team<8, RO, SVAL>(M, x, y, e, team_tid, team_size, want_sumsq);
-      case 16: return csr_rows_team<16, RO, SVAL>(M, x, y, e, team_tid, team_size, want_sumsq);
-      default: return csr_rows_team<32, RO, SVAL>(M, x, y, e, team_tid, team_size, want_sumsq);
+      case 2: return csr_rows_team<2, RO, SVAL, DOT>(M, x, y, e, team_tid, team_size, want_sumsq, dw);
+      case 4: return csr_rows_team<4, RO, SVAL, DOT>(M, x, y, e, team_tid, team_size, want_sumsq, dw);
+      case 8: return csr_rows_team<8, RO, SVAL, DOT>(M, x, y, e, team_tid, team_size, want_sumsq, dw);
+      case 16: return csr_rows_team<16, RO, SVAL, DOT>(M, x, y, e, team_tid, team_size, want_sumsq, dw);
+      default: return csr_rows_team<32, RO, SVAL, DOT>(M, x, y, e, team_tid, team_size, want_sumsq, dw);
    }
 }
 

@@ -26,13 +26,13 @@ static const StreamVariant kStreamVariants[AMGB_NUM_STREAM_VARIANTS] = {
    {256, 256, 0, 0}, {256, 128, 0, 0}, {256, 512, 0, 0}, {256, 256, 0, -1}, {256, 128, 0, -1},
 };
 
-// y = gamma*c + rs.*(beta*b + alpha*M*x); optional sum of y_i^2 into partial sums (one per CTA,
-// `partials` must hold >= grid entries; *grid_out receives the grid used).
+// y = gamma*c + rs.*(beta*b + alpha*M*x); optional sum of y_i^2 -- or of y_i*dot_w_i when dot_w is given -- into partial
+// sums (one per CTA, `partials` must hold >= grid entries; *grid_out receives the grid used).
 int launch_spmv(const LaunchCfg &cfg, cudaStream_t st, const DevCSR &M, bool use_sval, const double *x, double *y,
-                const SpmvEpilogue &e, double *partials, int *grid_out);
+                const SpmvEpilogue &e, double *partials, int *grid_out, const double *dot_w = nullptr);
 int spmv_units(const DevCSR &M);
 int launch_spmv_units(const LaunchCfg &cfg, cudaStream_t st, const DevCSR &M, int u0, int u1, bool use_sval, const double *x,
-                      double *y, const SpmvEpilogue &e, double *partials, int *grid_out);
+                      double *y, const SpmvEpilogue &e, double *partials, int *grid_out, const double *dot_w = nullptr);
 // out[0] = sum(partials[0..n)); if hist != nullptr: hist[k] = sqrt(out[0]) (and r0 handling on host)
 int launch_reduce_partials(cudaStream_t st, const double *partials, int n, double *out);
 // y = a.*x  (zero-guess Jacobi: u = (w/d).*f, src/SMEM_Smooth.cpp:381-389)
@@ -45,6 +45,14 @@ int launch_cheby(const LaunchCfg &cfg, cudaStream_t st, int n, double omega, dou
 // y = a*x + b*y [, z = y]; partial sums of x_i*y_i
 int launch_axpby(const LaunchCfg &cfg, cudaStream_t st, int n, double a, const double *x, double b, double *y, double *z);
 int launch_dot(const LaunchCfg &cfg, cudaStream_t st, int n, const double *x, const double *y, double *partials, int *grid_out);
+// preconditioned conjugate gradients (pcg.cu): slots of the device scalar array.  Each reduction writes its own slot;
+// k_pcg_update records rho_old and the number of completed iterations (0 = the next direction is the first)
+enum { PCG_RHO = 0, PCG_SIGMA = 1, PCG_RR = 2, PCG_RHO_OLD = 3, PCG_DONE = 4, PCG_NSCALARS = 8 };
+// p = z + beta p with beta from s (p = z on the first iteration)
+int launch_pcg_dir(const LaunchCfg &cfg, cudaStream_t st, int n, const double *z, double *p, const double *s);
+// alpha = rho / sigma from s; u += alpha p; r -= alpha q (skipped on a breakdown); partial sums of r_i^2
+int launch_pcg_update(const LaunchCfg &cfg, cudaStream_t st, int n, const double *p, const double *q, double *u, double *r,
+                      double *s, double *partials, int *grid_out);
 // u += e here and on every peer GPU (IPC-mapped pointers)
 #define AMGB_MAX_PEERS 15
 struct PeerPtrs { double *p[AMGB_MAX_PEERS]; int n; };

@@ -26,7 +26,7 @@ ABI_SYMBOLS = [
     "amgb_spgemv", "amgb_spgemv_transpose", "amgb_smooth", "amgb_set_jgs_blocks", "amgb_norm2", "amgb_cycle", "amgb_eigs_power", "amgb_solve_sync", "amgb_solve_async",
     "amgb_async_groups", "amgb_solve_extended", "amgb_solve_extended_async", "amgb_smooth_transfer", "amgb_host_csr_free", "amgb_smem_solve", "amgb_time_residual", "amgb_level_storage", "amgb_time_spmv", "amgb_stream_stats", "amgb_l2_arena_bytes", "amgb_sellu_stats",
     "amgb_sellu_encode_host", "amgb_host_free", "amgb_async_program", "amgb_async_group_times",
-    "amgb_solve_extended_implicit_async", "amgb_ext_async_program",
+    "amgb_solve_extended_implicit_async", "amgb_ext_async_program", "amgb_solve_pcg",
     "amgb_dist_unique_id", "amgb_dist_init", "amgb_dist_set_level", "amgb_dist_setup", "amgb_dist_set_rhs",
     "amgb_dist_get_solution", "amgb_dist_solve_sync", "amgb_dist_solve_sync_accel", "amgb_dist_stats", "amgb_dist_eigs_power",
     "amgb_dist_solve_async", "amgb_dist_async_groups", "amgb_dist_async_plan",
@@ -87,6 +87,7 @@ def load_library():
     L.amgb_eigs_power.argtypes = [C.c_void_p, C.c_int, DP, DP]
     L.amgb_set_jgs_blocks.argtypes = [C.c_void_p, C.c_int, C.c_int, IP]
     L.amgb_solve_sync.argtypes = [C.c_void_p, C.c_double, C.c_int, C.c_int, C.c_double, C.c_double, DP, IP, DP]
+    L.amgb_solve_pcg.argtypes = [C.c_void_p, C.c_double, C.c_int, DP, IP, DP, DP]
     L.amgb_solve_async.argtypes = [C.c_void_p, C.c_int, C.c_int, IP, DP, DP]
     L.amgb_solve_extended.argtypes = [C.c_void_p, C.c_double, C.c_int, C.c_double, C.c_double, DP, IP, DP, DP, DP]
     L.amgb_solve_extended_async.argtypes = [C.c_void_p, C.c_double, C.c_int, C.c_double, C.c_double, IP, IP, DP, DP]
@@ -320,6 +321,16 @@ class Solver:
         mu, delta = cheby if cheby else (1.0, 1.0)
         self._ck(self.L.amgb_solve_sync(self.ctx, tol, max_cycles, 1 if cheby else 0, mu, delta, _dp(hist), C.byref(n), C.byref(secs)))
         return hist[:n.value + 1], secs.value
+
+    def solve_pcg(self, tol=1e-9, max_iters=200):
+        """conjugate gradients preconditioned by the context's Multadd / BPX cycle on the resident f, u (amgb_solve_pcg; the
+        reference's -hypre_pcg).  -> dict(iters, hist (recurrence residual, hist[0] = 1), relres (true final residual),
+        seconds); the solution stays in u (get_solution)"""
+        hist = np.zeros(max(int(max_iters), 0) + 1)
+        it = C.c_int(0)
+        rel, secs = C.c_double(0), C.c_double(0)
+        self._ck(self.L.amgb_solve_pcg(self.ctx, tol, int(max_iters), _dp(hist), C.byref(it), C.byref(rel), C.byref(secs)))
+        return dict(iters=it.value, hist=hist[:it.value + 1], relres=rel.value, seconds=secs.value)
 
     def solve_async(self, num_cycles, converge=CONVERGE_LOCAL):
         corr = np.zeros(self.h.num_levels, dtype=np.int32)

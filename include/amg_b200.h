@@ -149,6 +149,21 @@ int amgb_solve_sync(amgb_ctx *ctx, double tol, int max_cycles, int cheby_flag, d
  * mu = (max+min)/(max-min), delta = 2/(max+min) (src/SMEM_Cheby.cpp:48-49) -> amgb_solve_sync(cheby_flag = 1). */
 int amgb_eigs_power(amgb_ctx *ctx, int iters, double *eig_min, double *eig_max);
 
+/* Conjugate gradients preconditioned by the selected additive cycle from a zero guess (the reference reaches this through
+ * hypre's PCG with its cycles as the preconditioner: -hypre_pcg, src/DMEM_Setup.cpp:129-167) on the resident f, u; the
+ * solution is left in u.  r = f - A u, then per iteration z = B r, rho = (r, z), p = z + (rho / rho_old) p (p = z on the
+ * first), q = A p, sigma = (p, q), u += (rho / sigma) p, r -= (rho / sigma) q, until ||r|| / ||r_0|| < tol or max_iters.
+ * relres_hist[0..*iters] holds that recurrence residual (caller provides max_iters + 1 doubles, may be NULL); final_relres is
+ * the true ||f - A u|| / ||r_0||, recomputed once (0 when r_0 = 0); solve_seconds the device time of the loop.
+ * AMGB_EINVAL, before any launch, unless the preconditioner is a fixed symmetric operator: solver MULTADD or BPX, smoother
+ * weighted or L1 Jacobi, Multadd with both or neither of pre / post smoothing (otherwise Rbar != Pbar^T); also for a
+ * distributed context and max_iters < 0.  coarse_solve = 1 (DMEM's convention) is allowed.  A must be symmetric positive
+ * definite -- the caller's contract, as for amgb_eigs_power: rho or sigma not positive and finite is a breakdown,
+ * AMGB_ESTATE with the quantity and the iteration in amgb_last_error; *iters, the history and u then hold the completed
+ * iterations.  Parity with hypre_PCGSolve itself is not pinned (hypre is not vendored). */
+int amgb_solve_pcg(amgb_ctx *ctx, double tol, int max_iters, double *relres_hist, int *iters, double *final_relres,
+                   double *solve_seconds);
+
 /* SMEM_Async_Add_AMG (src/SMEM_Async_AMG.cpp:7-437) as ONE persistent cooperative kernel: each
  * level's correction chain owns a CTA group; groups share u through fp64 global atomics, no grid
  * barrier.  Stop rule: LOCAL = every group stops after num_cycles own corrections; GLOBAL = all
