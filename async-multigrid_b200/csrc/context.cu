@@ -102,6 +102,7 @@ void amgb_default_options(amgb_options *o)
    o->res_compute_type = 0;
    o->read_type = 0;
    o->lean_storage = 0;
+   o->factor_restriction = 0;
 }
 
 int amgb_create(amgb_ctx **out, int device)
@@ -723,6 +724,9 @@ int amgb_setup(amgb_ctx *c)
    if (o.smoother == AMGB_SMOOTH_L1_HYBRID_JGS && o.solver != AMGB_SOLVER_BPX)
       return amgb_fail(c, AMGB_EINVAL, "L1_HYBRID_JACOBI_GAUSS_SEIDEL exists in the Parfor smoother only (BPX); the reference's ALL_LEVELS "
                                        "dispatcher silently runs weighted Jacobi for it (src/SMEM_Solve.cpp:277-323)");
+   if (o.factor_restriction && !(o.solver == AMGB_SOLVER_MULTADD && c->symmetric && o.factor_level0 && o.num_fine_smooth_sweeps == 1 && !c->dist))
+      return amgb_fail(c, AMGB_EINVAL, "factor_restriction applies to synchronous Multadd on one GPU with factor_level0, the symmetrised "
+                                       "(L1-)Jacobi smoother and num_fine_smooth_sweeps = 1");
    if (o.factor_level0 && !((o.solver == AMGB_SOLVER_MULTADD || o.solver == AMGB_SOLVER_ASYNC_MULTADD) && c->symmetric))
       return amgb_fail(c, AMGB_EINVAL, "factor_level0 applies to Multadd with the symmetrised (L1-)Jacobi smoother");
    int rc;
@@ -959,16 +963,26 @@ void enq_cycle(amgb_ctx *c, double *target, bool accumulate, const double *dot_w
    // u += e_0 + Pbar_0 e_1 = (w/d) o (r_0 + t_0 - A_0 v) + v with v = P_0 e_1.  Two passes over A_0 (sliced ELL, HBM
    // speed) and two over the plain P_0 / R_0 replace A_0 + Pbar_0 + Rbar_0 (3.5x the entries of P_0, L1-bound).
    const bool fact0 = o.factor_level0 && multadd && c->symmetric && last_r >= 1;
+   // the same on the levels 1 <= l < last_r (amgb_options.factor_restriction, one smoothing sweep): the smoother's pass over
+   // A_l also writes t_l = r_l - A_l diag(s) r_l, and e_l = s o (r_l + t_l) comes out of it as a second output; then
+   // Rbar_l r_l = R_l t_l with the plain R_l = P_l^T (about a fifth of Rbar_l's entries).  Same launches as the explicit form.
+   const bool factr = fact0 && o.factor_restriction;
    for (int l = 0; l < last_r; l++) {
       if (fact0 && l == 0) {
          enq_spmv(c, c->A[0], true, c->r[0], c->t[0], epi(-1.0, 1.0, c->r[0]), false);        // t_0
          enq_spmv(c, c->R[0], false, c->t[0], c->r[1], epi(1.0, 0.0, nullptr), false);       // r_1 = R_0 t_0
+      } else if (factr) {
+         const double *rs = (o.smoother == AMGB_SMOOTH_L1_JACOBI) ? c->inv_l1[l] : c->ws[l];
+         c->launches += launch_spmv(c->cfg, c->stream, c->A[l], true, c->r[l], c->t[l], epi(-1.0, 1.0, c->r[l]), nullptr, nullptr,
+                                    nullptr, c->e[l], rs);                                     // t_l and e_l
+         enq_spmv(c, c->R[l], false, c->t[l], c->r[l + 1], epi(1.0, 0.0, nullptr), false);   // r_{l+1} = R_l t_l
       } else enq_spmv(c, c->R[l], false, c->r[l], c->r[l + 1], epi(1.0, 0.0, nullptr), false);
    }
    // per-level corrections e_l (levels are independent)
    const int top = (bpx || direct) ? L : L - 1;  // BPX also smooths the coarsest level (:217-236)
    for (int l = 0; l < top; l++) {
       if (fact0 && l == 0) continue;                  // e_0 is folded into the last launch of the cycle
+      if (factr && l < last_r) continue;              // e_l came with t_l
       if (direct && l == L - 1) enq_spmv(c, c->Ainv, false, c->r[l], c->e[l], epi(1.0, 0.0, nullptr), false);
       else if (multadd) enq_smooth_zero(c, l, c->r[l], c->e[l], o.num_fine_smooth_sweeps, c->symmetric, false, c->t[l], c->w[l]);
       else if (bpx) enq_smooth_zero(c, l, c->r[l], c->e[l], o.num_pre_smooth_sweeps, false, true, c->t[l], c->w[l]);
@@ -1231,6 +1245,7 @@ int amgb_async_dist_correct(amgb_ctx *c, int level)
    const amgb_options &o = c->opt;
    if (o.solver != AMGB_SOLVER_MULTADD || (o.smoother != AMGB_SMOOTH_JACOBI && o.smoother != AMGB_SMOOTH_L1_JACOBI))
       return amgb_fail(c, AMGB_EINVAL, "the cross-GPU asynchronous solve runs Multadd with (L1-)Jacobi smoothing");
+   if (o.factor_restriction) return amgb_fail(c, AMGB_EINVAL, "the cross-GPU asynchronous solve reads the explicit Rbar_l (factor_restriction = 0)");
    if (level == L - 1 && L > 1) return AMGB_OK;           // SMEM convention: the coarsest level contributes nothing
    double *ul = c->u_outer;                                // private copy of the solution (level_vector[k].u)
    CUDA_OK(c, cudaMemcpyAsync(ul, c->u, sizeof(double) * n0, cudaMemcpyDeviceToDevice, c->stream));
@@ -1440,14 +1455,19 @@ int amgb_time_spmv(amgb_ctx *c, int kind, int level, int use_sval, int reps, dou
    if (level < 0 || level >= c->L || (kind != AMGB_MAT_A && level >= c->L - 1) || reps < 1 || !ms_per_launch)
       return amgb_fail(c, AMGB_EINVAL, "bad arguments");
    const DevCSR &M = kind == AMGB_MAT_A ? c->A[level] : (kind == AMGB_MAT_P ? c->P[level] : c->R[level]);
+   if (use_sval < 0 || use_sval > 3 || (use_sval > 1 && kind != AMGB_MAT_A)) return amgb_fail(c, AMGB_EINVAL, "bad arguments");
    if (use_sval && !M.sval && !M.sell_sval) return amgb_fail(c, AMGB_EINVAL, "no scaled values for this matrix");
    const double *x = kind == AMGB_MAT_A ? c->r[level] : (kind == AMGB_MAT_P ? c->e[level + 1] : c->r[level]);
    double *y = kind == AMGB_MAT_A ? c->e[level] : (kind == AMGB_MAT_P ? c->t[level] : c->t[level + 1]);
+   const double *rs = (c->opt.smoother == AMGB_SMOOTH_L1_JACOBI) ? c->inv_l1[level] : c->ws[level];
+   // 2: the symmetrised smoother's pass as the explicit cycle launches it; 3: the factorised restriction's pass (t and e)
+   const SpmvEpilogue e = use_sval == 2 ? epi(-1.0, 2.0, x, 0.0, nullptr, rs) : (use_sval == 3 ? epi(-1.0, 1.0, x) : epi(1.0, 0.0, nullptr));
+   double *y1 = use_sval == 3 ? c->t[level] : y, *y2 = use_sval == 3 ? c->e[level] : nullptr;
    int grid;
-   for (int k = 0; k < 3; k++) c->launches += launch_spmv(c->cfg, c->stream, M, use_sval != 0, x, y, epi(1.0, 0.0, nullptr), nullptr, &grid);
+   for (int k = 0; k < 3; k++) c->launches += launch_spmv(c->cfg, c->stream, M, use_sval != 0, x, y1, e, nullptr, &grid, nullptr, y2, rs);
    CUDA_OK(c, cudaStreamSynchronize(c->stream));
    CUDA_OK(c, cudaEventRecord(c->ev0, c->stream));
-   for (int k = 0; k < reps; k++) c->launches += launch_spmv(c->cfg, c->stream, M, use_sval != 0, x, y, epi(1.0, 0.0, nullptr), nullptr, &grid);
+   for (int k = 0; k < reps; k++) c->launches += launch_spmv(c->cfg, c->stream, M, use_sval != 0, x, y1, e, nullptr, &grid, nullptr, y2, rs);
    CUDA_OK(c, cudaEventRecord(c->ev1, c->stream));
    CUDA_OK(c, cudaEventSynchronize(c->ev1));
    float ms = 0;

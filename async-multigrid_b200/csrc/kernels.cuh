@@ -21,14 +21,17 @@ __device__ __forceinline__ double ld_x(const double *p)
 // DOT (stand-alone kernels): the fused per-CTA sum of a launch that wants one is sum_i y_i * dw_i instead of sum_i y_i^2 (the
 // dot products of the conjugate-gradient solve, pcg.cu).  It is written inline at every row store: routed through a helper
 // or a field of SpmvEpilogue, it changed the persistent kernel's spills although that kernel never takes the DOT path.
+// DUAL (stand-alone kernels, the same way): a second output y2_i = s2_i * (b_i + y_i) beside y_i.  With the column-scaled
+// values and y = b - (A diag(s)) b, y is the t_l of the factorised restriction Rbar_l b = P_l^T t_l and y2 the symmetrised
+// smoother's e_l = s o (2b - (A diag(s)) b): one pass over A_l serves both (amgb_options.factor_restriction).
 
 // ---- CSR, LPR lanes per row (vector-per-row; LPR = 32 is warp-per-row) --------------------------
 // reference loop: src/SMEM_MatVec.cpp:316-322 (+ the epilogues listed in common.cuh)
-template <int LPR, bool RO, bool SVAL, bool DOT = false>
+template <int LPR, bool RO, bool SVAL, bool DOT = false, bool DUAL = false>
 __device__ __forceinline__ double csr_rows_team(const DevCSR &M, const double *__restrict__ x,
                                                 double *y, const SpmvEpilogue &e,
                                                 int team_tid, int team_size, bool want_sumsq,
-                                                const double *dw = nullptr)
+                                                const double *dw = nullptr, double *y2 = nullptr, const double *s2 = nullptr)
 {
    const int lane = team_tid & (LPR - 1);
    constexpr int RPW = 32 / LPR;                       // rows per warp and iteration
@@ -47,6 +50,7 @@ __device__ __forceinline__ double csr_rows_team(const DevCSR &M, const double *_
          double v = epilogue_apply<RO>(e, row, acc);
          epilogue_store<RO>(e, y, row, v);
          if (want_sumsq) sumsq += DOT ? v * __ldg(dw + row) : v * v;
+         if (DUAL) y2[row] = __ldg(s2 + row) * (e.b[row] + v);
       }
    }
    return sumsq;
@@ -64,10 +68,11 @@ __device__ __forceinline__ double csr_rows_team(const DevCSR &M, const double *_
 //          (profiles/README.md R2.3): it is bound by instruction issue and by the number of resident warps, not by HBM --
 //          a variant with every value and the epilogue operands held in registers (80 registers, 3 CTAs/SM) was SLOWER
 //          (0.226 ms against 0.19) than the generic loop at 56 registers; so this path is written for <= 40 registers.
-template <bool RO, bool SVAL, int SU = 0, bool FAST = false, bool DOT = false>
+template <bool RO, bool SVAL, int SU = 0, bool FAST = false, bool DOT = false, bool DUAL = false>
 __device__ __forceinline__ double sell_rows_team(const DevCSR &M, const double *__restrict__ x,
                                                  double *y, const SpmvEpilogue &e,
-                                                 int team_tid, int team_size, bool want_sumsq, const double *dw = nullptr)
+                                                 int team_tid, int team_size, bool want_sumsq, const double *dw = nullptr,
+                                                 double *y2 = nullptr, const double *s2 = nullptr)
 {
    const int lane = team_tid & 31;
    const int nwarp = team_size >> 5;
@@ -110,6 +115,7 @@ __device__ __forceinline__ double sell_rows_team(const DevCSR &M, const double *
          const double v = epilogue_apply<RO>(e, row, acc);
          epilogue_store<RO>(e, y, row, v);
          if (want_sumsq) sumsq += DOT ? v * __ldg(dw + row) : v * v;
+         if (DUAL) y2[row] = __ldg(s2 + row) * (e.b[row] + v);
       } else if (SU > 0 && dsc.y > 0) {
          const double *__restrict__ gv = SVAL ? M.su_sval : M.su_va;
          const bool ok = row < M.nrows;
@@ -136,6 +142,7 @@ __device__ __forceinline__ double sell_rows_team(const DevCSR &M, const double *
             const double v = PRELOAD ? epilogue_finish(e, ops, acc) : epilogue_apply<RO>(e, row, acc);
             epilogue_store<RO>(e, y, row, v);
             if (want_sumsq) sumsq += DOT ? v * __ldg(dw + row) : v * v;
+            if (DUAL) y2[row] = __ldg(s2 + row) * (e.b[row] + v);
          }
       } else {
          const int off = __ldg(M.sell_off + sl);
@@ -148,6 +155,7 @@ __device__ __forceinline__ double sell_rows_team(const DevCSR &M, const double *
             double v = epilogue_apply<RO>(e, row, acc);
             epilogue_store<RO>(e, y, row, v);
             if (want_sumsq) sumsq += DOT ? v * __ldg(dw + row) : v * v;
+            if (DUAL) y2[row] = __ldg(s2 + row) * (e.b[row] + v);
          }
       }
       dsc = dnext;
@@ -169,11 +177,11 @@ __device__ __forceinline__ double sell_rows_team(const DevCSR &M, const double *
 __host__ __device__ constexpr int stream_stage_bytes(int cap, int xcap) { return cap * 12 + xcap * 8; }
 __host__ __device__ constexpr int stream_smem_bytes(int cap, int xcap, int st) { return st * stream_stage_bytes(cap, xcap) + 64; }
 
-template <bool RO, bool SVAL, int NT, int CAP, int XCAP, int ST, bool DOT = false>
+template <bool RO, bool SVAL, int NT, int CAP, int XCAP, int ST, bool DOT = false, bool DUAL = false>
 __device__ __forceinline__ double stream_rows_team(const DevCSR &M, const double *__restrict__ x, double *y,
                                                    const SpmvEpilogue &e, int team_cta, int team_nctas,
                                                    unsigned char *smem, bool want_sumsq, const int4 *blk, int nblk,
-                                                   const double *dw = nullptr)
+                                                   const double *dw = nullptr, double *y2 = nullptr, const double *s2 = nullptr)
 {
    constexpr int SB = stream_stage_bytes(CAP, XCAP);
    constexpr int EPT = CAP / NT;                      // entries per thread
@@ -259,6 +267,7 @@ __device__ __forceinline__ double stream_rows_team(const DevCSR &M, const double
             const double v = epilogue_apply<RO>(e, r0, acc);
             y[r0] = v;
             if (want_sumsq) sumsq += DOT ? v * __ldg(dw + r0) : v * v;
+            if (DUAL) y2[r0] = __ldg(s2 + r0) * (e.b[r0] + v);
          }
          __syncthreads();
       } else {
@@ -316,6 +325,7 @@ __device__ __forceinline__ double stream_rows_team(const DevCSR &M, const double
                const double v = epilogue_finish(e, o_a, acc);
                y[row_a] = v;
                if (want_sumsq) sumsq += DOT ? v * __ldg(dw + row_a) : v * v;
+               if (DUAL) y2[row_a] = __ldg(s2 + row_a) * (e.b[row_a] + v);
             }
          }
          for (int base = rows_per_pass; base < nr; base += rows_per_pass) {   // only when lpr == 1
@@ -327,6 +337,7 @@ __device__ __forceinline__ double stream_rows_team(const DevCSR &M, const double
                const double v = epilogue_apply<RO>(e, row, acc);
                y[row] = v;
                if (want_sumsq) sumsq += DOT ? v * __ldg(dw + row) : v * v;
+               if (DUAL) y2[row] = __ldg(s2 + row) * (e.b[row] + v);
             }
          }
          __syncthreads();                              // the stage is free again
@@ -353,10 +364,11 @@ __device__ __forceinline__ double stream_rows_team(const DevCSR &M, const double
 // for each other, so the load / gather / reduce phases of the 32-64 resident warps of an SM overlap
 // freely -- the CTA-synchronous variant above spends ~20 % of its issue slots in barrier stalls and ~45 %
 // waiting on gathers with only 3-5 CTAs to hide them (profiles/).  swarp: EPT*32 doubles per warp.
-template <bool RO, bool SVAL, int EPT, bool SORTED = false, bool DOT = false>
+template <bool RO, bool SVAL, int EPT, bool SORTED = false, bool DOT = false, bool DUAL = false>
 __device__ __forceinline__ double warp_stream_rows_team(const DevCSR &M, const double *__restrict__ x, double *y,
                                                         const SpmvEpilogue &e, int team_warp, int team_nwarps,
-                                                        double *swarp, bool want_sumsq, const double *dw = nullptr)
+                                                        double *swarp, bool want_sumsq, const double *dw = nullptr,
+                                                        double *y2 = nullptr, const double *s2 = nullptr)
 {
    constexpr int CAP = EPT * 32;
    const int lane = threadIdx.x & 31;
@@ -375,6 +387,7 @@ __device__ __forceinline__ double warp_stream_rows_team(const DevCSR &M, const d
             const double v = epilogue_apply<RO>(e, r0, acc);
             y[r0] = v;
             if (want_sumsq) sumsq += DOT ? v * __ldg(dw + r0) : v * v;
+            if (DUAL) y2[r0] = __ldg(s2 + r0) * (e.b[r0] + v);
          }
          continue;
       }
@@ -426,6 +439,7 @@ __device__ __forceinline__ double warp_stream_rows_team(const DevCSR &M, const d
             const double v = epilogue_finish(e, o_a, acc);
             y[row_a] = v;
             if (want_sumsq) sumsq += DOT ? v * __ldg(dw + row_a) : v * v;
+            if (DUAL) y2[row_a] = __ldg(s2 + row_a) * (e.b[row_a] + v);
          }
       }
       for (int base = 32; base < nr; base += 32) {     // only when lpr == 1
@@ -437,6 +451,7 @@ __device__ __forceinline__ double warp_stream_rows_team(const DevCSR &M, const d
             const double v = epilogue_apply<RO>(e, row, acc);
             y[row] = v;
             if (want_sumsq) sumsq += DOT ? v * __ldg(dw + row) : v * v;
+            if (DUAL) y2[row] = __ldg(s2 + row) * (e.b[row] + v);
          }
       }
    }
@@ -444,16 +459,17 @@ __device__ __forceinline__ double warp_stream_rows_team(const DevCSR &M, const d
 }
 
 // vector-per-row CSR with the lanes-per-row chosen at upload time
-template <bool RO, bool SVAL, bool DOT = false>
+template <bool RO, bool SVAL, bool DOT = false, bool DUAL = false>
 __device__ __forceinline__ double csr_rows_dispatch(const DevCSR &M, const double *x, double *y, const SpmvEpilogue &e,
-                                                    int team_tid, int team_size, bool want_sumsq, const double *dw = nullptr)
+                                                    int team_tid, int team_size, bool want_sumsq, const double *dw = nullptr,
+                                                 double *y2 = nullptr, const double *s2 = nullptr)
 {
    switch (M.lpr) {
-      case 2: return csr_rows_team<2, RO, SVAL, DOT>(M, x, y, e, team_tid, team_size, want_sumsq, dw);
-      case 4: return csr_rows_team<4, RO, SVAL, DOT>(M, x, y, e, team_tid, team_size, want_sumsq, dw);
-      case 8: return csr_rows_team<8, RO, SVAL, DOT>(M, x, y, e, team_tid, team_size, want_sumsq, dw);
-      case 16: return csr_rows_team<16, RO, SVAL, DOT>(M, x, y, e, team_tid, team_size, want_sumsq, dw);
-      default: return csr_rows_team<32, RO, SVAL, DOT>(M, x, y, e, team_tid, team_size, want_sumsq, dw);
+      case 2: return csr_rows_team<2, RO, SVAL, DOT, DUAL>(M, x, y, e, team_tid, team_size, want_sumsq, dw, y2, s2);
+      case 4: return csr_rows_team<4, RO, SVAL, DOT, DUAL>(M, x, y, e, team_tid, team_size, want_sumsq, dw, y2, s2);
+      case 8: return csr_rows_team<8, RO, SVAL, DOT, DUAL>(M, x, y, e, team_tid, team_size, want_sumsq, dw, y2, s2);
+      case 16: return csr_rows_team<16, RO, SVAL, DOT, DUAL>(M, x, y, e, team_tid, team_size, want_sumsq, dw, y2, s2);
+      default: return csr_rows_team<32, RO, SVAL, DOT, DUAL>(M, x, y, e, team_tid, team_size, want_sumsq, dw, y2, s2);
    }
 }
 

@@ -27,9 +27,11 @@ static const StreamVariant kStreamVariants[AMGB_NUM_STREAM_VARIANTS] = {
 };
 
 // y = gamma*c + rs.*(beta*b + alpha*M*x); optional sum of y_i^2 -- or of y_i*dot_w_i when dot_w is given -- into partial
-// sums (one per CTA, `partials` must hold >= grid entries; *grid_out receives the grid used).
+// sums (one per CTA, `partials` must hold >= grid entries; *grid_out receives the grid used).  y2 != nullptr: the
+// column-scaled values, a second output y2 = s2 .* (b + y), no partial sums (the factorised restriction's pass over A_l).
 int launch_spmv(const LaunchCfg &cfg, cudaStream_t st, const DevCSR &M, bool use_sval, const double *x, double *y,
-                const SpmvEpilogue &e, double *partials, int *grid_out, const double *dot_w = nullptr);
+                const SpmvEpilogue &e, double *partials, int *grid_out, const double *dot_w = nullptr, double *y2 = nullptr,
+                const double *s2 = nullptr);
 int spmv_units(const DevCSR &M);
 int launch_spmv_units(const LaunchCfg &cfg, cudaStream_t st, const DevCSR &M, int u0, int u1, bool use_sval, const double *x,
                       double *y, const SpmvEpilogue &e, double *partials, int *grid_out, const double *dot_w = nullptr);

@@ -90,7 +90,7 @@ def _build_and_scatter(args, world, d, dims):
     b = H.rand_rhs(A.nrows)
     info = {"levels": h.num_levels, "n": [int(x) for x in h.n], "nnz_A": [int(a.nnz) for a in h.A],
             "operator_complexity": round(h.operator_complexity(), 3),
-            "bytes_per_cycle": int(H.bytes_sync_multadd_cycle_factored(h) if fact0 else H.bytes_sync_multadd_cycle(h, args.num_post > 0)),
+            "bytes_per_cycle": int(H.bytes_sync_multadd_cycle_factored(h, factor_restriction=False) if fact0 else H.bytes_sync_multadd_cycle(h, args.num_post > 0)),
             "host_setup_s": round(time.time() - t0, 1)}
     _log("[bench] global hierarchy %dx%dx%d: %d levels, n=%s, host setup %.1fs" % (nx, ny, nz, h.num_levels, h.n, time.time() - t0))
     starts, num_dist, halos = PT.plan_layouts(h, world, plane=nx * ny, min_rows_per_rank=args.min_rows_per_rank)

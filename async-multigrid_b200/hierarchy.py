@@ -353,6 +353,7 @@ class Hierarchy:
         self.n = [a.nrows for a in A]
         self.P = None
         self.R = None
+        self.R_plain = [None] * (len(A) - 1)     # P_l^T, built on demand (plain_restriction)
         self.smooth_weight = None
         self.l1 = None
         self.cpts = None      # cpts[l][j]: level-l index of coarse point j of level l+1 (row partitions follow it)
@@ -379,6 +380,13 @@ class Hierarchy:
                 self.P.append(self.P_plain[l])
                 self.R.append(self._transpose(self.P_plain[l]))
         return self
+
+    def plain_restriction(self, l):
+        """P_l^T from the plain interpolation, built once and kept: what amgb_options.factor_restriction uploads as R_l for
+        l >= 1 (the explicit products in self.R stay for the other solvers)"""
+        if self.R_plain[l] is None:
+            self.R_plain[l] = self._transpose(self.P_plain[l])
+        return self.R_plain[l]
 
     @staticmethod
     def _transpose(p):
@@ -595,9 +603,17 @@ def bytes_sync_multadd_cycle(h, symmetric=True):
     return tot
 
 
-def bytes_sync_multadd_cycle_factored(h):
+def bytes_plain_restriction(p):
+    """bytes_spmv(P^T, False) from the interpolation P itself, without forming the transpose"""
+    return 12 * p.nnz + 4 * (p.ncols + 1) + 8 * p.nrows + 8 * p.ncols
+
+
+def bytes_sync_multadd_cycle_factored(h, factor_restriction=True):
     """the same cycle with the level-0 transfers in factorised form (amgb_options.factor_level0; h.P[0] / h.R[0] plain):
-    residual on A_0, t_0 pass on A_0 (reads r_0, writes t_0), R_0, P_0, final pass on A_0 (reads v, r_0, t_0, w/d, u; writes u)"""
+    residual on A_0, t_0 pass on A_0 (reads r_0, writes t_0), R_0, P_0, final pass on A_0 (reads v, r_0, t_0, w/d, u; writes u).
+    factor_restriction (amgb_options.factor_restriction, the single-GPU default): on the levels l >= 1 the plain P_l^T
+    replaces Rbar_l and the smoother's pass over A_l also stores t_l (8 n_l); False: the explicit h.R[l] (the partitioned
+    multi-GPU cycle).  As in bytes_sync_multadd_cycle, every level below the coarsest counts one restriction."""
     L = h.num_levels
     n0 = h.n[0]
     tot = bytes_spmv(h.A[0], True)                                  # r = f - A u
@@ -605,7 +621,8 @@ def bytes_sync_multadd_cycle_factored(h):
     tot += bytes_spmv(h.R[0], False) + bytes_spmv(h.P[0], False)    # plain transfers
     tot += bytes_spmv(h.A[0], True) + 3 * 8 * n0                    # u += v + (w/d) o (r_0 + t_0 - A_0 v): extra reads t_0, w/d, u
     for l in range(1, L - 1):                                       # coarser levels as in bytes_sync_multadd_cycle
-        tot += bytes_spmv(h.R[l], False) + bytes_spmv(h.A[l], False) + 8 * h.n[l] + bytes_spmv(h.P[l], True)
+        rb = bytes_plain_restriction(h.P_plain[l]) + 8 * h.n[l] if factor_restriction else bytes_spmv(h.R[l], False)
+        tot += rb + bytes_spmv(h.A[l], False) + 8 * h.n[l] + bytes_spmv(h.P[l], True)
     return tot
 
 

@@ -43,7 +43,7 @@ class Options(C.Structure):
                 ("jgs_block_rows", C.c_int), ("use_sell", C.c_int), ("l2_persist", C.c_int), ("use_stream", C.c_int),
                 ("factor_level0", C.c_int), ("coarse_solve", C.c_int), ("sell_sigma", C.c_int), ("stream_variant", C.c_int),
                 ("sell_uniform", C.c_int), ("async_type", C.c_int), ("res_compute_type", C.c_int), ("read_type", C.c_int),
-                ("lean_storage", C.c_int)]
+                ("lean_storage", C.c_int), ("factor_restriction", C.c_int)]
 
 
 class HostCSR(C.Structure):
@@ -154,7 +154,10 @@ class Solver:
     def __init__(self, h, solver=H.MULTADD, smoother=H.JACOBI, smooth_weight=1.0, num_pre=1, num_post=1,
                  fine_sweeps=1, coarse_sweeps=1, jgs_block_rows=8, use_sell=True, l2_persist=True, use_stream=True,
                  stream_variant=None, sell_sigma=None, coarse_solve=False, factor_level0=False, device=0, jgs_blocks=None,
-                 sell_uniform=None, async_type=0, res_compute_type=0, read_type=0, lean_storage=False):
+                 sell_uniform=None, async_type=0, res_compute_type=0, read_type=0, lean_storage=False, factor_restriction=None):
+        """factor_restriction (amgb_options.factor_restriction): None = on exactly where amgb_setup accepts it, i.e. with
+        factor_level0 for the synchronous Multadd cycle with the symmetrised (L1-)Jacobi smoother and one fine sweep; the
+        plain P_l^T (Hierarchy.plain_restriction) is then uploaded for the levels l >= 1 in place of h.R[l], which stays as it is"""
         self.L = load_library()
         self.h = h
         self.ctx = C.c_void_p()
@@ -186,6 +189,10 @@ class Solver:
             o.sell_uniform = int(os.environ["AMGB_SELL_UNIFORM"])
         o.async_type, o.res_compute_type, o.read_type = int(async_type), int(res_compute_type), int(read_type)
         o.lean_storage = int(lean_storage)
+        if factor_restriction is None:
+            factor_restriction = (factor_level0 and solver == H.MULTADD and smoother in (H.JACOBI, H.L1_JACOBI) and num_pre > 0
+                                  and num_post > 0 and fine_sweeps == 1)
+        o.factor_restriction = int(factor_restriction)
         self.options = o
         self._ck(self.L.amgb_set_options(self.ctx, C.byref(o)))
         self._ck(self.L.amgb_set_num_levels(self.ctx, h.num_levels))
@@ -193,7 +200,7 @@ class Solver:
             self._set(MAT_A, l, h.A[l])
             if l < h.num_levels - 1:
                 self._set(MAT_P, l, h.P[l])
-                self._set(MAT_R, l, h.R[l])
+                self._set(MAT_R, l, h.plain_restriction(l) if factor_restriction and l >= 1 else h.R[l])
         self._ck(self.L.amgb_setup(self.ctx))
         self.n0 = h.n[0]
         if jgs_blocks is not None:

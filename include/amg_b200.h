@@ -83,6 +83,12 @@ typedef struct {
    int lean_storage;            /* 1: a matrix stored as sliced ELL keeps no second (CSR) copy in HBM -- what lets the 512^3 hierarchy
                                    (2.7 G entries in the A_l alone) fit one 180 GB GPU.  (L1-)Jacobi smoothers only; the transposed
                                    product is then unavailable for those matrices.  0 (default): both copies */
+   int factor_restriction;      /* 1 (with factor_level0; synchronous Multadd, symmetrised (L1-)Jacobi smoother, num_fine_smooth_sweeps = 1,
+                                   one GPU): the restrictions R_l of the levels l >= 1 the cycle restricts from are uploaded PLAIN (P_l^T)
+                                   too, and Rbar_l r = P_l^T (r - A_l diag(s) r) (s = w/d, or 1/l1) is applied on the fly: the pass over
+                                   A_l that the level's smoother makes anyway writes t_l = r_l - A_l diag(s) r_l beside e_l = s o (r_l + t_l),
+                                   then r_{l+1} = R_l t_l.  P_l stay the explicit Pbar_l.  Same operator, rounding-level differences;
+                                   AMGB_EINVAL from amgb_setup where the algebra does not hold.  0 (default): explicit Rbar_l */
 } amgb_options;
 
 void amgb_default_options(amgb_options *opt);
@@ -251,7 +257,9 @@ void amgb_host_csr_free(amgb_host_csr *m);
  * r = f - A_0 u (the dominant kernel), on the context's stream */
 int amgb_time_residual(amgb_ctx *ctx, int reps, double *ms_per_launch);
 int amgb_level_storage(amgb_ctx *ctx, int kind, int level, int *is_sell);
-/* event-timed y = M x for one matrix of the hierarchy (tools/spmv_sweep.py) and CSR-stream block statistics */
+/* event-timed y = M x for one matrix of the hierarchy (tools/spmv_sweep.py) and CSR-stream block statistics.  use_scaled_values:
+ * 0 the values, 1 the column-scaled values; A_l only: 2 the symmetrised smoother's pass e = s o (2x - (A diag(s)) x) of the
+ * explicit cycle, 3 the factorised restriction's pass t = x - (A diag(s)) x, e = s o (x + t) (amgb_options.factor_restriction) */
 int amgb_time_spmv(amgb_ctx *ctx, int kind, int level, int use_scaled_values, int reps, double *ms_per_launch);
 int amgb_stream_stats(amgb_ctx *ctx, long long *blocks, long long *blocks_with_staged_x);
 /* slices stored in the SELL-U encoding (amgb_options.sell_uniform) and their (delta, mask, value) groups */

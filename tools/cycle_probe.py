@@ -3,7 +3,7 @@
 builds the hierarchy, runs `--cycles` cycles and prints the event-timed SpMV of every large operator against its
 algorithmic bytes (SURVEY.md 8d).  Under ncu this is the command whose launch list / --set full capture goes to profiles/.
 
-    python tools/cycle_probe.py --n 256 --cycles 2 [--explicit] [--problem 27pt]"""
+    python tools/cycle_probe.py --n 256 --cycles 2 [--explicit] [--no-factor-restriction] [--problem 27pt]"""
 import argparse
 import json
 import os
@@ -23,6 +23,8 @@ def main():
     ap.add_argument("--cycles", type=int, default=2)
     ap.add_argument("--w", type=float, default=0.9)
     ap.add_argument("--explicit", action="store_true", help="explicit Pbar_0 / Rbar_0 instead of the factorised level-0 transfers")
+    ap.add_argument("--no-factor-restriction", action="store_true",
+                    help="explicit Rbar_l on the levels l >= 1 instead of the factorised restriction (amgb_options.factor_restriction)")
     ap.add_argument("--time-ops", action="store_true", help="event-time every large operator (skip under ncu)")
     ap.add_argument("--peak", type=float, default=6555.5)
     a = ap.parse_args()
@@ -33,7 +35,7 @@ def main():
     h.build_transfers(H.MULTADD, a.w, factor_level0=fact)
     b = H.rand_rhs(A.nrows)
     host_s = time.time() - t0
-    s = amg.Solver(h, H.MULTADD, H.JACOBI, a.w, factor_level0=fact)
+    s = amg.Solver(h, H.MULTADD, H.JACOBI, a.w, factor_level0=fact, factor_restriction=False if a.no_factor_restriction else None)
     s.set_rhs(b)
     s.set_solution(None)
     hist, secs = s.solve_sync(1e-300, a.cycles)
