@@ -1,7 +1,6 @@
 // common.cuh -- shared device helpers for the sm_100a additive-AMG kernels.
 #pragma once
 #include <cuda_runtime.h>
-#include <stdint.h>
 
 #define AMGB_WARP 32
 #define AMGB_FULL 0xffffffffu
@@ -36,31 +35,15 @@ struct DevCSR {
    const double *su_va = nullptr;
    const double *su_sval = nullptr;
    int lpr = 8;                      // lanes per row chosen for the CSR vector kernel
-   // CSR-stream row blocks: CTA b owns rows [blk[b], blk[b+1]) whose entries (<= AMGB_STREAM_CAP,
-   // counted from the 4-aligned start) are streamed with 128-bit loads into shared memory and then
-   // reduced per row; a block made of ONE longer row is reduced by the whole CTA.
+   // warp-stream row chunks (warp_stream_rows_team): consecutive rows whose entries fit AMGB_WARP_CHUNK; a row longer
+   // than that is a chunk of its own, reduced by the whole warp.  Also the launch units of the multi-GPU interior split.
    int nblk = 0;
-   const int4 *blk = nullptr;        // per block {first row, end row, first entry, end entry}
-   // staged-x form of a block: the columns its entries touch are covered by <= 32 contiguous windows of x
-   // (total <= AMGB_STREAM_XCAP entries) that are bulk-copied into shared memory next to the block; `li`
-   // then holds, per entry, the 16-bit position of its column inside that window buffer.
-   const int4 *blkx = nullptr;       // per block {offset into win, #windows (0 = gather from global memory), 0, 0}
-   const int2 *win = nullptr;        // {first column (even), length (even)} per window
-   const unsigned short *li = nullptr;
-   int wept = 0;                     // > 0: the blocks are WARP chunks of <= 32*wept entries (warp_stream_rows_team)
-   // column-sorted copy of the warp chunks (wept > 0, DevCSR::pos != nullptr): inside every chunk the entries
-   // are stored in ascending column order (pci / pva / psval) and pos[k] is the entry's original position
-   // within the chunk, so consecutive lanes gather neighbouring x (few L1 tag look-ups per instruction) and
-   // the products are scattered back to row order in shared memory.
-   const int *pci = nullptr;
-   const double *pva = nullptr;
-   const double *psval = nullptr;
-   const unsigned char *pos = nullptr;
+   const int4 *blk = nullptr;        // per chunk {first row, end row, first entry, end entry}
    // multi-GPU: launch units (slices / chunks / rows) [ulo, uhi) read only OWNED entries of the input vector, so
    // they can run while the halo exchange is in flight; the units outside wait for it.  uhi <= ulo: no split.
    int ulo = 0, uhi = 0;
 };
-#define AMGB_STREAM_CAP 2048          // largest row block any variant uses (and the persistent kernel's)
+#define AMGB_WARP_CHUNK 256           // largest warp-stream chunk, in entries (8 per lane)
 
 // y_i = gamma*c_i + rs_i * (beta*b_i + alpha * sum_j M_ij x_j)       (rs == nullptr -> 1)
 // covers: MatVec (alpha=1), Residual (alpha=-1,beta=1,b=f), prolong-and-add (beta=1,b=y),
@@ -99,25 +82,6 @@ __device__ __forceinline__ int ld_stream(const int *p)
    asm volatile("ld.global.nc.L1::no_allocate.s32 %0, [%1];" : "=r"(v) : "l"(p));
    return v;
 }
-__device__ __forceinline__ int ld_stream(const unsigned char *p)
-{
-   unsigned int v;
-   asm volatile("ld.global.nc.L1::no_allocate.u8 %0, [%1];" : "=r"(v) : "l"(p));
-   return (int)v;
-}
-// 128-bit streaming loads (4 column indices / 2 values per instruction), 16-byte aligned
-__device__ __forceinline__ int4 ld_stream4(const int *p)
-{
-   int4 v;
-   asm volatile("ld.global.nc.L1::no_allocate.v4.s32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p));
-   return v;
-}
-__device__ __forceinline__ double2 ld_stream2(const double *p)
-{
-   double2 v;
-   asm volatile("ld.global.nc.L1::no_allocate.v2.f64 {%0,%1}, [%2];" : "=d"(v.x), "=d"(v.y) : "l"(p));
-   return v;
-}
 // coherent (L2) load for vectors that other CTA groups update concurrently inside the persistent
 // asynchronous kernel
 __device__ __forceinline__ double ld_cg(const double *p)
@@ -142,48 +106,6 @@ __device__ __forceinline__ void st_cg(double *p, double v)
 __device__ __forceinline__ void red_add_f64(double *p, double v)
 {
    asm volatile("red.global.add.f64 [%0], %1;" ::"l"(p), "d"(v) : "memory");
-}
-
-// ---- TMA bulk copy + mbarrier (sm_90+/sm_100a): global -> shared without register staging -----------
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count)
-{
-   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_inval(uint32_t bar) { asm volatile("mbarrier.inval.shared::cta.b64 [%0];" ::"r"(bar) : "memory"); }
-__device__ __forceinline__ void mbar_init_fence() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes)
-{
-   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity)
-{
-   uint32_t done;
-   do {
-      asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                   : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-   } while (!done);
-}
-// generic-proxy accesses to shared memory (the in-place products) are ordered before the next bulk copy
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ uint64_t l2_evict_first_policy()
-{
-   uint64_t pol;
-   asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-   return pol;
-}
-__device__ __forceinline__ uint64_t l2_evict_last_policy()
-{
-   uint64_t pol;
-   asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
-   return pol;
-}
-// bytes: multiple of 16; src and dst 16-byte aligned.  The matrix streams are read once: evict_first keeps
-// the gathered vectors resident in L2.
-__device__ __forceinline__ void tma_bulk_g2s(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar, uint64_t pol)
-{
-   asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;"
-                ::"r"(dst), "l"(src), "r"(bytes), "r"(bar), "l"(pol) : "memory");
 }
 
 template <int W>

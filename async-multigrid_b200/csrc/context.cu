@@ -120,7 +120,6 @@ int amgb_create(amgb_ctx **out, int device)
    cudaGetDeviceProperties(&prop, device);
    c->cfg.num_sms = prop.multiProcessorCount;
    c->cfg.ctas_per_sm = 8;
-   if (const char *sc = getenv("AMGB_SELLU_CTAS")) c->cfg.sellu_ctas = (atoi(sc) == 4 || atoi(sc) == 6 || atoi(sc) == 8) ? atoi(sc) : 5;      // 8: the generic batch-of-8 loop
    c->host_threads = std::max(1, std::min(16, omp_get_num_procs()));
    c->l2_bytes = prop.l2CacheSize;
    c->max_window = prop.accessPolicyMaxWindowSize;
@@ -183,11 +182,11 @@ int amgb_set_num_levels(amgb_ctx *c, int L)
 int amgb_set_options(amgb_ctx *c, const amgb_options *o)
 {
    if (!c || !o) return AMGB_EINVAL;
-   if (o->smooth_weight == 0.0 || o->jgs_block_rows < 1 || o->stream_variant < 0 || o->stream_variant >= AMGB_NUM_STREAM_VARIANTS)
-      return amgb_fail(c, AMGB_EINVAL, "bad options");
+   if (o->smooth_weight == 0.0 || o->jgs_block_rows < 1) return amgb_fail(c, AMGB_EINVAL, "bad options");
+   if (o->stream_variant != 8)
+      return amgb_fail(c, AMGB_EINVAL, "stream_variant %d: the field is retired, only 8 (the warp-stream kernel) is accepted", o->stream_variant);
    if (c->L) return amgb_fail(c, AMGB_ESTATE, "amgb_set_options must precede the hierarchy upload");
    c->opt = *o;
-   c->cfg.stream_variant = o->stream_variant;
    return AMGB_OK;
 }
 
@@ -423,124 +422,26 @@ int amgb_sellu_encode_host(int nrows, const int *rp, const int *ci, const double
 }
 void amgb_host_free(void *p) { free(p); }
 
-// Row blocks of the CSR-stream kernel: consecutive rows whose entries, counted from the 4-aligned
-// start of the block, fit AMGB_STREAM_CAP (and at most AMGB_STREAM_CAP rows); a longer row is a
-// block of its own.
-static int build_stream_blocks(amgb_ctx *c, DevCSR &M, int nrows, int ncols, const int *rp, const int *ci, const double *va)
+// Row chunks of the warp-stream kernel: consecutive rows whose entries fit AMGB_WARP_CHUNK (and at most AMGB_WARP_CHUNK
+// rows); a longer row is a chunk of its own.
+static int build_stream_blocks(amgb_ctx *c, DevCSR &M, int nrows, const int *rp)
 {
-   const StreamVariant &sv = kStreamVariants[c->cfg.stream_variant];
-   const int CAPV = sv.cap, XCAPV = sv.xcap;
    std::vector<int4> blk;
    blk.reserve((size_t)rp[nrows] / 1024 + 16);
    int r = 0;
    while (r < nrows) {
       const int start = r;
-      const long q0 = sv.stages <= 0 ? rp[start] : (rp[start] & ~7);   // bulk copies start 8-entry aligned
-      while (r < nrows && r - start < CAPV && (long)rp[r + 1] - q0 <= CAPV) r++;
+      while (r < nrows && r - start < AMGB_WARP_CHUNK && rp[r + 1] - rp[start] <= AMGB_WARP_CHUNK) r++;
       if (r == start) r++;
       blk.push_back(make_int4(start, r, rp[start], rp[r]));
    }
-   const int nb = (int)blk.size();
    c->last_blk = blk;
-   // x windows per block (see DevCSR): built in parallel, then concatenated
-   std::vector<int4> blkx((size_t)nb, make_int4(0, 0, 0, 0));
-   std::vector<std::vector<int2>> wins((size_t)nb);
-   std::vector<unsigned short> li((size_t)rp[nrows] + 16, 0);
-   long staged = 0;
-#pragma omp parallel reduction(+ : staged)
-   {
-      std::vector<int> u;
-      std::vector<int2> w;
-      std::vector<int> wbase;
-#pragma omp for schedule(dynamic, 64)
-      for (int b = 0; b < nb; b++) {
-         const int p0 = blk[b].z, p1 = blk[b].w;
-         if (XCAPV == 0 || p1 <= p0 || p1 - (p0 & ~7) > CAPV) continue;   // no staging / empty / long-row block
-         u.assign(ci + p0, ci + p1);
-         std::sort(u.begin(), u.end());
-         u.erase(std::unique(u.begin(), u.end()), u.end());
-         bool ok = false;
-         for (int gap = 8; gap <= 512 && !ok; gap *= 4) {
-            w.clear();
-            int ws = u[0] & ~1, we = (u[0] + 2) & ~1;
-            for (size_t k = 1; k < u.size(); k++) {
-               if (u[k] < we + gap) we = (u[k] + 2) & ~1;
-               else { w.push_back(make_int2(ws, we - ws)); ws = u[k] & ~1; we = (u[k] + 2) & ~1; }
-            }
-            w.push_back(make_int2(ws, we - ws));
-            long tot = 0;
-            for (auto &x : w) tot += x.y;
-            if (tot > XCAPV) break;                       // larger gaps only add entries
-            ok = (int)w.size() <= 32;
-         }
-         if (!ok) continue;
-         (void)ncols;   // a window may end one entry past ncols: vectors are allocated with slack
-         wbase.resize(w.size());
-         int acc = 0;
-         for (size_t k = 0; k < w.size(); k++) { wbase[k] = acc; acc += w[k].y; }
-         for (int p = p0; p < p1; p++) {
-            const int col = ci[p];
-            size_t lo = 0, hi = w.size();                 // last window with start <= col
-            while (hi - lo > 1) { size_t mid = (lo + hi) / 2; if (w[mid].x <= col) lo = mid; else hi = mid; }
-            li[p] = (unsigned short)(wbase[lo] + (col - w[lo].x));
-         }
-         wins[b] = w;
-         blkx[b].y = (int)w.size();
-         staged++;
-      }
-   }
-   std::vector<int2> win;
-   for (int b = 0; b < nb; b++) {
-      blkx[b].x = (int)win.size();
-      win.insert(win.end(), wins[b].begin(), wins[b].end());
-   }
-   int4 *d_blk, *d_blkx;
-   int2 *d_win;
-   unsigned short *d_li;
+   int4 *d_blk;
    int rc;
    if ((rc = dev_upload(c, &d_blk, blk.data(), blk.size()))) return rc;
-   if ((rc = dev_upload(c, &d_blkx, blkx.data(), blkx.size()))) return rc;
-   if ((rc = dev_upload(c, &d_win, win.data(), win.size()))) return rc;
-   if ((rc = dev_upload(c, &d_li, li.data(), li.size()))) return rc;
    CUDA_OK(c, cudaStreamSynchronize(c->stream));
-   M.nblk = nb;
-   M.blk = d_blk; M.blkx = d_blkx; M.win = d_win; M.li = d_li;
-   M.wept = sv.stages <= 0 ? sv.cap / 32 : 0;
-   if (sv.stages < 0) {
-      // column-sorted copy of every warp chunk (see DevCSR::pos)
-      const size_t nnz = (size_t)rp[nrows];
-      std::vector<int> pci(nnz);
-      std::vector<double> pva(nnz);
-      std::vector<unsigned char> pos(nnz + 16, 0);
-#pragma omp parallel
-      {
-         std::vector<int> idx;
-#pragma omp for schedule(dynamic, 256)
-         for (int b = 0; b < nb; b++) {
-            const int p0 = blk[b].z, p1 = blk[b].w, cnt = p1 - p0;
-            if (cnt > CAPV || cnt > 256) {      // long row: read unsorted by the whole warp
-               for (int p = p0; p < p1; p++) { pci[p] = ci[p]; pva[p] = va[p]; }
-               continue;
-            }
-            idx.resize(cnt);
-            for (int k = 0; k < cnt; k++) idx[k] = k;
-            std::stable_sort(idx.begin(), idx.end(), [&](int a, int bb) { return ci[p0 + a] < ci[p0 + bb]; });
-            for (int k = 0; k < cnt; k++) {
-               pci[p0 + k] = ci[p0 + idx[k]];
-               pva[p0 + k] = va[p0 + idx[k]];
-               pos[p0 + k] = (unsigned char)idx[k];
-            }
-         }
-      }
-      int *d_pci; double *d_pva; unsigned char *d_pos;
-      if ((rc = dev_upload(c, &d_pci, pci.data(), pci.size()))) return rc;
-      if ((rc = dev_upload(c, &d_pva, pva.data(), pva.size()))) return rc;
-      if ((rc = dev_upload(c, &d_pos, pos.data(), pos.size()))) return rc;
-      CUDA_OK(c, cudaStreamSynchronize(c->stream));
-      M.pci = d_pci; M.pva = d_pva; M.pos = d_pos;
-   }
-   c->stream_blocks += nb;
-   c->stream_blocks_staged_x += staged;
+   M.nblk = (int)blk.size();
+   M.blk = d_blk;
    return AMGB_OK;
 }
 
@@ -612,8 +513,8 @@ int amgb_set_matrix(amgb_ctx *c, int kind, int level, int nrows, int ncols, int 
    // shorter goes through the stream kernel (measured per matrix with tools/spmv_sweep.py, profiles/)
    const bool long_rows = nrows > 0 && (double)nnz / nrows >= 96.0;
    if (long_rows) M.lpr = 32;
-   if (c->opt.use_stream && M.sell_slices == 0 && nrows > 0 && !(long_rows && kStreamVariants[c->opt.stream_variant].stages <= 0)) {
-      if ((rc = build_stream_blocks(c, M, nrows, ncols, rp, ci, va))) return rc;
+   if (c->opt.use_stream && M.sell_slices == 0 && nrows > 0 && !long_rows) {
+      if ((rc = build_stream_blocks(c, M, nrows, rp))) return rc;
    }
    // DMEM convention: dense inverse of the coarsest operator (hypre_GaussElimSetup, src/DMEM_Setup.cpp:385-388),
    // applied later as one full SpMV
@@ -757,12 +658,6 @@ int amgb_setup(amgb_ctx *c)
          if (!part) c->launches += launch_colscale(c->stream, c->A[l].nnz, c->A[l].ci, c->A[l].va, cs, sv);
       }
       c->A[l].sval = sv;
-      if (c->A[l].pos) {   // scaled values of the column-sorted chunk copy
-         double *psv = nullptr;
-         if ((rc = dev_alloc(c, &psv, (size_t)c->A[l].nnz))) return rc;
-         if (!part) c->launches += launch_colscale(c->stream, c->A[l].nnz, c->A[l].pci, c->A[l].pva, cs, psv);
-         c->A[l].psval = psv;
-      }
       if (c->A[l].sell_slices > 0) {
          long pe = c->sell_entries[&c->A[l]];
          double *ssv = nullptr;
@@ -1474,15 +1369,6 @@ int amgb_time_spmv(amgb_ctx *c, int kind, int level, int use_sval, int reps, dou
    cudaEventElapsedTime(&ms, c->ev0, c->ev1);
    *ms_per_launch = ms / reps;
    CUDA_OK(c, cudaGetLastError());
-   return AMGB_OK;
-}
-
-// CSR-stream row blocks over the whole hierarchy and how many of them carry staged x windows
-int amgb_stream_stats(amgb_ctx *c, long long *blocks, long long *blocks_staged_x)
-{
-   if (!c) return AMGB_EINVAL;
-   if (blocks) *blocks = c->stream_blocks;
-   if (blocks_staged_x) *blocks_staged_x = c->stream_blocks_staged_x;
    return AMGB_OK;
 }
 

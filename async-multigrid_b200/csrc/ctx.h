@@ -46,7 +46,6 @@ struct amgb_ctx {
    size_t bytes_allocated = 0;
    int host_threads = 1;   // threads for the upload-time layout conversions (set in amgb_create)
    long sellu_slices = 0, sellu_groups = 0;               // SELL-U: encoded slices / groups over the whole hierarchy
-   long stream_blocks = 0, stream_blocks_staged_x = 0;   // CSR-stream row blocks / those with staged x windows
    size_t l2_bytes = 0, max_window = 0, persist_max = 0;
    std::vector<void *> allocs;
    // async

@@ -343,8 +343,6 @@ int amgb_dist_setup(amgb_ctx *c)
          if ((rc = dist_halo(c, l, d->ws[l]))) return rc;
          if (c->A[l].va)      // (lean storage keeps no CSR copy of a sliced-ELL matrix)
             c->launches += launch_colscale(c->stream, c->A[l].nnz, c->A[l].ci, c->A[l].va, d->ws[l], const_cast<double *>(c->A[l].sval));
-         if (c->A[l].pos)
-            c->launches += launch_colscale(c->stream, c->A[l].nnz, c->A[l].pci, c->A[l].pva, d->ws[l], const_cast<double *>(c->A[l].psval));
          if (c->A[l].sell_slices > 0)
             c->launches += launch_colscale(c->stream, (int)c->sell_entries[&c->A[l]], c->A[l].sell_ci, c->A[l].sell_va, d->ws[l],
                                            const_cast<double *>(c->A[l].sell_sval));

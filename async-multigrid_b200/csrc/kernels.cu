@@ -13,35 +13,20 @@ namespace {
 constexpr int kBlock = 256;
 
 // One kernel per storage scheme (separate register budgets): MODE 0 = vector-per-row CSR, 1 = sliced ELL,
-// 2 (3, 4: other register budgets) = sliced ELL with the SELL-U encoding (stencil levels); the CSR-stream kernel (row blocks through shared memory) is k_spmv_stream.
+// 2 = sliced ELL with the SELL-U encoding (stencil levels); the warp-stream CSR kernel is k_spmv_wstream.
 // DOT: the fused per-CTA partial is sum_i y_i * w_i instead of sum_i y_i^2; DUAL: the second output y2 = s2 o (b + y) (kernels.cuh).
 // Separate instantiations, so that the others keep their registers.
 template <int MODE, bool SVAL, bool DOT = false, bool DUAL = false>
-__global__ void __launch_bounds__(kBlock, MODE == 2 ? 5 : (MODE == 3 ? 4 : (MODE == 4 ? 6 : (MODE == 5 ? 4 : 1)))) k_spmv(DevCSR M, const double *x, double *y, SpmvEpilogue e, double *partials,
-                                                                                                                                          const double *w, double *y2, const double *s2)
+__global__ void __launch_bounds__(kBlock, MODE == 2 ? 5 : 1) k_spmv(DevCSR M, const double *x, double *y, SpmvEpilogue e, double *partials,
+                                                                    const double *w, double *y2, const double *s2)
 {
    const int tid = blockIdx.x * kBlock + threadIdx.x;
    const int tsz = gridDim.x * kBlock;
    const bool norm = partials != nullptr;
    double ss;
-   if (MODE == 5) ss = sell_rows_team<true, SVAL, 8, false, DOT, DUAL>(M, x, y, e, tid, tsz, norm, w, y2, s2);  // the generic batch-of-8 loop ("v2", 56 registers)
-   else if (MODE >= 2) ss = sell_rows_team<true, SVAL, 4, true, DOT, DUAL>(M, x, y, e, tid, tsz, norm, w, y2, s2);   // (2 / 3 / 4: the cached-delta path at 5 / 4 / 6 CTAs per SM)
+   if (MODE == 2) ss = sell_rows_team<true, SVAL, 4, true, DOT, DUAL>(M, x, y, e, tid, tsz, norm, w, y2, s2);   // the cached-delta path, 5 CTAs per SM
    else if (MODE == 1) ss = sell_rows_team<true, SVAL, 0, false, DOT, DUAL>(M, x, y, e, tid, tsz, norm, w, y2, s2);
    else ss = csr_rows_dispatch<true, SVAL, DOT, DUAL>(M, x, y, e, tid, tsz, norm, w, y2, s2);
-   if (norm) {
-      ss = block_sum(ss);
-      if (threadIdx.x == 0) partials[blockIdx.x] = ss;
-   }
-}
-
-template <int NT, int CAP, int XCAP, int ST, bool SVAL, bool DOT = false, bool DUAL = false>
-__global__ void __launch_bounds__(NT) k_spmv_stream(DevCSR M, const double *x, double *y, SpmvEpilogue e, double *partials, const double *w,
-                                                    double *y2, const double *s2)
-{
-   extern __shared__ __align__(128) unsigned char dyn_smem[];
-   const bool norm = partials != nullptr;
-   double ss = stream_rows_team<true, SVAL, NT, CAP, XCAP, ST, DOT, DUAL>(M, x, y, e, blockIdx.x, gridDim.x, dyn_smem, norm, M.blk, M.nblk, w,
-                                                                      y2, s2);
    if (norm) {
       ss = block_sum(ss);
       if (threadIdx.x == 0) partials[blockIdx.x] = ss;
@@ -256,15 +241,15 @@ inline int grid_for(const LaunchCfg &cfg, long work_threads)
 
 }  // namespace
 
-template <int EPT, bool SVAL, bool SORTED, bool DOT = false, bool DUAL = false>
+template <bool SVAL, bool DOT = false, bool DUAL = false>
 __global__ void __launch_bounds__(kBlock) k_spmv_wstream(DevCSR M, const double *x, double *y, SpmvEpilogue e, double *partials, const double *w,
                                                          double *y2, const double *s2)
 {
-   __shared__ __align__(16) double swarp[(kBlock / 32) * EPT * 32];
+   __shared__ __align__(16) double swarp[(kBlock / 32) * AMGB_WARP_CHUNK];
    const bool norm = partials != nullptr;
    const int warp = threadIdx.x >> 5;
-   double ss = warp_stream_rows_team<true, SVAL, EPT, SORTED, DOT, DUAL>(M, x, y, e, blockIdx.x * (kBlock / 32) + warp, gridDim.x * (kBlock / 32),
-                                                                    swarp + warp * EPT * 32, norm, w, y2, s2);
+   double ss = warp_stream_rows_team<true, SVAL, DOT, DUAL>(M, x, y, e, blockIdx.x * (kBlock / 32) + warp, gridDim.x * (kBlock / 32),
+                                                            swarp + warp * AMGB_WARP_CHUNK, norm, w, y2, s2);
    if (norm) {
       ss = block_sum(ss);
       if (threadIdx.x == 0) partials[blockIdx.x] = ss;
@@ -272,14 +257,12 @@ __global__ void __launch_bounds__(kBlock) k_spmv_wstream(DevCSR M, const double 
 }
 
 template <class K>
-static int resident_ctas(K kernel, int block, size_t dyn, int num_sms, int *cache)
+static int resident_ctas(K kernel, int block, int num_sms, int *cache)
 {
    // co-resident CTAs of this kernel on the device: grids are sized to exactly one wave
-   // (the opt-in for more than 48 KB of dynamic shared memory is per device: set it on every call, it is cheap)
-   if (dyn) cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
    if (*cache == 0) {
       int v = 0;
-      if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&v, kernel, block, dyn) != cudaSuccess || v < 1) v = 1;
+      if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&v, kernel, block, 0) != cudaSuccess || v < 1) v = 1;
       *cache = std::min(v, 8);      // the per-CTA partial sums of the fused norms are sized for 8 CTAs per SM (LaunchCfg::ctas_per_sm)
    }
    return num_sms * *cache;
@@ -291,7 +274,7 @@ static int spmv_mode_go(const LaunchCfg &cfg, cudaStream_t st, const DevCSR &M, 
                         double *partials, long ctas_of_work, const double *w, double *y2 = nullptr, const double *s2 = nullptr)
 {
    static int occ = 0;
-   const int cap = resident_ctas(k_spmv<MODE, SVAL, DOT, DUAL>, kBlock, 0, cfg.num_sms, &occ);
+   const int cap = resident_ctas(k_spmv<MODE, SVAL, DOT, DUAL>, kBlock, cfg.num_sms, &occ);
    const int grid = (int)std::max(1L, std::min(ctas_of_work, (long)cap));
    k_spmv<MODE, SVAL, DOT, DUAL><<<grid, kBlock, 0, st>>>(M, x, y, e, partials, w, y2, s2);
    return grid;
@@ -307,78 +290,35 @@ static int launch_spmv_mode(const LaunchCfg &cfg, cudaStream_t st, const DevCSR 
                    : spmv_mode_go<MODE, false, false>(cfg, st, M, x, y, e, partials, ctas_of_work, nullptr);
 }
 
-template <int NT, int CAP, int XCAP, int ST, bool SVAL, bool DOT, bool DUAL = false>
-static int stream_go(const LaunchCfg &cfg, cudaStream_t st, const DevCSR &M, const double *x, double *y, const SpmvEpilogue &e,
-                     double *partials, const double *w, double *y2 = nullptr, const double *s2 = nullptr)
-{
-   static int occ = 0;
-   constexpr size_t dyn = stream_smem_bytes(CAP, XCAP, ST);
-   const int cap = resident_ctas(k_spmv_stream<NT, CAP, XCAP, ST, SVAL, DOT, DUAL>, NT, dyn, cfg.num_sms, &occ);
-   const int grid = (int)std::max(1L, std::min((long)M.nblk, (long)cap));
-   k_spmv_stream<NT, CAP, XCAP, ST, SVAL, DOT, DUAL><<<grid, NT, dyn, st>>>(M, x, y, e, partials, w, y2, s2);
-   return grid;
-}
-template <int NT, int CAP, int XCAP, int ST>
-static int launch_stream_variant(const LaunchCfg &cfg, cudaStream_t st, const DevCSR &M, bool use_sval, const double *x, double *y,
-                                 const SpmvEpilogue &e, double *partials, const double *w, double *y2, const double *s2)
-{
-   if (y2) return stream_go<NT, CAP, XCAP, ST, true, false, true>(cfg, st, M, x, y, e, nullptr, nullptr, y2, s2);
-   if (w) return use_sval ? stream_go<NT, CAP, XCAP, ST, true, true>(cfg, st, M, x, y, e, partials, w)
-                          : stream_go<NT, CAP, XCAP, ST, false, true>(cfg, st, M, x, y, e, partials, w);
-   return use_sval ? stream_go<NT, CAP, XCAP, ST, true, false>(cfg, st, M, x, y, e, partials, nullptr)
-                   : stream_go<NT, CAP, XCAP, ST, false, false>(cfg, st, M, x, y, e, partials, nullptr);
-}
-
-template <int EPT, bool SORTED, bool SVAL, bool DOT, bool DUAL = false>
+template <bool SVAL, bool DOT, bool DUAL = false>
 static int wstream_go(const LaunchCfg &cfg, cudaStream_t st, const DevCSR &M, const double *x, double *y, const SpmvEpilogue &e,
                       double *partials, const double *w, double *y2 = nullptr, const double *s2 = nullptr)
 {
    static int occ = 0;
-   const int cap = resident_ctas(k_spmv_wstream<EPT, SVAL, SORTED, DOT, DUAL>, kBlock, 0, cfg.num_sms, &occ);
+   const int cap = resident_ctas(k_spmv_wstream<SVAL, DOT, DUAL>, kBlock, cfg.num_sms, &occ);
    const long want = ((long)M.nblk + kBlock / 32 - 1) / (kBlock / 32);
    const int grid = (int)std::max(1L, std::min(want, (long)cap));
-   k_spmv_wstream<EPT, SVAL, SORTED, DOT, DUAL><<<grid, kBlock, 0, st>>>(M, x, y, e, partials, w, y2, s2);
+   k_spmv_wstream<SVAL, DOT, DUAL><<<grid, kBlock, 0, st>>>(M, x, y, e, partials, w, y2, s2);
    return grid;
 }
-template <int EPT, bool SORTED>
 static int launch_wstream(const LaunchCfg &cfg, cudaStream_t st, const DevCSR &M, bool use_sval, const double *x, double *y,
                           const SpmvEpilogue &e, double *partials, const double *w, double *y2, const double *s2)
 {
-   if (y2) return wstream_go<EPT, SORTED, true, false, true>(cfg, st, M, x, y, e, nullptr, nullptr, y2, s2);
-   if (w) return use_sval ? wstream_go<EPT, SORTED, true, true>(cfg, st, M, x, y, e, partials, w)
-                          : wstream_go<EPT, SORTED, false, true>(cfg, st, M, x, y, e, partials, w);
-   return use_sval ? wstream_go<EPT, SORTED, true, false>(cfg, st, M, x, y, e, partials, nullptr)
-                   : wstream_go<EPT, SORTED, false, false>(cfg, st, M, x, y, e, partials, nullptr);
+   if (y2) return wstream_go<true, false, true>(cfg, st, M, x, y, e, nullptr, nullptr, y2, s2);
+   if (w) return use_sval ? wstream_go<true, true>(cfg, st, M, x, y, e, partials, w)
+                          : wstream_go<false, true>(cfg, st, M, x, y, e, partials, w);
+   return use_sval ? wstream_go<true, false>(cfg, st, M, x, y, e, partials, nullptr)
+                   : wstream_go<false, false>(cfg, st, M, x, y, e, partials, nullptr);
 }
 
 int launch_spmv(const LaunchCfg &cfg, cudaStream_t st, const DevCSR &M, bool use_sval, const double *x, double *y,
                 const SpmvEpilogue &e, double *partials, int *grid_out, const double *dot_w, double *y2, const double *s2)
 {
    int grid;
-   if (M.sell_slices > 0 && M.su_desc && cfg.sellu_ctas == 4) grid = launch_spmv_mode<3>(cfg, st, M, use_sval, x, y, e, partials, ((long)M.sell_slices * 32 + kBlock - 1) / kBlock, dot_w, y2, s2);
-   else if (M.sell_slices > 0 && M.su_desc && cfg.sellu_ctas == 6) grid = launch_spmv_mode<4>(cfg, st, M, use_sval, x, y, e, partials, ((long)M.sell_slices * 32 + kBlock - 1) / kBlock, dot_w, y2, s2);
-   else if (M.sell_slices > 0 && M.su_desc && cfg.sellu_ctas == 8) grid = launch_spmv_mode<5>(cfg, st, M, use_sval, x, y, e, partials, ((long)M.sell_slices * 32 + kBlock - 1) / kBlock, dot_w, y2, s2);
-   else if (M.sell_slices > 0 && M.su_desc) grid = launch_spmv_mode<2>(cfg, st, M, use_sval, x, y, e, partials, ((long)M.sell_slices * 32 + kBlock - 1) / kBlock, dot_w, y2, s2);
+   if (M.sell_slices > 0 && M.su_desc) grid = launch_spmv_mode<2>(cfg, st, M, use_sval, x, y, e, partials, ((long)M.sell_slices * 32 + kBlock - 1) / kBlock, dot_w, y2, s2);
    else if (M.sell_slices > 0) grid = launch_spmv_mode<1>(cfg, st, M, use_sval, x, y, e, partials, ((long)M.sell_slices * 32 + kBlock - 1) / kBlock, dot_w, y2, s2);
-   else if (M.nblk > 0 && M.wept > 0) {
-      if (M.pos) {
-         if (M.wept <= 4) grid = launch_wstream<4, true>(cfg, st, M, use_sval, x, y, e, partials, dot_w, y2, s2);
-         else grid = launch_wstream<8, true>(cfg, st, M, use_sval, x, y, e, partials, dot_w, y2, s2);
-      } else if (M.wept <= 4) grid = launch_wstream<4, false>(cfg, st, M, use_sval, x, y, e, partials, dot_w, y2, s2);
-      else if (M.wept <= 8) grid = launch_wstream<8, false>(cfg, st, M, use_sval, x, y, e, partials, dot_w, y2, s2);
-      else grid = launch_wstream<16, false>(cfg, st, M, use_sval, x, y, e, partials, dot_w, y2, s2);
-   } else if (M.nblk > 0) {
-      switch (cfg.stream_variant) {   // keep in step with kStreamVariants (launch.h)
-         case 1: grid = launch_stream_variant<128, 1024, 0, 2>(cfg, st, M, use_sval, x, y, e, partials, dot_w, y2, s2); break;
-         case 2: grid = launch_stream_variant<128, 1024, 0, 3>(cfg, st, M, use_sval, x, y, e, partials, dot_w, y2, s2); break;
-         case 3: grid = launch_stream_variant<256, 2048, 1536, 2>(cfg, st, M, use_sval, x, y, e, partials, dot_w, y2, s2); break;
-         case 4: grid = launch_stream_variant<128, 1024, 1024, 2>(cfg, st, M, use_sval, x, y, e, partials, dot_w, y2, s2); break;
-         case 5: grid = launch_stream_variant<256, 1024, 0, 2>(cfg, st, M, use_sval, x, y, e, partials, dot_w, y2, s2); break;
-         case 6: grid = launch_stream_variant<128, 1024, 1024, 3>(cfg, st, M, use_sval, x, y, e, partials, dot_w, y2, s2); break;
-         case 7: grid = launch_stream_variant<128, 2048, 0, 2>(cfg, st, M, use_sval, x, y, e, partials, dot_w, y2, s2); break;
-         default: grid = launch_stream_variant<256, 2048, 0, 3>(cfg, st, M, use_sval, x, y, e, partials, dot_w, y2, s2); break;
-      }
-   } else grid = launch_spmv_mode<0>(cfg, st, M, use_sval, x, y, e, partials, ((long)M.nrows * M.lpr + kBlock - 1) / kBlock, dot_w, y2, s2);
+   else if (M.nblk > 0) grid = launch_wstream(cfg, st, M, use_sval, x, y, e, partials, dot_w, y2, s2);
+   else grid = launch_spmv_mode<0>(cfg, st, M, use_sval, x, y, e, partials, ((long)M.nrows * M.lpr + kBlock - 1) / kBlock, dot_w, y2, s2);
    if (grid_out) *grid_out = grid;
    return 1;
 }
@@ -395,7 +335,7 @@ int launch_spmv_units(const LaunchCfg &cfg, cudaStream_t st, const DevCSR &M, in
    SpmvEpilogue ev = e;
    double *yv = y;
    if (M.sell_slices > 0) { V.sell_off += u0; V.sell_base += u0; V.sell_slices = u1 - u0; if (V.su_desc) V.su_desc += u0; }
-   else if (M.nblk > 0) { V.blk += u0; if (V.blkx) V.blkx += u0; V.nblk = u1 - u0; }
+   else if (M.nblk > 0) { V.blk += u0; V.nblk = u1 - u0; }
    else {
       V.rp += u0; V.nrows = u1 - u0; yv += u0;
       if (ev.b) ev.b += u0;

@@ -119,10 +119,6 @@ __device__ __forceinline__ double sell_rows_team(const DevCSR &M, const double *
       } else if (SU > 0 && dsc.y > 0) {
          const double *__restrict__ gv = SVAL ? M.su_sval : M.su_va;
          const bool ok = row < M.nrows;
-         constexpr bool PRELOAD = RO && !FAST;        // (the variant measured as "v2": epilogue operands in flight with the gathers)
-         EpiOps ops;
-         ops.b = 0.0; ops.c = 0.0; ops.rs = 1.0;
-         if (PRELOAD && ok) ops = epilogue_load<RO>(e, row);
          for (int g = 0; g < dsc.y; g += (SU > 0 ? SU : 1)) {
             double xv[SU > 0 ? SU : 1];
             const int2 *__restrict__ dmp = M.su_dm + dsc.x + g;
@@ -139,7 +135,7 @@ __device__ __forceinline__ double sell_rows_team(const DevCSR &M, const double *
                if (k < left) acc += __ldg(gv + dsc.x + g + k) * xv[k];
          }
          if (ok) {
-            const double v = PRELOAD ? epilogue_finish(e, ops, acc) : epilogue_apply<RO>(e, row, acc);
+            const double v = epilogue_apply<RO>(e, row, acc);
             epilogue_store<RO>(e, y, row, v);
             if (want_sumsq) sumsq += DOT ? v * __ldg(dw + row) : v * v;
             if (DUAL) y2[row] = __ldg(s2 + row) * (e.b[row] + v);
@@ -163,214 +159,21 @@ __device__ __forceinline__ double sell_rows_team(const DevCSR &M, const double *
    return sumsq;
 }
 
-// ---- CSR-stream: row blocks staged through shared memory by TMA bulk copies ---------------------
-// A CTA of NT threads owns every team_nctas-th row block (<= CAP entries).  Warp 0 keeps ST blocks in
-// flight with cp.async.bulk copies (SASS UBLKCP) that complete on the stage's mbarrier: the block's
-// values, its column indices and -- when XS and the host found that the block's columns are covered by
-// <= 32 contiguous windows of x (DevCSR::blkx/win/li) -- those windows of x themselves, one bulk copy per
-// lane.  No register staging: the HBM stream never stalls on the row structure.  Per block the threads
-// then (1) multiply the staged values by the gathered x in place (consecutive lanes take consecutive
-// entries), (2) sum each row's products with a sub-warp sized to the block's row count and apply the
-// fused epilogue, whose row operands were loaded before the barrier wait.  A block made of ONE row longer
-// than CAP is read straight from global memory by the whole CTA.
-// `smem`: stream_smem_bytes(CAP, XCAP, ST) bytes, 128-byte aligned.  Called by all NT threads of the CTA.
-__host__ __device__ constexpr int stream_stage_bytes(int cap, int xcap) { return cap * 12 + xcap * 8; }
-__host__ __device__ constexpr int stream_smem_bytes(int cap, int xcap, int st) { return st * stream_stage_bytes(cap, xcap) + 64; }
-
-template <bool RO, bool SVAL, int NT, int CAP, int XCAP, int ST, bool DOT = false, bool DUAL = false>
-__device__ __forceinline__ double stream_rows_team(const DevCSR &M, const double *__restrict__ x, double *y,
-                                                   const SpmvEpilogue &e, int team_cta, int team_nctas,
-                                                   unsigned char *smem, bool want_sumsq, const int4 *blk, int nblk,
-                                                   const double *dw = nullptr, double *y2 = nullptr, const double *s2 = nullptr)
-{
-   constexpr int SB = stream_stage_bytes(CAP, XCAP);
-   constexpr int EPT = CAP / NT;                      // entries per thread
-   const int tid = threadIdx.x;
-   const double *__restrict__ va = SVAL ? M.sval : M.va;
-   auto st_vals = [&](int s) { return reinterpret_cast<double *>(smem + (size_t)s * SB); };
-   auto st_cols = [&](int s) { return smem + (size_t)s * SB + (size_t)CAP * 8; };
-   auto st_xwin = [&](int s) { return reinterpret_cast<double *>(smem + (size_t)s * SB + (size_t)CAP * 12); };
-   const uint32_t bar0 = smem_u32(smem + (size_t)ST * SB);
-   const int nmine = team_cta < nblk ? (nblk - team_cta + team_nctas - 1) / team_nctas : 0;
-   // staged x needs x read-only for the whole launch (bulk copies read through the async proxy) and 16-byte aligned
-   const bool xstage = XCAP > 0 && RO && M.blkx != nullptr && ((reinterpret_cast<uintptr_t>(x) & 15) == 0);
-   double sumsq = 0.0;
-   uint64_t pol = 0, polx = 0;
-
-   // executed by all 32 lanes of warp 0
-   auto issue = [&](const int4 d, const int4 dx, int stage) {
-      const int lane = tid & 31;
-      const int q0 = d.z & ~7;
-      if (d.w - q0 > CAP || d.w == d.z) return;       // long row / no entries: not staged
-      const uint32_t n8 = (uint32_t)((d.w - q0 + 7) & ~7);
-      const uint32_t bar = bar0 + 8u * stage;
-      const bool usex = xstage && dx.y > 0;
-      int2 w = make_int2(0, 0);
-      if (usex && lane < dx.y) w = __ldg(M.win + dx.x + lane);
-      int wtot = w.y;
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) wtot += __shfl_xor_sync(AMGB_FULL, wtot, o);
-      int woff = w.y;                                  // exclusive prefix of the window lengths
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-         const int t = __shfl_up_sync(AMGB_FULL, woff, o);
-         if (lane >= o) woff += t;
-      }
-      woff -= w.y;
-      if (lane == 0) {
-         mbar_expect_tx(bar, n8 * 8u + (usex ? n8 * 2u : n8 * 4u) + (uint32_t)wtot * 8u);
-         tma_bulk_g2s(smem_u32(st_vals(stage)), va + q0, n8 * 8u, bar, pol);
-         if (usex) tma_bulk_g2s(smem_u32(st_cols(stage)), M.li + q0, n8 * 2u, bar, pol);
-         else tma_bulk_g2s(smem_u32(st_cols(stage)), M.ci + q0, n8 * 4u, bar, pol);
-      }
-      if (w.y > 0) tma_bulk_g2s(smem_u32(st_xwin(stage) + woff), x + w.x, (uint32_t)w.y * 8u, bar, polx);
-   };
-
-   __syncthreads();                                   // previous users of smem (and of the barriers) are done
-   if (tid < 32) {
-      pol = l2_evict_first_policy();
-      polx = l2_evict_last_policy();
-      if (tid == 0) {
-         for (int s = 0; s < ST; s++) mbar_init(bar0 + 8u * s, 1);
-         mbar_init_fence();
-         fence_proxy_async();
-      }
-      __syncwarp();
-      for (int s = 0; s < ST && s < nmine; s++) {
-         const int b = team_cta + s * team_nctas;
-         issue(__ldg(blk + b), xstage ? __ldg(M.blkx + b) : make_int4(0, 0, 0, 0), s);
-      }
-   }
-   __syncthreads();
-   uint32_t phase = 0;                                // bit s: parity to wait for on stage s
-   int4 d = nmine > 0 ? __ldg(blk + team_cta) : make_int4(0, 0, 0, 0);
-   int4 dx = (nmine > 0 && xstage) ? __ldg(M.blkx + team_cta) : make_int4(0, 0, 0, 0);
-   for (int i = 0; i < nmine; i++) {
-      const int b = team_cta + i * team_nctas;
-      const int stage = i % ST;
-      const int r0 = d.x, r1 = d.y, p0 = d.z, p1 = d.w, q0 = p0 & ~7, nr = r1 - r0;
-      const bool usex = xstage && dx.y > 0;
-      int4 dn = make_int4(0, 0, 0, 0), dnx = dn, dp = dn, dpx = dn;
-      if (i + 1 < nmine) {
-         dn = __ldg(blk + b + team_nctas);
-         if (xstage) dnx = __ldg(M.blkx + b + team_nctas);
-      }
-      if (tid < 32 && i + ST < nmine) {
-         dp = __ldg(blk + b + ST * team_nctas);
-         if (xstage) dpx = __ldg(M.blkx + b + ST * team_nctas);
-      }
-      if (p1 - q0 > CAP) {
-         double acc = 0.0;
-         for (int p = p0 + tid; p < p1; p += NT) acc += ld_stream(va + p) * ld_x<RO>(x + ld_stream(M.ci + p));
-         acc = block_sum(acc);
-         if (tid == 0) {
-            const double v = epilogue_apply<RO>(e, r0, acc);
-            y[r0] = v;
-            if (want_sumsq) sumsq += DOT ? v * __ldg(dw + r0) : v * v;
-            if (DUAL) y2[r0] = __ldg(s2 + r0) * (e.b[r0] + v);
-         }
-         __syncthreads();
-      } else {
-         // lanes per row: the largest power of two (<= 32) such that all rows fit in one pass
-         int lpr = 1;
-         while (lpr < 32 && nr * (lpr << 1) <= NT) lpr <<= 1;
-         const int lane = tid & (lpr - 1);
-         const int rows_per_pass = NT / lpr;
-         // first pass: row pointers and epilogue operands loaded before the barrier wait
-         const int row_a = r0 + tid / lpr;
-         const bool ok_a = row_a < r1;
-         int s_a = 0, t_a = 0;
-         EpiOps o_a;
-         o_a.b = 0.0; o_a.c = 0.0; o_a.rs = 1.0;
-         if (ok_a) {
-            s_a = __ldg(M.rp + row_a) - q0;
-            t_a = __ldg(M.rp + row_a + 1) - q0;
-            if (lane == 0) o_a = epilogue_load<RO>(e, row_a);
-         }
-         if (p1 > p0) {
-            mbar_wait(bar0 + 8u * stage, (phase >> stage) & 1u);
-            phase ^= 1u << stage;
-         }
-         double *vs = st_vals(stage);
-         // products in place; consecutive lanes take consecutive entries
-         const int first = p0 - q0, cnt = p1 - q0;
-         double xv[EPT];
-         if (usex) {
-            const unsigned short *cs = reinterpret_cast<const unsigned short *>(st_cols(stage));
-            const double *xs = st_xwin(stage);
-#pragma unroll
-            for (int k = 0; k < EPT; k++) {
-               const int q = tid + NT * k;
-               xv[k] = (q >= first && q < cnt) ? xs[cs[q]] : 0.0;
-            }
-         } else {
-            const int *cs = reinterpret_cast<const int *>(st_cols(stage));
-#pragma unroll
-            for (int k = 0; k < EPT; k++) {
-               const int q = tid + NT * k;
-               xv[k] = (q >= first && q < cnt) ? ld_x<RO>(x + cs[q]) : 0.0;
-            }
-         }
-#pragma unroll
-         for (int k = 0; k < EPT; k++) {
-            const int q = tid + NT * k;
-            if (q < cnt) vs[q] = (q >= first) ? vs[q] * xv[k] : 0.0;
-         }
-         __syncthreads();
-         {
-            double acc = 0.0;
-            for (int q = s_a + lane; q < t_a; q += lpr) acc += vs[q];
-            for (int o = lpr >> 1; o > 0; o >>= 1) acc += __shfl_down_sync(AMGB_FULL, acc, o, 32);
-            if (lane == 0 && ok_a) {
-               const double v = epilogue_finish(e, o_a, acc);
-               y[row_a] = v;
-               if (want_sumsq) sumsq += DOT ? v * __ldg(dw + row_a) : v * v;
-               if (DUAL) y2[row_a] = __ldg(s2 + row_a) * (e.b[row_a] + v);
-            }
-         }
-         for (int base = rows_per_pass; base < nr; base += rows_per_pass) {   // only when lpr == 1
-            const int row = r0 + base + tid;
-            if (row < r1) {
-               const int s1 = __ldg(M.rp + row) - q0, t1 = __ldg(M.rp + row + 1) - q0;
-               double acc = 0.0;
-               for (int q = s1; q < t1; q++) acc += vs[q];
-               const double v = epilogue_apply<RO>(e, row, acc);
-               y[row] = v;
-               if (want_sumsq) sumsq += DOT ? v * __ldg(dw + row) : v * v;
-               if (DUAL) y2[row] = __ldg(s2 + row) * (e.b[row] + v);
-            }
-         }
-         __syncthreads();                              // the stage is free again
-      }
-      if (tid < 32 && i + ST < nmine) {
-         if (tid == 0) fence_proxy_async();
-         __syncwarp();
-         issue(dp, dpx, stage);
-      }
-      d = dn;
-      dx = dnx;
-   }
-   __syncthreads();
-   if (tid == 0)
-      for (int s = 0; s < ST; s++) mbar_inval(bar0 + 8u * s);   // the memory may be re-initialised by the next call
-   return sumsq;
-}
-
-// ---- warp-stream: the CSR-stream idea at warp granularity, no CTA-wide barriers ----------------
-// Every WARP owns every team_nwarps-th row chunk (<= EPT*32 entries, same descriptors as the row blocks).
+// ---- warp-stream: CSR row chunks at warp granularity, no CTA-wide barriers -----------------------
+// Every WARP owns every team_nwarps-th row chunk (DevCSR::blk, <= AMGB_WARP_CHUNK entries).
 // Lanes load the chunk's (col,val) pairs coalesced (consecutive lanes = consecutive entries, all 2*EPT
 // loads issued before the first use), gather x, park the products in the warp's private slice of shared
 // memory, __syncwarp, and sum each row with a sub-warp sized to the chunk's row count.  Warps never wait
 // for each other, so the load / gather / reduce phases of the 32-64 resident warps of an SM overlap
-// freely -- the CTA-synchronous variant above spends ~20 % of its issue slots in barrier stalls and ~45 %
-// waiting on gathers with only 3-5 CTAs to hide them (profiles/).  swarp: EPT*32 doubles per warp.
-template <bool RO, bool SVAL, int EPT, bool SORTED = false, bool DOT = false, bool DUAL = false>
+// freely -- a CTA-synchronous form of the same idea spent ~20 % of its issue slots in barrier stalls and ~45 %
+// waiting on gathers with only 3-5 CTAs to hide them (DESIGN.md 3.3).  swarp: AMGB_WARP_CHUNK doubles per warp.
+template <bool RO, bool SVAL, bool DOT = false, bool DUAL = false>
 __device__ __forceinline__ double warp_stream_rows_team(const DevCSR &M, const double *__restrict__ x, double *y,
                                                         const SpmvEpilogue &e, int team_warp, int team_nwarps,
                                                         double *swarp, bool want_sumsq, const double *dw = nullptr,
                                                         double *y2 = nullptr, const double *s2 = nullptr)
 {
-   constexpr int CAP = EPT * 32;
+   constexpr int CAP = AMGB_WARP_CHUNK, EPT = CAP / 32;
    const int lane = threadIdx.x & 31;
    const double *__restrict__ va = SVAL ? M.sval : M.va;
    double sumsq = 0.0;
@@ -391,18 +194,16 @@ __device__ __forceinline__ double warp_stream_rows_team(const DevCSR &M, const d
          }
          continue;
       }
-      int cc[EPT], pp[EPT];
+      int cc[EPT];
       double vv[EPT];
-      const int *__restrict__ cip = SORTED ? M.pci : M.ci;
-      const double *__restrict__ vap = SORTED ? (SVAL ? M.psval : M.pva) : va;
+      const int *__restrict__ ci = M.ci;               // (read through M.ci directly, ptxas lays the long-row branch out differently)
 #pragma unroll
       for (int k = 0; k < EPT; k++) {
          const int q = lane + 32 * k;
-         cc[k] = 0; vv[k] = 0.0; pp[k] = q;
+         cc[k] = 0; vv[k] = 0.0;
          if (q < cnt) {
-            cc[k] = ld_stream(cip + p0 + q);
-            vv[k] = ld_stream(vap + p0 + q);
-            if (SORTED) pp[k] = ld_stream(M.pos + p0 + q);
+            cc[k] = ld_stream(ci + p0 + q);
+            vv[k] = ld_stream(va + p0 + q);
          }
       }
       // lanes per row: the largest power of two such that all rows fit in one pass
@@ -428,7 +229,7 @@ __device__ __forceinline__ double warp_stream_rows_team(const DevCSR &M, const d
 #pragma unroll
       for (int k = 0; k < EPT; k++) {
          const int q = lane + 32 * k;
-         if (q < cnt) swarp[pp[k]] = vv[k];
+         if (q < cnt) swarp[q] = vv[k];
       }
       __syncwarp();
       {

@@ -8,22 +8,6 @@
 struct LaunchCfg {
    int num_sms = 148;
    int ctas_per_sm = 8;
-   int stream_variant = 0;
-   int sellu_ctas = 5;          // SELL-U kernel variant (AMGB_SELLU_CTAS): cached-delta path at 5 (48 registers, default), 4 (64) or 6 (40, spills)
-                                // CTAs per SM; 8 = the generic batch-of-8 loop at 4 CTAs per SM (56 registers)
-};
-
-// geometry of the CSR-stream kernel (kernels.cuh stream_rows_team): threads per CTA, entries per row block,
-// staged-x window capacity (0 = gather x from global memory), bulk-copy stages.  amgb_options.stream_variant
-// selects one; the row blocks are built for its cap / xcap at upload time.
-struct StreamVariant { int nt, cap, xcap, stages; };
-// stages == 0: the warp-granular variant (warp_stream_rows_team), cap = entries per warp chunk
-// stages == -1: warp-granular with column-sorted chunks (DevCSR::pci/pva/pos)
-#define AMGB_NUM_STREAM_VARIANTS 13
-static const StreamVariant kStreamVariants[AMGB_NUM_STREAM_VARIANTS] = {
-   {256, 2048, 0, 3}, {128, 1024, 0, 2}, {128, 1024, 0, 3}, {256, 2048, 1536, 2},
-   {128, 1024, 1024, 2}, {256, 1024, 0, 2}, {128, 1024, 1024, 3}, {128, 2048, 0, 2},
-   {256, 256, 0, 0}, {256, 128, 0, 0}, {256, 512, 0, 0}, {256, 256, 0, -1}, {256, 128, 0, -1},
 };
 
 // y = gamma*c + rs.*(beta*b + alpha*M*x); optional sum of y_i^2 -- or of y_i*dot_w_i when dot_w is given -- into partial

@@ -24,7 +24,7 @@ ABI_SYMBOLS = [
     "amgb_set_num_levels", "amgb_set_matrix", "amgb_set_options", "amgb_setup",
     "amgb_set_rhs", "amgb_set_solution", "amgb_get_solution", "amgb_get_residual",
     "amgb_spgemv", "amgb_spgemv_transpose", "amgb_smooth", "amgb_set_jgs_blocks", "amgb_norm2", "amgb_cycle", "amgb_eigs_power", "amgb_solve_sync", "amgb_solve_async",
-    "amgb_async_groups", "amgb_solve_extended", "amgb_solve_extended_async", "amgb_smooth_transfer", "amgb_host_csr_free", "amgb_smem_solve", "amgb_time_residual", "amgb_level_storage", "amgb_time_spmv", "amgb_stream_stats", "amgb_l2_arena_bytes", "amgb_sellu_stats",
+    "amgb_async_groups", "amgb_solve_extended", "amgb_solve_extended_async", "amgb_smooth_transfer", "amgb_host_csr_free", "amgb_smem_solve", "amgb_time_residual", "amgb_level_storage", "amgb_time_spmv", "amgb_l2_arena_bytes", "amgb_sellu_stats",
     "amgb_sellu_encode_host", "amgb_host_free", "amgb_async_program", "amgb_async_group_times",
     "amgb_solve_extended_implicit_async", "amgb_ext_async_program", "amgb_solve_pcg",
     "amgb_dist_unique_id", "amgb_dist_init", "amgb_dist_set_level", "amgb_dist_setup", "amgb_dist_set_rhs",
@@ -101,7 +101,6 @@ def load_library():
     L.amgb_time_residual.argtypes = [C.c_void_p, C.c_int, DP]
     L.amgb_level_storage.argtypes = [C.c_void_p, C.c_int, C.c_int, IP]
     L.amgb_time_spmv.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, DP]
-    L.amgb_stream_stats.argtypes = [C.c_void_p, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)]
     L.amgb_l2_arena_bytes.argtypes = [C.c_void_p, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)]
     L.amgb_sellu_stats.argtypes = [C.c_void_p, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)]
     L.amgb_async_groups.argtypes = [C.c_void_p, IP, IP]
@@ -153,7 +152,7 @@ class Solver:
 
     def __init__(self, h, solver=H.MULTADD, smoother=H.JACOBI, smooth_weight=1.0, num_pre=1, num_post=1,
                  fine_sweeps=1, coarse_sweeps=1, jgs_block_rows=8, use_sell=True, l2_persist=True, use_stream=True,
-                 stream_variant=None, sell_sigma=None, coarse_solve=False, factor_level0=False, device=0, jgs_blocks=None,
+                 sell_sigma=None, coarse_solve=False, factor_level0=False, device=0, jgs_blocks=None,
                  sell_uniform=None, async_type=0, res_compute_type=0, read_type=0, lean_storage=False, factor_restriction=None):
         """factor_restriction (amgb_options.factor_restriction): None = on exactly where amgb_setup accepts it, i.e. with
         factor_level0 for the synchronous Multadd cycle with the symmetrised (L1-)Jacobi smoother and one fine sweep; the
@@ -175,10 +174,6 @@ class Solver:
         o.use_stream = int(use_stream)
         o.coarse_solve = int(coarse_solve)
         o.factor_level0 = int(factor_level0)
-        if stream_variant is not None:
-            o.stream_variant = int(stream_variant)
-        elif "AMGB_STREAM_VARIANT" in os.environ:
-            o.stream_variant = int(os.environ["AMGB_STREAM_VARIANT"])
         if sell_sigma is not None:
             o.sell_sigma = int(sell_sigma)
         elif "AMGB_SELL_SIGMA" in os.environ:
@@ -395,11 +390,6 @@ class Solver:
         ms = C.c_double(0)
         self._ck(self.L.amgb_time_spmv(self.ctx, kind, level, int(use_sval), reps, C.byref(ms)))
         return ms.value
-
-    def stream_stats(self):
-        a, b = C.c_longlong(0), C.c_longlong(0)
-        self._ck(self.L.amgb_stream_stats(self.ctx, C.byref(a), C.byref(b)))
-        return a.value, b.value
 
     def l2_arena_bytes(self):
         a, b = C.c_longlong(0), C.c_longlong(0)

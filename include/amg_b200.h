@@ -54,8 +54,9 @@ typedef struct {
                                    src/SMEM_Smooth.cpp:567-581; SURVEY.md 5.9e) */
    int use_sell;                /* 1: sliced-ELL (C=32) storage for low-variance levels, 0: CSR only */
    int l2_persist;              /* 1: pin the coarse hierarchy in L2 with an access-policy window */
-   int use_stream;              /* 1: CSR-stream kernel (row blocks staged through shared memory with 128-bit
-                                   loads) for every matrix not stored as sliced ELL; 0: vector-per-row CSR */
+   int use_stream;              /* 1: warp-stream CSR kernel (each warp reduces chunks of <= 256 consecutive entries through
+                                   shared memory) for every matrix not stored as sliced ELL whose rows average fewer than
+                                   96 entries; 0, and those long-row matrices: vector-per-row CSR */
    int factor_level0;           /* 1 (synchronous Multadd with the symmetrised smoother only): P_0 / R_0 are uploaded PLAIN and the
                                    smoothing factors are applied on the fly, Pbar_0 e = (I - w D^-1 A_0)(P_0 e), Rbar_0 r = R_0 (r - w A_0 D^-1 r):
                                    the level-0 smoother and Rbar_0 then share ONE pass over A_0.  Same operator, rounding-level
@@ -68,7 +69,8 @@ typedef struct {
                                    works like the others: restrict, solve directly (AddCycle), prolong, update */
    int sell_sigma;              /* > 1: SELL-C-sigma (rows sorted by length inside windows of sigma rows) for the
                                    non-stencil matrices whose padding then stays <= 25 %; 0/1: off */
-   int stream_variant;          /* geometry of the CSR-stream kernel (csrc/launch.h kStreamVariants; default 8 = warp-granular, 256-entry chunks) */
+   int stream_variant;          /* retired: must be 8, what amgb_default_options sets (the warp-stream kernel); any other value
+                                   is refused by amgb_set_options with AMGB_EINVAL.  Kept so that the fields after it stay in place */
    int sell_uniform;            /* 1 (default): SELL-U, a lossless re-encoding of sliced-ELL slices whose entries take few distinct
                                    (column - row, value) pairs (constant-coefficient stencil levels): the kernel then streams the vectors
                                    only.  Same CSR semantics, a row's terms summed in another order; 0: off */
@@ -257,11 +259,10 @@ void amgb_host_csr_free(amgb_host_csr *m);
  * r = f - A_0 u (the dominant kernel), on the context's stream */
 int amgb_time_residual(amgb_ctx *ctx, int reps, double *ms_per_launch);
 int amgb_level_storage(amgb_ctx *ctx, int kind, int level, int *is_sell);
-/* event-timed y = M x for one matrix of the hierarchy (tools/spmv_sweep.py) and CSR-stream block statistics.  use_scaled_values:
+/* event-timed y = M x for one matrix of the hierarchy (tools/spmv_sweep.py).  use_scaled_values:
  * 0 the values, 1 the column-scaled values; A_l only: 2 the symmetrised smoother's pass e = s o (2x - (A diag(s)) x) of the
  * explicit cycle, 3 the factorised restriction's pass t = x - (A diag(s)) x, e = s o (x + t) (amgb_options.factor_restriction) */
 int amgb_time_spmv(amgb_ctx *ctx, int kind, int level, int use_scaled_values, int reps, double *ms_per_launch);
-int amgb_stream_stats(amgb_ctx *ctx, long long *blocks, long long *blocks_with_staged_x);
 /* slices stored in the SELL-U encoding (amgb_options.sell_uniform) and their (delta, mask, value) groups */
 int amgb_sellu_stats(amgb_ctx *ctx, long long *slices, long long *groups);
 /* Host-only probe of the SELL-U encoder (no CUDA call; CPU test suite): CSR + column-scaled values in; out, per slice, the

@@ -66,9 +66,6 @@ LAYOUTS = [
     ("no_sellu", dict(sell_uniform=0)),
     ("sell_sigma_off", dict(sell_sigma=0)),
     ("warp_stream", dict(use_sell=False)),
-    ("warp_stream_sorted", dict(use_sell=False, stream_variant=11)),
-    ("cta_stream", dict(use_sell=False, stream_variant=0)),
-    ("cta_stream_xstaged", dict(use_sell=False, stream_variant=3)),
     ("csr_per_row", dict(use_sell=False, use_stream=False)),
 ]
 
@@ -80,6 +77,26 @@ def test_every_storage_layout(layout):
     b = H.rand_rhs(h.n[0])
     assert _rel(s.cycle(b), pb.cycle(b)) <= 1e-12
     s.close()
+
+
+def test_retired_stream_variant_is_refused():
+    """amgb_options.stream_variant only keeps its place in the struct: 8 (the default, the warp-stream kernel) is accepted,
+    any other value is an error rather than a silent fall-back to another kernel"""
+    L = amg.solver.load_library()
+    ctx = C.c_void_p()
+    assert L.amgb_create(C.byref(ctx), 0) == 0
+    try:
+        o = amg.solver.Options()
+        L.amgb_default_options(C.byref(o))
+        assert o.stream_variant == 8
+        for v in (0, 3, 11, 13, -1):
+            o.stream_variant = v
+            assert L.amgb_set_options(ctx, C.byref(o)) == EINVAL, v
+            assert b"stream_variant" in L.amgb_last_error(ctx)
+        o.stream_variant = 8
+        assert L.amgb_set_options(ctx, C.byref(o)) == 0
+    finally:
+        L.amgb_destroy(ctx)
 
 
 def test_sell_sigma_level():

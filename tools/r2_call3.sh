@@ -4,7 +4,6 @@ set -x
 mkdir -p gpurun_out
 timeout 900 python -m pytest tests -m gpu -q -rfEs 2>&1 | tail -40
 timeout 300 python tools/cycle_probe.py --n 256 --cycles 36 --time-ops
-AMGB_SELLU_CTAS=5 timeout 300 python tools/cycle_probe.py --n 256 --cycles 36 --time-ops | cut -c1-1200
 timeout 600 python tools/async_time.py --n 256 --corrections 35 --reps 2 --variants default,global
 ( time timeout 1500 python bench.py --impl reference --steps 2 --warmup 1 ) > gpurun_out/bench_r2_call3_ref.json 2> gpurun_out/bench_r2_call3_ref.err; tail -c 1500 gpurun_out/bench_r2_call3_ref.json; tail -4 gpurun_out/bench_r2_call3_ref.err
 ( time timeout 1500 python bench.py ) > gpurun_out/bench_r2_call3.json 2> gpurun_out/bench_r2_call3.err; tail -c 3000 gpurun_out/bench_r2_call3.json; tail -12 gpurun_out/bench_r2_call3.err
