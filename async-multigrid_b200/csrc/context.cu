@@ -103,6 +103,7 @@ void amgb_default_options(amgb_options *o)
    o->read_type = 0;
    o->lean_storage = 0;
    o->factor_restriction = 0;
+   o->sell_window_epilogue = 1;
 }
 
 int amgb_create(amgb_ctx **out, int device)
@@ -140,6 +141,7 @@ int amgb_create(amgb_ctx **out, int device)
    cudaEventCreate(&c->ev1);
    cudaMallocHost((void **)&c->h_scalars, 64 * sizeof(double));
    amgb_default_options(&c->opt);
+   c->cfg.sell_window_sigma = c->opt.sell_window_epilogue ? c->opt.sell_sigma : 0;
    *out = c;
    return AMGB_OK;
 }
@@ -187,6 +189,7 @@ int amgb_set_options(amgb_ctx *c, const amgb_options *o)
       return amgb_fail(c, AMGB_EINVAL, "stream_variant %d: the field is retired, only 8 (the warp-stream kernel) is accepted", o->stream_variant);
    if (c->L) return amgb_fail(c, AMGB_ESTATE, "amgb_set_options must precede the hierarchy upload");
    c->opt = *o;
+   c->cfg.sell_window_sigma = o->sell_window_epilogue ? o->sell_sigma : 0;
    return AMGB_OK;
 }
 
@@ -1350,19 +1353,23 @@ int amgb_time_spmv(amgb_ctx *c, int kind, int level, int use_sval, int reps, dou
    if (level < 0 || level >= c->L || (kind != AMGB_MAT_A && level >= c->L - 1) || reps < 1 || !ms_per_launch)
       return amgb_fail(c, AMGB_EINVAL, "bad arguments");
    const DevCSR &M = kind == AMGB_MAT_A ? c->A[level] : (kind == AMGB_MAT_P ? c->P[level] : c->R[level]);
-   if (use_sval < 0 || use_sval > 3 || (use_sval > 1 && kind != AMGB_MAT_A)) return amgb_fail(c, AMGB_EINVAL, "bad arguments");
-   if (use_sval && !M.sval && !M.sell_sval) return amgb_fail(c, AMGB_EINVAL, "no scaled values for this matrix");
+   if (use_sval < 0 || use_sval > 4 || (use_sval > 1 && use_sval < 4 && kind != AMGB_MAT_A) || (use_sval == 4 && kind != AMGB_MAT_P))
+      return amgb_fail(c, AMGB_EINVAL, "bad arguments");
+   const bool sval = use_sval >= 1 && use_sval <= 3;
+   if (sval && !M.sval && !M.sell_sval) return amgb_fail(c, AMGB_EINVAL, "no scaled values for this matrix");
    const double *x = kind == AMGB_MAT_A ? c->r[level] : (kind == AMGB_MAT_P ? c->e[level + 1] : c->r[level]);
    double *y = kind == AMGB_MAT_A ? c->e[level] : (kind == AMGB_MAT_P ? c->t[level] : c->t[level + 1]);
    const double *rs = (c->opt.smoother == AMGB_SMOOTH_L1_JACOBI) ? c->inv_l1[level] : c->ws[level];
-   // 2: the symmetrised smoother's pass as the explicit cycle launches it; 3: the factorised restriction's pass (t and e)
-   const SpmvEpilogue e = use_sval == 2 ? epi(-1.0, 2.0, x, 0.0, nullptr, rs) : (use_sval == 3 ? epi(-1.0, 1.0, x) : epi(1.0, 0.0, nullptr));
-   double *y1 = use_sval == 3 ? c->t[level] : y, *y2 = use_sval == 3 ? c->e[level] : nullptr;
+   // 2: the symmetrised smoother's pass as the explicit cycle launches it; 3: the factorised restriction's pass (t and e);
+   // 4: the Horner prolongation's e_l += P_l e_{l+1} (in place, as enq_cycle launches it)
+   const SpmvEpilogue e = use_sval == 2 ? epi(-1.0, 2.0, x, 0.0, nullptr, rs)
+                          : (use_sval == 3 ? epi(-1.0, 1.0, x) : (use_sval == 4 ? epi(1.0, 1.0, c->e[level]) : epi(1.0, 0.0, nullptr)));
+   double *y1 = use_sval == 3 ? c->t[level] : (use_sval == 4 ? c->e[level] : y), *y2 = use_sval == 3 ? c->e[level] : nullptr;
    int grid;
-   for (int k = 0; k < 3; k++) c->launches += launch_spmv(c->cfg, c->stream, M, use_sval != 0, x, y1, e, nullptr, &grid, nullptr, y2, rs);
+   for (int k = 0; k < 3; k++) c->launches += launch_spmv(c->cfg, c->stream, M, sval, x, y1, e, nullptr, &grid, nullptr, y2, rs);
    CUDA_OK(c, cudaStreamSynchronize(c->stream));
    CUDA_OK(c, cudaEventRecord(c->ev0, c->stream));
-   for (int k = 0; k < reps; k++) c->launches += launch_spmv(c->cfg, c->stream, M, use_sval != 0, x, y1, e, nullptr, &grid, nullptr, y2, rs);
+   for (int k = 0; k < reps; k++) c->launches += launch_spmv(c->cfg, c->stream, M, sval, x, y1, e, nullptr, &grid, nullptr, y2, rs);
    CUDA_OK(c, cudaEventRecord(c->ev1, c->stream));
    CUDA_OK(c, cudaEventSynchronize(c->ev1));
    float ms = 0;
@@ -1370,6 +1377,53 @@ int amgb_time_spmv(amgb_ctx *c, int kind, int level, int use_sval, int reps, dou
    *ms_per_launch = ms / reps;
    CUDA_OK(c, cudaGetLastError());
    return AMGB_OK;
+}
+
+// one product with every epilogue operand launch_spmv takes, host in / host out (tests of the SpMV paths)
+int amgb_spmv_probe(amgb_ctx *c, int kind, int level, int use_sval, const double *coef, const double *x, const double *b,
+                    const double *cc, const double *rs, const double *b2, const double *xs, const double *w, int mode, double *y,
+                    double *y2, double *sum, int *window_path)
+{
+   NEED_READY(c);
+   if (level < 0 || level >= c->L || (kind != AMGB_MAT_A && level >= c->L - 1)) return amgb_fail(c, AMGB_EINVAL, "bad level");
+   const DevCSR &M = kind == AMGB_MAT_A ? c->A[level] : (kind == AMGB_MAT_P ? c->P[level] : c->R[level]);
+   if (!coef || !x || !y || mode < 0 || mode > 3 || (mode >= 2 && !w) || ((mode == 1 || mode == 2) && !sum) ||
+       (mode == 3 && (!b || !y2 || !use_sval)))
+      return amgb_fail(c, AMGB_EINVAL, "bad probe arguments");
+   if (use_sval && !M.sval && !M.sell_sval) return amgb_fail(c, AMGB_EINVAL, "no scaled values for this matrix");
+   const size_t nr = M.nrows, nc = M.ncols;
+   const double *host[8] = {x, b, cc, rs, b2, xs, mode == 1 ? nullptr : w, nullptr};
+   const size_t len[8] = {nc, nr, nr, nr, nr, nr, nr, nr};
+   double *dev[8] = {};
+   int rc = AMGB_OK;
+   double *dy = nullptr, *dy2 = nullptr;
+   for (int i = 0; i < 7 && rc == AMGB_OK; i++)
+      if (host[i]) {
+         if (cudaMalloc((void **)&dev[i], sizeof(double) * len[i]) != cudaSuccess) rc = AMGB_ECUDA;
+         else if (cudaMemcpyAsync(dev[i], host[i], sizeof(double) * len[i], cudaMemcpyHostToDevice, c->stream) != cudaSuccess) rc = AMGB_ECUDA;
+      }
+   if (rc == AMGB_OK && cudaMalloc((void **)&dy, sizeof(double) * nr) != cudaSuccess) rc = AMGB_ECUDA;
+   if (rc == AMGB_OK && mode == 3 && cudaMalloc((void **)&dy2, sizeof(double) * nr) != cudaSuccess) rc = AMGB_ECUDA;
+   if (rc == AMGB_OK) {
+      SpmvEpilogue e = epi(coef[0], coef[1], dev[1], coef[2], dev[2], dev[3]);
+      e.beta2 = coef[3]; e.b2 = dev[4];
+      e.xself = coef[4]; e.xs = dev[5];
+      int grid = 0;
+      if (window_path) *window_path = spmv_window_path(c->cfg, M) ? 1 : 0;
+      c->launches += launch_spmv(c->cfg, c->stream, M, use_sval != 0, dev[0], dy, e, mode == 1 || mode == 2 ? c->partials : nullptr,
+                                 &grid, mode == 2 ? dev[6] : nullptr, dy2, mode == 3 ? dev[6] : nullptr);
+      if (mode == 1 || mode == 2) c->launches += launch_reduce_partials(c->stream, c->partials, grid, c->d_scalars);
+      if (cudaMemcpyAsync(y, dy, sizeof(double) * nr, cudaMemcpyDeviceToHost, c->stream) != cudaSuccess) rc = AMGB_ECUDA;
+      if (rc == AMGB_OK && dy2 && cudaMemcpyAsync(y2, dy2, sizeof(double) * nr, cudaMemcpyDeviceToHost, c->stream) != cudaSuccess) rc = AMGB_ECUDA;
+      if (rc == AMGB_OK && (mode == 1 || mode == 2)) rc = amgb_fetch_scalar(c, sum);
+      if (rc == AMGB_OK && cudaStreamSynchronize(c->stream) != cudaSuccess) rc = AMGB_ECUDA;
+   }
+   cudaStreamSynchronize(c->stream);
+   for (double *p : dev) cudaFree(p);
+   cudaFree(dy);
+   cudaFree(dy2);
+   if (rc == AMGB_ECUDA) return amgb_fail(c, rc, "spmv probe: %s", cudaGetErrorString(cudaGetLastError()));
+   return rc;
 }
 
 // bytes of coarse-hierarchy data placed in the L2-pinned arena (the access-policy window of the persistent kernel)

@@ -15,8 +15,9 @@ constexpr int kBlock = 256;
 // One kernel per storage scheme (separate register budgets): MODE 0 = vector-per-row CSR, 1 = sliced ELL,
 // 2 = sliced ELL with the SELL-U encoding (stencil levels); the warp-stream CSR kernel is k_spmv_wstream.
 // DOT: the fused per-CTA partial is sum_i y_i * w_i instead of sum_i y_i^2; DUAL: the second output y2 = s2 o (b + y) (kernels.cuh).
-// Separate instantiations, so that the others keep their registers.
-template <int MODE, bool SVAL, bool DOT = false, bool DUAL = false>
+// Separate instantiations, so that the others keep their registers.  WIN (MODE 1 on SELL-C-sigma only): the epilogue in row
+// order through shared memory (sell_window_rows_cta; spmv_window_path says when).
+template <int MODE, bool SVAL, bool DOT = false, bool DUAL = false, bool WIN = false>
 __global__ void __launch_bounds__(kBlock, MODE == 2 ? 5 : 1) k_spmv(DevCSR M, const double *x, double *y, SpmvEpilogue e, double *partials,
                                                                     const double *w, double *y2, const double *s2)
 {
@@ -24,7 +25,11 @@ __global__ void __launch_bounds__(kBlock, MODE == 2 ? 5 : 1) k_spmv(DevCSR M, co
    const int tsz = gridDim.x * kBlock;
    const bool norm = partials != nullptr;
    double ss;
-   if (MODE == 2) ss = sell_rows_team<true, SVAL, 4, true, DOT, DUAL>(M, x, y, e, tid, tsz, norm, w, y2, s2);   // the cached-delta path, 5 CTAs per SM
+   if constexpr (WIN) {
+      static_assert(MODE == 1, "the window-staged epilogue is a path of the sliced-ELL kernel");
+      __shared__ double sacc[2 * kBlock];
+      ss = sell_window_rows_cta<kBlock, SVAL, DOT, DUAL>(M, x, y, e, norm, w, y2, s2, sacc);
+   } else if (MODE == 2) ss = sell_rows_team<true, SVAL, 4, true, DOT, DUAL>(M, x, y, e, tid, tsz, norm, w, y2, s2);   // the cached-delta path, 5 CTAs per SM
    else if (MODE == 1) ss = sell_rows_team<true, SVAL, 0, false, DOT, DUAL>(M, x, y, e, tid, tsz, norm, w, y2, s2);
    else ss = csr_rows_dispatch<true, SVAL, DOT, DUAL>(M, x, y, e, tid, tsz, norm, w, y2, s2);
    if (norm) {
@@ -269,25 +274,33 @@ static int resident_ctas(K kernel, int block, int num_sms, int *cache)
 }
 
 // (per instantiation: a function template has one set of statics per instantiation)
-template <int MODE, bool SVAL, bool DOT, bool DUAL = false>
+template <int MODE, bool SVAL, bool DOT, bool DUAL = false, bool WIN = false>
 static int spmv_mode_go(const LaunchCfg &cfg, cudaStream_t st, const DevCSR &M, const double *x, double *y, const SpmvEpilogue &e,
                         double *partials, long ctas_of_work, const double *w, double *y2 = nullptr, const double *s2 = nullptr)
 {
    static int occ = 0;
-   const int cap = resident_ctas(k_spmv<MODE, SVAL, DOT, DUAL>, kBlock, cfg.num_sms, &occ);
+   const int cap = resident_ctas(k_spmv<MODE, SVAL, DOT, DUAL, WIN>, kBlock, cfg.num_sms, &occ);
    const int grid = (int)std::max(1L, std::min(ctas_of_work, (long)cap));
-   k_spmv<MODE, SVAL, DOT, DUAL><<<grid, kBlock, 0, st>>>(M, x, y, e, partials, w, y2, s2);
+   k_spmv<MODE, SVAL, DOT, DUAL, WIN><<<grid, kBlock, 0, st>>>(M, x, y, e, partials, w, y2, s2);
    return grid;
 }
-template <int MODE>
+template <int MODE, bool WIN = false>
 static int launch_spmv_mode(const LaunchCfg &cfg, cudaStream_t st, const DevCSR &M, bool use_sval, const double *x, double *y,
                             const SpmvEpilogue &e, double *partials, long ctas_of_work, const double *w, double *y2, const double *s2)
 {
-   if (y2) return spmv_mode_go<MODE, true, false, true>(cfg, st, M, x, y, e, nullptr, ctas_of_work, nullptr, y2, s2);
-   if (w) return use_sval ? spmv_mode_go<MODE, true, true>(cfg, st, M, x, y, e, partials, ctas_of_work, w)
-                          : spmv_mode_go<MODE, false, true>(cfg, st, M, x, y, e, partials, ctas_of_work, w);
-   return use_sval ? spmv_mode_go<MODE, true, false>(cfg, st, M, x, y, e, partials, ctas_of_work, nullptr)
-                   : spmv_mode_go<MODE, false, false>(cfg, st, M, x, y, e, partials, ctas_of_work, nullptr);
+   if (y2) return spmv_mode_go<MODE, true, false, true, WIN>(cfg, st, M, x, y, e, nullptr, ctas_of_work, nullptr, y2, s2);
+   if (w) return use_sval ? spmv_mode_go<MODE, true, true, false, WIN>(cfg, st, M, x, y, e, partials, ctas_of_work, w)
+                          : spmv_mode_go<MODE, false, true, false, WIN>(cfg, st, M, x, y, e, partials, ctas_of_work, w);
+   return use_sval ? spmv_mode_go<MODE, true, false, false, WIN>(cfg, st, M, x, y, e, partials, ctas_of_work, nullptr)
+                   : spmv_mode_go<MODE, false, false, false, WIN>(cfg, st, M, x, y, e, partials, ctas_of_work, nullptr);
+}
+
+// The window-staged epilogue (sell_window_rows_cta) needs a SELL-C-sigma matrix whose sorting windows never straddle the
+// kBlock slots a CTA takes per iteration: sigma divides kBlock and the view starts at a multiple of kBlock / 32 slices.
+bool spmv_window_path(const LaunchCfg &cfg, const DevCSR &M)
+{
+   return M.sell_perm && !M.su_desc && M.sell_slices > 0 && cfg.sell_window_sigma > 1 && kBlock % cfg.sell_window_sigma == 0 &&
+          M.sell_base % (kBlock / 32) == 0;
 }
 
 template <bool SVAL, bool DOT, bool DUAL = false>
@@ -316,6 +329,8 @@ int launch_spmv(const LaunchCfg &cfg, cudaStream_t st, const DevCSR &M, bool use
 {
    int grid;
    if (M.sell_slices > 0 && M.su_desc) grid = launch_spmv_mode<2>(cfg, st, M, use_sval, x, y, e, partials, ((long)M.sell_slices * 32 + kBlock - 1) / kBlock, dot_w, y2, s2);
+   else if (spmv_window_path(cfg, M))
+      grid = launch_spmv_mode<1, true>(cfg, st, M, use_sval, x, y, e, partials, ((long)M.sell_slices * 32 + kBlock - 1) / kBlock, dot_w, y2, s2);
    else if (M.sell_slices > 0) grid = launch_spmv_mode<1>(cfg, st, M, use_sval, x, y, e, partials, ((long)M.sell_slices * 32 + kBlock - 1) / kBlock, dot_w, y2, s2);
    else if (M.nblk > 0) grid = launch_wstream(cfg, st, M, use_sval, x, y, e, partials, dot_w, y2, s2);
    else grid = launch_spmv_mode<0>(cfg, st, M, use_sval, x, y, e, partials, ((long)M.nrows * M.lpr + kBlock - 1) / kBlock, dot_w, y2, s2);
@@ -331,6 +346,9 @@ int launch_spmv_units(const LaunchCfg &cfg, cudaStream_t st, const DevCSR &M, in
 {
    if (grid_out) *grid_out = 0;
    if (u1 <= u0) return 0;
+   // a view that ends inside a CTA's slots would have the window-staged epilogue write rows of slots outside the view
+   LaunchCfg cv = cfg;
+   cv.sell_window_sigma = 0;
    DevCSR V = M;
    SpmvEpilogue ev = e;
    double *yv = y;
@@ -345,7 +363,7 @@ int launch_spmv_units(const LaunchCfg &cfg, cudaStream_t st, const DevCSR &M, in
       if (ev.xs) ev.xs += u0;
       if (dot_w) dot_w += u0;
    }
-   return launch_spmv(cfg, st, V, use_sval, x, yv, ev, partials, grid_out, dot_w);
+   return launch_spmv(cv, st, V, use_sval, x, yv, ev, partials, grid_out, dot_w);
 }
 
 int launch_reduce_partials(cudaStream_t st, const double *partials, int n, double *out)

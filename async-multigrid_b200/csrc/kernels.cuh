@@ -159,6 +159,52 @@ __device__ __forceinline__ double sell_rows_team(const DevCSR &M, const double *
    return sumsq;
 }
 
+// ---- SELL-C-sigma with the epilogue applied in row order (stand-alone kernel only) ---------------
+// Inside a window of sigma rows the rows are sorted by length, so in sell_rows_team lane l of a slice owns a row scattered over
+// the window, and every epilogue load and store is a warp access spread over up to 8 lines.  Here a CTA of NT threads takes the
+// NT / 32 consecutive slices [s0, s0 + NT / 32) per iteration: when sigma divides NT and the view starts at a multiple of
+// NT / 32 slices, their slots hold exactly the rows [32 (s0 + sell_base), + NT) (launch_spmv checks that).  Each lane sums
+// its row as sell_rows_team does (same entries, same order), parks the sum in shared memory at the row's place, and after a
+// barrier thread t applies the unchanged epilogue to the t-th row of the range: the epilogue's loads and stores are coalesced.
+// The trip count is CTA-uniform, so every thread reaches every barrier; the two halves of `sacc` ([2 * NT]) alternate, so one
+// barrier per iteration separates the writes of an iteration from the reads of the one before.
+template <int NT, bool SVAL, bool DOT = false, bool DUAL = false>
+__device__ __forceinline__ double sell_window_rows_cta(const DevCSR &M, const double *__restrict__ x, double *y,
+                                                       const SpmvEpilogue &e, bool want_sumsq, const double *dw, double *y2,
+                                                       const double *s2, double *sacc)
+{
+   constexpr int SPC = NT / 32;                        // slices per CTA and iteration
+   const int lane = threadIdx.x & 31;
+   const double *__restrict__ va = SVAL ? M.sell_sval : M.sell_va;
+   double sumsq = 0.0;
+   double *buf = sacc;
+   for (int s0 = blockIdx.x * SPC; s0 < M.sell_slices; s0 += gridDim.x * SPC) {
+      const int sl = s0 + (threadIdx.x >> 5);
+      const int base = (s0 + M.sell_base) << 5;        // first slot of the CTA's slices = first row of its windows
+      if (sl < M.sell_slices) {
+         const int row = __ldg(M.sell_perm + base + threadIdx.x);
+         const int off = __ldg(M.sell_off + sl);
+         const int width = (__ldg(M.sell_off + sl + 1) - off) >> 5;
+         const int *__restrict__ cp = M.sell_ci + off + lane;
+         const double *__restrict__ vp = va + off + lane;
+         double acc = 0.0;
+#pragma unroll 4
+         for (int k = 0; k < width; k++) acc += ld_stream(vp + (k << 5)) * ld_x<true>(x + ld_stream(cp + (k << 5)));
+         if (row >= 0 && row < M.nrows) buf[row - base] = acc;
+      }
+      __syncthreads();
+      const int row = base + threadIdx.x;
+      if (row < M.nrows) {
+         const double v = epilogue_apply<true>(e, row, buf[threadIdx.x]);
+         epilogue_store<true>(e, y, row, v);
+         if (want_sumsq) sumsq += DOT ? v * __ldg(dw + row) : v * v;
+         if (DUAL) y2[row] = __ldg(s2 + row) * (e.b[row] + v);
+      }
+      buf = buf == sacc ? sacc + NT : sacc;
+   }
+   return sumsq;
+}
+
 // ---- warp-stream: CSR row chunks at warp granularity, no CTA-wide barriers -----------------------
 // Every WARP owns every team_nwarps-th row chunk (DevCSR::blk, <= AMGB_WARP_CHUNK entries).
 // Lanes load the chunk's (col,val) pairs coalesced (consecutive lanes = consecutive entries, all 2*EPT

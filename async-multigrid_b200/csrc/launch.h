@@ -8,6 +8,7 @@
 struct LaunchCfg {
    int num_sms = 148;
    int ctas_per_sm = 8;
+   int sell_window_sigma = 0;        // sigma of the SELL-C-sigma matrices when amgb_options.sell_window_epilogue is on, else 0
 };
 
 // y = gamma*c + rs.*(beta*b + alpha*M*x); optional sum of y_i^2 -- or of y_i*dot_w_i when dot_w is given -- into partial
@@ -16,6 +17,8 @@ struct LaunchCfg {
 int launch_spmv(const LaunchCfg &cfg, cudaStream_t st, const DevCSR &M, bool use_sval, const double *x, double *y,
                 const SpmvEpilogue &e, double *partials, int *grid_out, const double *dot_w = nullptr, double *y2 = nullptr,
                 const double *s2 = nullptr);
+// true when launch_spmv runs M on the window-staged SELL-C-sigma path (epilogue in row order through shared memory)
+bool spmv_window_path(const LaunchCfg &cfg, const DevCSR &M);
 int spmv_units(const DevCSR &M);
 int launch_spmv_units(const LaunchCfg &cfg, cudaStream_t st, const DevCSR &M, int u0, int u1, bool use_sval, const double *x,
                       double *y, const SpmvEpilogue &e, double *partials, int *grid_out, const double *dot_w = nullptr);

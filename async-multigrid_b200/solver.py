@@ -24,7 +24,7 @@ ABI_SYMBOLS = [
     "amgb_set_num_levels", "amgb_set_matrix", "amgb_set_options", "amgb_setup",
     "amgb_set_rhs", "amgb_set_solution", "amgb_get_solution", "amgb_get_residual",
     "amgb_spgemv", "amgb_spgemv_transpose", "amgb_smooth", "amgb_set_jgs_blocks", "amgb_norm2", "amgb_cycle", "amgb_eigs_power", "amgb_solve_sync", "amgb_solve_async",
-    "amgb_async_groups", "amgb_solve_extended", "amgb_solve_extended_async", "amgb_smooth_transfer", "amgb_host_csr_free", "amgb_smem_solve", "amgb_time_residual", "amgb_level_storage", "amgb_time_spmv", "amgb_l2_arena_bytes", "amgb_sellu_stats",
+    "amgb_async_groups", "amgb_solve_extended", "amgb_solve_extended_async", "amgb_smooth_transfer", "amgb_host_csr_free", "amgb_smem_solve", "amgb_time_residual", "amgb_level_storage", "amgb_time_spmv", "amgb_spmv_probe", "amgb_l2_arena_bytes", "amgb_sellu_stats",
     "amgb_sellu_encode_host", "amgb_host_free", "amgb_async_program", "amgb_async_group_times",
     "amgb_solve_extended_implicit_async", "amgb_ext_async_program", "amgb_solve_pcg",
     "amgb_dist_unique_id", "amgb_dist_init", "amgb_dist_set_level", "amgb_dist_setup", "amgb_dist_set_rhs",
@@ -43,7 +43,7 @@ class Options(C.Structure):
                 ("jgs_block_rows", C.c_int), ("use_sell", C.c_int), ("l2_persist", C.c_int), ("use_stream", C.c_int),
                 ("factor_level0", C.c_int), ("coarse_solve", C.c_int), ("sell_sigma", C.c_int), ("stream_variant", C.c_int),
                 ("sell_uniform", C.c_int), ("async_type", C.c_int), ("res_compute_type", C.c_int), ("read_type", C.c_int),
-                ("lean_storage", C.c_int), ("factor_restriction", C.c_int)]
+                ("lean_storage", C.c_int), ("factor_restriction", C.c_int), ("sell_window_epilogue", C.c_int)]
 
 
 class HostCSR(C.Structure):
@@ -101,6 +101,7 @@ def load_library():
     L.amgb_time_residual.argtypes = [C.c_void_p, C.c_int, DP]
     L.amgb_level_storage.argtypes = [C.c_void_p, C.c_int, C.c_int, IP]
     L.amgb_time_spmv.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, DP]
+    L.amgb_spmv_probe.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, DP, DP, DP, DP, DP, DP, DP, DP, C.c_int, DP, DP, DP, IP]
     L.amgb_l2_arena_bytes.argtypes = [C.c_void_p, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)]
     L.amgb_sellu_stats.argtypes = [C.c_void_p, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)]
     L.amgb_async_groups.argtypes = [C.c_void_p, IP, IP]
@@ -153,10 +154,13 @@ class Solver:
     def __init__(self, h, solver=H.MULTADD, smoother=H.JACOBI, smooth_weight=1.0, num_pre=1, num_post=1,
                  fine_sweeps=1, coarse_sweeps=1, jgs_block_rows=8, use_sell=True, l2_persist=True, use_stream=True,
                  sell_sigma=None, coarse_solve=False, factor_level0=False, device=0, jgs_blocks=None,
-                 sell_uniform=None, async_type=0, res_compute_type=0, read_type=0, lean_storage=False, factor_restriction=None):
+                 sell_uniform=None, async_type=0, res_compute_type=0, read_type=0, lean_storage=False, factor_restriction=None,
+                 sell_window_epilogue=None):
         """factor_restriction (amgb_options.factor_restriction): None = on exactly where amgb_setup accepts it, i.e. with
         factor_level0 for the synchronous Multadd cycle with the symmetrised (L1-)Jacobi smoother and one fine sweep; the
-        plain P_l^T (Hierarchy.plain_restriction) is then uploaded for the levels l >= 1 in place of h.R[l], which stays as it is"""
+        plain P_l^T (Hierarchy.plain_restriction) is then uploaded for the levels l >= 1 in place of h.R[l], which stays as it is.
+        sell_window_epilogue (amgb_options.sell_window_epilogue): None = the library's default (on); False = the SELL-C-sigma
+        products apply their epilogue at the sorted slot instead of in row order (same results, for A/B timing)"""
         self.L = load_library()
         self.h = h
         self.ctx = C.c_void_p()
@@ -188,6 +192,8 @@ class Solver:
             factor_restriction = (factor_level0 and solver == H.MULTADD and smoother in (H.JACOBI, H.L1_JACOBI) and num_pre > 0
                                   and num_post > 0 and fine_sweeps == 1)
         o.factor_restriction = int(factor_restriction)
+        if sell_window_epilogue is not None:
+            o.sell_window_epilogue = int(sell_window_epilogue)
         self.options = o
         self._ck(self.L.amgb_set_options(self.ctx, C.byref(o)))
         self._ck(self.L.amgb_set_num_levels(self.ctx, h.num_levels))
@@ -390,6 +396,25 @@ class Solver:
         ms = C.c_double(0)
         self._ck(self.L.amgb_time_spmv(self.ctx, kind, level, int(use_sval), reps, C.byref(ms)))
         return ms.value
+
+    def spmv_probe(self, kind, level, x, alpha=1.0, b=None, beta=0.0, c=None, gamma=0.0, rs=None, b2=None, beta2=0.0,
+                   xs=None, xself=0.0, use_sval=False, norm=False, dot_w=None, dual_s2=None):
+        """y = gamma c + rs o (beta b + beta2 b2 + alpha M x) + xself xs through the solve's SpMV kernels (amgb_spmv_probe).
+        norm: also sum y_i^2; dot_w: also sum y_i dot_w_i; dual_s2 (column-scaled values, b given): also y2 = dual_s2 o (b + y).
+        Returns (y, y2 or None, sum or None, whether the window-staged SELL-C-sigma kernel ran)."""
+        m = {MAT_A: self.h.A, MAT_P: self.h.P, MAT_R: self.h.R}[kind][level]
+        vec = lambda v: None if v is None else np.ascontiguousarray(v, dtype=np.float64)
+        x, b, c, rs, b2, xs = vec(x), vec(b), vec(c), vec(rs), vec(b2), vec(xs)
+        w = vec(dot_w if dot_w is not None else dual_s2)
+        mode = 3 if dual_s2 is not None else (2 if dot_w is not None else (1 if norm else 0))
+        coef = np.array([alpha, beta, gamma, beta2, xself], dtype=np.float64)
+        y = np.empty(m.nrows)
+        y2 = np.empty(m.nrows) if mode == 3 else None
+        ss, win = C.c_double(0), C.c_int(0)
+        p = lambda v: None if v is None else _dp(v)
+        self._ck(self.L.amgb_spmv_probe(self.ctx, kind, level, int(use_sval), _dp(coef), _dp(x), p(b), p(c), p(rs), p(b2), p(xs),
+                                        p(w), mode, _dp(y), p(y2), C.byref(ss), C.byref(win)))
+        return y, y2, (ss.value if mode in (1, 2) else None), bool(win.value)
 
     def l2_arena_bytes(self):
         a, b = C.c_longlong(0), C.c_longlong(0)

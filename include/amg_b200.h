@@ -91,6 +91,10 @@ typedef struct {
                                    A_l that the level's smoother makes anyway writes t_l = r_l - A_l diag(s) r_l beside e_l = s o (r_l + t_l),
                                    then r_{l+1} = R_l t_l.  P_l stay the explicit Pbar_l.  Same operator, rounding-level differences;
                                    AMGB_EINVAL from amgb_setup where the algebra does not hold.  0 (default): explicit Rbar_l */
+   int sell_window_epilogue;    /* 1 (default): the products with a SELL-C-sigma matrix (sell_sigma dividing 256) park every row sum in
+                                   shared memory and apply the epilogue (operand loads, stores of y) in row order, coalesced, instead
+                                   of at the row's sorted slot.  The same arithmetic per row: identical results; only the order of the
+                                   fused per-CTA norm / dot partial sums differs.  0: the epilogue at the slot */
 } amgb_options;
 
 void amgb_default_options(amgb_options *opt);
@@ -261,8 +265,16 @@ int amgb_time_residual(amgb_ctx *ctx, int reps, double *ms_per_launch);
 int amgb_level_storage(amgb_ctx *ctx, int kind, int level, int *is_sell);
 /* event-timed y = M x for one matrix of the hierarchy (tools/spmv_sweep.py).  use_scaled_values:
  * 0 the values, 1 the column-scaled values; A_l only: 2 the symmetrised smoother's pass e = s o (2x - (A diag(s)) x) of the
- * explicit cycle, 3 the factorised restriction's pass t = x - (A diag(s)) x, e = s o (x + t) (amgb_options.factor_restriction) */
+ * explicit cycle, 3 the factorised restriction's pass t = x - (A diag(s)) x, e = s o (x + t) (amgb_options.factor_restriction);
+ * P_l only: 4 the prolongation's e_l += P_l e_{l+1} (in place) */
 int amgb_time_spmv(amgb_ctx *ctx, int kind, int level, int use_scaled_values, int reps, double *ms_per_launch);
+/* One product y = gamma c + rs o (beta b + beta2 b2 + alpha M x) + xself xs through the solve's SpMV kernels, host in / host out,
+ * for tests of the kernel paths.  coef = {alpha, beta, gamma, beta2, xself}; b, c, rs, b2, xs may be NULL (term absent).
+ * mode 0: y only; 1: also *sum = sum_i y_i^2; 2: also *sum = sum_i y_i w_i; 3 (use_scaled_values = 1, b given): also
+ * y2 = w o (b + y).  *window_path (may be NULL): 1 when the window-staged SELL-C-sigma kernel ran (sell_window_epilogue) */
+int amgb_spmv_probe(amgb_ctx *ctx, int kind, int level, int use_scaled_values, const double *coef, const double *x, const double *b,
+                    const double *c, const double *rs, const double *b2, const double *xs, const double *w, int mode, double *y,
+                    double *y2, double *sum, int *window_path);
 /* slices stored in the SELL-U encoding (amgb_options.sell_uniform) and their (delta, mask, value) groups */
 int amgb_sellu_stats(amgb_ctx *ctx, long long *slices, long long *groups);
 /* Host-only probe of the SELL-U encoder (no CUDA call; CPU test suite): CSR + column-scaled values in; out, per slice, the
