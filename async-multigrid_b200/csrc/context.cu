@@ -521,7 +521,7 @@ int amgb_set_matrix(amgb_ctx *c, int kind, int level, int nrows, int ncols, int 
    }
    // DMEM convention: dense inverse of the coarsest operator (hypre_GaussElimSetup, src/DMEM_Setup.cpp:385-388),
    // applied later as one full SpMV
-   if (kind == AMGB_MAT_A && level == c->L - 1 && c->opt.coarse_solve && c->L > 1) {
+   if (kind == AMGB_MAT_A && level == c->L - 1 && c->opt.coarse_solve && c->L > 1 && !amgb_dist_level_distributed(c, level)) {
       const int n = nrows;
       if (n > 2048) return amgb_fail(c, AMGB_EINVAL, "coarsest level has %d rows: too large for the dense direct solve", n);
       std::vector<double> Mx((size_t)n * 2 * n, 0.0);         // [A | I]

@@ -227,6 +227,94 @@ static int dist_cycle(amgb_ctx *c, double *tgt, bool accumulate)
    }
    return AMGB_OK;
 }
+
+// `sweeps` (L1-)Jacobi sweeps u <- u + s o (f - A_l u) on level l.  u (level layout) starts in *cur, one of the level's two
+// buffers a / b, and ping-pongs between them; *cur names the buffer that holds the result.  f: the level's rows.
+static int dist_sweeps(amgb_ctx *c, int l, const double *f, double **cur, double *a, double *b, int sweeps)
+{
+   DistState *d = c->dist;
+   const int off = d->lv[l].off();
+   const double *s = d->ws[l] + off;
+   int rc;
+   for (int k = 0; k < sweeps; k++) {
+      double *nxt = *cur == a ? b : a;
+      if ((rc = dist_spmv(c, c->A[l], false, l, *cur, nxt + off, epi(-1.0, 1.0, f, 1.0, *cur + off, s), false))) return rc;
+      *cur = nxt;
+   }
+   return AMGB_OK;
+}
+
+// One multiplicative V-cycle on (f, u) of level 0, row-partitioned: SMEM_Sync_Parfor_Vcycle (src/SMEM_Sync_AMG.cpp:8-145) with
+// the meaning and the quirks of enq_vcycle (context.cu) -- level right-hand sides in r[l], level solutions in e[l] (l >= 1), the
+// first pre-sweep of levels 1..L-2 from a zero guess, the coarsest level's num_pre + num_post sweeps continuing from what the
+// previous cycle left in e[L-1], or with coarse_solve DMEM_MultCycle's direct solve there (src/DMEM_Mult.cpp:207).  Every SpMV
+// that reads a distributed vector exchanges its ghosts first (dist_spmv); the restricted residual of the first replicated level
+// is all-gathered as in dist_cycle.  A level's iterate ping-pongs between its home buffer and t[l]; the prolongation writes
+// into whichever of the two makes the post-sweeps end in the home buffer, so only the coarsest level (whose iterate must
+// persist across cycles) may need a copy.
+static int dist_vcycle(amgb_ctx *c)
+{
+   DistState *d = c->dist;
+   const int L = c->L;
+   const int pre = c->opt.num_pre_smooth_sweeps, post = c->opt.num_post_smooth_sweeps;
+   int rc;
+   auto rhs = [&](int l) -> const double * { return l == 0 ? d->f : d->r[l] + d->lv[l].off(); };
+   auto home = [&](int l) -> double * { return l == 0 ? d->u : d->e[l]; };
+   std::vector<double *> down((size_t)L);                    // where each level's iterate is after the pre-smoothing
+   for (int l = 0; l < L - 1; l++) {
+      const DistLevel &lv = d->lv[l], &nx = d->lv[l + 1];
+      const int off = lv.off();
+      const double *f = rhs(l);
+      double *cur = home(l);
+      if (l > 0 && pre > 0) {
+         // zero guess: u = s o f; with one sweep the residual f - A (s o f) comes from the column-scaled values (ghosts of f)
+         c->launches += launch_scale(c->cfg, c->stream, c->A[l].nrows, d->ws[l] + off, f, cur + off);
+         if (pre == 1) {
+            if ((rc = dist_spmv(c, c->A[l], true, l, d->r[l], d->w[l] + off, epi(-1.0, 1.0, f), false))) return rc;
+         } else {
+            if ((rc = dist_sweeps(c, l, f, &cur, home(l), d->t[l], pre - 1))) return rc;
+            if ((rc = dist_spmv(c, c->A[l], false, l, cur, d->w[l] + off, epi(-1.0, 1.0, f), false))) return rc;
+         }
+      } else {
+         // level 0 continues from the current u; with no pre-sweep a coarser level keeps the previous cycle's iterate
+         if ((rc = dist_sweeps(c, l, f, &cur, home(l), d->t[l], pre))) return rc;
+         if ((rc = dist_spmv(c, c->A[l], false, l, cur, d->w[l] + off, epi(-1.0, 1.0, f), false))) return rc;
+      }
+      down[l] = cur;
+      const bool gather = lv.distributed && !nx.distributed;
+      double *out = d->r[l + 1] + (gather ? nx.row_start : nx.off());
+      if ((rc = dist_spmv(c, c->R[l], false, l, d->w[l], out, epi(1.0, 0.0, nullptr), false))) return rc;
+      if (gather && (rc = allgather_level(c, l + 1, d->r[l + 1]))) return rc;
+   }
+   {
+      const int cl = L - 1, off = d->lv[cl].off();
+      if (c->opt.coarse_solve && c->Ainv.rp) {
+         enq_spmv(c, c->Ainv, false, d->r[cl], d->e[cl], epi(1.0, 0.0, nullptr), false);     // replicated level (amgb_dist_setup)
+      } else {
+         double *cur = home(cl);
+         if ((rc = dist_sweeps(c, cl, rhs(cl), &cur, home(cl), d->t[cl], pre + post))) return rc;
+         if (cur != home(cl))
+            CUDA_OK(c, cudaMemcpyAsync(home(cl) + off, cur + off, sizeof(double) * c->A[cl].nrows, cudaMemcpyDeviceToDevice, c->stream));
+      }
+   }
+   for (int l = L - 2; l >= 0; l--) {
+      const int off = d->lv[l].off();
+      // u_l += P_l u_{l+1} (ghosts of u_{l+1} when level l+1 is distributed), written where the post-sweeps end in home(l)
+      double *cur = (post & 1) ? d->t[l] : home(l);
+      if ((rc = dist_spmv(c, c->P[l], false, l + 1, home(l + 1), cur + off, epi(1.0, 1.0, down[l] + off), false))) return rc;
+      if ((rc = dist_sweeps(c, l, rhs(l), &cur, home(l), d->t[l], post))) return rc;
+   }
+   return AMGB_OK;
+}
+
+// one iteration of the synchronous solve without acceleration: the cycle on u, then r = f - A u and its all-reduced norm
+static int dist_iteration(amgb_ctx *c)
+{
+   int rc;
+   if (c->opt.solver == AMGB_SOLVER_MULT) rc = dist_vcycle(c);
+   else rc = dist_cycle(c, c->dist->u + c->dist->lv[0].off(), true);
+   return rc ? rc : dist_residual(c);
+}
 #endif   // AMG_HAVE_NCCL
 
 extern "C" {
@@ -299,9 +387,16 @@ int amgb_dist_setup(amgb_ctx *c)
    if (d->ready) return amgb_fail(c, AMGB_ESTATE, "amgb_dist_setup already done");
    const int L = c->L;
    const amgb_options &o = c->opt;
-   if ((o.solver != AMGB_SOLVER_MULTADD && o.solver != AMGB_SOLVER_BPX && o.solver != AMGB_SOLVER_AFACX) ||
+   const bool mult = o.solver == AMGB_SOLVER_MULT;
+   if (mult && o.smoother != AMGB_SMOOTH_JACOBI && o.smoother != AMGB_SMOOTH_L1_JACOBI)
+      return amgb_fail(c, AMGB_EINVAL, "partitioned MULT smooths with weighted or L1 Jacobi: smoother %d (hybrid JGS or a Gauss-Seidel "
+                                       "type) is not implemented on the partitioned path", o.smoother);
+   if ((o.solver != AMGB_SOLVER_MULTADD && o.solver != AMGB_SOLVER_BPX && o.solver != AMGB_SOLVER_AFACX && !mult) ||
        (o.smoother != AMGB_SMOOTH_JACOBI && o.smoother != AMGB_SMOOTH_L1_JACOBI))
-      return amgb_fail(c, AMGB_EINVAL, "the partitioned path implements synchronous Multadd, AFACx and BPX with weighted or L1 Jacobi");
+      return amgb_fail(c, AMGB_EINVAL, "the partitioned path implements synchronous Multadd, AFACx, BPX and MULT with weighted or L1 Jacobi");
+   if (mult && (o.num_pre_smooth_sweeps < 0 || o.num_post_smooth_sweeps < 0 || o.num_pre_smooth_sweeps + o.num_post_smooth_sweeps < 1))
+      return amgb_fail(c, AMGB_EINVAL, "partitioned MULT needs num_pre_smooth_sweeps >= 0, num_post_smooth_sweeps >= 0, one of them positive");
+   if (mult && (o.coarse_solve < 0 || o.coarse_solve > 1)) return amgb_fail(c, AMGB_EINVAL, "coarse_solve must be 0 or 1");
    if (o.solver == AMGB_SOLVER_BPX && o.num_pre_smooth_sweeps != 1)
       return amgb_fail(c, AMGB_EINVAL, "partitioned BPX runs one Jacobi sweep per level");
    if (o.solver == AMGB_SOLVER_AFACX && (o.num_fine_smooth_sweeps != 1 || o.num_coarse_smooth_sweeps != 1 || o.coarse_solve))
@@ -310,6 +405,9 @@ int amgb_dist_setup(amgb_ctx *c)
       return amgb_fail(c, AMGB_EINVAL, "partitioned Multadd runs one smoothing sweep per level");
    const bool l1s = o.smoother == AMGB_SMOOTH_L1_JACOBI;
    if ((int)d->lv.size() != L) return amgb_fail(c, AMGB_ESTATE, "level layouts missing");
+   // (amgb_set_matrix builds no inverse of a partitioned row block)
+   if (o.coarse_solve && L > 1 && d->lv[L - 1].distributed)
+      return amgb_fail(c, AMGB_EINVAL, "coarse_solve (direct coarsest solve) needs a replicated coarsest level; level %d is distributed", L - 1);
    int rc;
    for (int l = 0; l < L; l++) {
       const DistLevel &lv = d->lv[l];
@@ -332,7 +430,7 @@ int amgb_dist_setup(amgb_ctx *c)
       if ((rc = amgb_dev_alloc_bytes(c, (void **)&d->ws[l], bytes, true))) return rc;
       if ((rc = amgb_dev_alloc_bytes(c, (void **)&d->r[l], bytes, true))) return rc;
       if ((rc = amgb_dev_alloc_bytes(c, (void **)&d->e[l], bytes, true))) return rc;
-      if (o.solver == AMGB_SOLVER_AFACX) {
+      if (o.solver == AMGB_SOLVER_AFACX || mult) {
          if ((rc = amgb_dev_alloc_bytes(c, (void **)&d->t[l], bytes, true))) return rc;
          if ((rc = amgb_dev_alloc_bytes(c, (void **)&d->w[l], bytes, true))) return rc;
       }
@@ -409,6 +507,9 @@ int amgb_dist_solve_sync_accel(amgb_ctx *c, double tol, int max_cycles, int acce
    DistState *d = c->dist;
    if (!d || !d->ready) return amgb_fail(c, AMGB_ESTATE, "amgb_dist_setup not called");
    if (max_cycles < 0 || accel < 0 || accel > 2) return amgb_fail(c, AMGB_EINVAL, "bad arguments");
+   const bool mult = c->opt.solver == AMGB_SOLVER_MULT;
+   if (mult && accel)
+      return amgb_fail(c, AMGB_EINVAL, "accel %d: DMEM_ChebyUpdate accelerates the additive correction, not the MULT V-cycle", accel);
    int rc;
    const int nown = c->A[0].nrows;
    double *uo = d->u + d->lv[0].off();
@@ -418,6 +519,8 @@ int amgb_dist_solve_sync_accel(amgb_ctx *c, double tol, int max_cycles, int acce
    }
    double c_prev = 1.0, c_cur = mu;
    CUDA_OK(c, cudaMemsetAsync(d->u, 0, sizeof(double) * (size_t)d->lv[0].n_ext(), c->stream));
+   if (mult)     // the level iterates of the V-cycle start from zero in every solve (the coarsest one carries over between cycles)
+      for (int l = 1; l < c->L; l++) CUDA_OK(c, cudaMemsetAsync(d->e[l], 0, sizeof(double) * (size_t)d->lv[l].n_ext(), c->stream));
    if ((rc = dist_residual(c))) return rc;
    double ss;
    if ((rc = amgb_fetch_scalar(c, &ss))) return rc;
@@ -433,8 +536,7 @@ int amgb_dist_solve_sync_accel(amgb_ctx *c, double tol, int max_cycles, int acce
       cudaGraph_t g;
       const long long l0 = c->launches, h0 = d->halo_bytes, c0 = d->collectives;
       CUDA_OK(c, cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal));
-      rc = dist_cycle(c, uo, true);
-      if (!rc) rc = dist_residual(c);
+      rc = dist_iteration(c);
       cudaMemcpyAsync(c->h_scalars, c->d_scalars, sizeof(double), cudaMemcpyDeviceToHost, c->stream);
       cudaError_t ce = cudaStreamEndCapture(c->stream, &g);
       if (rc) return rc;
@@ -467,7 +569,7 @@ int amgb_dist_solve_sync_accel(amgb_ctx *c, double tol, int max_cycles, int acce
          continue;
       }
       if (!accel) {
-         if ((rc = dist_cycle(c, uo, true))) return rc;
+         if ((rc = dist_iteration(c))) return rc;
       } else {
          if ((rc = dist_cycle(c, d->ecyc, false))) return rc;
          if (k == 1) c->launches += launch_axpby(c->cfg, c->stream, nown, 1.0, d->ecyc, 0.0, d->dacc, nullptr);
@@ -483,8 +585,8 @@ int amgb_dist_solve_sync_accel(amgb_ctx *c, double tol, int max_cycles, int acce
             c->launches += launch_axpby(c->cfg, c->stream, nown, omega * delta, d->ecyc, omega - 1.0, d->dacc, nullptr);
          }
          c->launches += launch_add(c->cfg, c->stream, nown, d->dacc, uo);
+         if ((rc = dist_residual(c))) return rc;
       }
-      if ((rc = dist_residual(c))) return rc;
       if ((rc = amgb_fetch_scalar(c, &ss))) return rc;
       done = k;
       const double rel = sqrt(ss) / r0;
@@ -496,8 +598,7 @@ int amgb_dist_solve_sync_accel(amgb_ctx *c, double tol, int max_cycles, int acce
          cudaGraph_t g;
          const long long l0 = c->launches, h0 = d->halo_bytes, c0 = d->collectives;
          CUDA_OK(c, cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal));
-         rc = dist_cycle(c, uo, true);
-         if (!rc) rc = dist_residual(c);
+         rc = dist_iteration(c);
          cudaMemcpyAsync(c->h_scalars, c->d_scalars, sizeof(double), cudaMemcpyDeviceToHost, c->stream);
          cudaError_t ce = cudaStreamEndCapture(c->stream, &g);
          if (rc) return rc;
@@ -537,6 +638,8 @@ int amgb_dist_eigs_power(amgb_ctx *c, int iters, const double *u0_owned, double 
    DistState *d = c->dist;
    if (!d || !d->ready) return amgb_fail(c, AMGB_ESTATE, "amgb_dist_setup not called");
    if (iters < 1 || !eig_min || !eig_max) return amgb_fail(c, AMGB_EINVAL, "bad arguments");
+   if (c->opt.solver == AMGB_SOLVER_MULT)
+      return amgb_fail(c, AMGB_EINVAL, "DMEM_PowerMult applies the additive cycles: the MULT V-cycle has no zero-guess linear form here");
    int rc;
    const int nown = c->A[0].nrows, off0 = d->lv[0].off();
    if (!d->ecyc) {

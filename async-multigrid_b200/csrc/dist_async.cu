@@ -541,6 +541,7 @@ extern "C" int amgb_dist_solve_async(amgb_ctx *c, int num_cycles, int *correctio
    DistState *d = c->dist;
    if (!d || !d->ready) return amgb_fail(c, AMGB_ESTATE, "amgb_dist_setup not called");
    if (num_cycles < 1) return amgb_fail(c, AMGB_EINVAL, "num_cycles < 1");
+   if (c->opt.solver == AMGB_SOLVER_MULT) return amgb_fail(c, AMGB_EINVAL, "there is no asynchronous MULT: DMEM_Add_async runs Multadd or AFACx");
    if (c->opt.coarse_solve && c->L > 1 && !c->Ainv.rp) return amgb_fail(c, AMGB_ESTATE, "coarse_solve: the inverse of the coarsest operator was not built");
    int rc;
    if ((rc = dist_async_prepare(c))) return rc;

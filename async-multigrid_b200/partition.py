@@ -180,24 +180,36 @@ class RankPlan:
 
 
 # ---------------------------------------------------------------------------------------------------
-# numpy / gloo executor of the distributed synchronous Multadd cycle (tests; mirrors csrc/dist.cu)
+# numpy / gloo executor of the distributed synchronous cycles (tests; mirrors csrc/dist.cu)
 # ---------------------------------------------------------------------------------------------------
 class DistEmulator:
     """Runs the plan with numpy kernels; communication through a `comm` object with
-    sendrecv(send_lo, send_hi, n_lo, n_hi) -> (from_lo, from_hi), allgatherv(x, counts) and allreduce_sum(v)."""
+    sendrecv(send_lo, send_hi, n_lo, n_hi) -> (from_lo, from_hi), allgatherv(x, counts) and allreduce_sum(v).
+    solver: Multadd, AFACx or BPX (`cycle`, one sweep per level) or MULT (`vcycle`, num_pre / num_post sweeps, coarse_solve:
+    direct solve on the replicated coarsest level).  `counts` tallies the halo exchanges (of distributed levels), all-gathers
+    and all-reduces; `per_cycle` the collectives of every iteration of the last `solve` (cycle + residual norm)."""
 
-    def __init__(self, plan, comm, smooth_weight, solver=H.MULTADD, smoother=H.JACOBI, symmetric=True):
+    def __init__(self, plan, comm, smooth_weight, solver=H.MULTADD, smoother=H.JACOBI, symmetric=True, num_pre=1, num_post=1,
+                 coarse_solve=False):
         import scipy.sparse as sp
         self.pl, self.comm, self.w = plan, comm, smooth_weight
         self.solver, self.smoother = solver, smoother
         self.symmetric = bool(symmetric) and solver == H.MULTADD
+        self.num_pre, self.num_post = int(num_pre), int(num_post)
+        self.coarse_solve = bool(coarse_solve) and plan.num_levels > 1
+        if self.coarse_solve and plan.layouts[-1].distributed:
+            raise ValueError("coarse_solve needs a replicated coarsest level")
+        self.counts = {"halo": 0, "allgather": 0, "allreduce": 0}
+        self.per_cycle = []
         self.sp = sp
         self.A = [m.to_scipy() for m in plan.A]
         self.P = [m.to_scipy() for m in plan.P]
         self.R = [m.to_scipy() for m in plan.R]
+        self.Ac = self.A[-1].toarray() if self.coarse_solve else None
         # omega/d (1/l1 for L1-Jacobi: the row sums of a local row block are the global ones) in the level's vector
         # layout (ghosts filled by one halo exchange at setup)
         self.ws = []
+        self.e = [self.new_vec(l) for l in range(plan.num_levels)]     # level iterates of the V-cycle (l >= 1)
         for l, lay in enumerate(plan.layouts):
             v = self.new_vec(l)
             if smoother == H.L1_JACOBI:
@@ -206,6 +218,7 @@ class DistEmulator:
                 self.owned(l, v)[:] = smooth_weight / plan.A[l].data[plan.A[l].indptr[:-1]]
             self.halo(l, v)
             self.ws.append(v)
+        self.counts["halo"] = 0
 
     def new_vec(self, l):
         return np.zeros(self.pl.layouts[l].n_ext)
@@ -218,6 +231,7 @@ class DistEmulator:
         lay = self.pl.layouts[l]
         if not lay.distributed:
             return
+        self.counts["halo"] += 1
         o = self.owned(l, v)
         lo, hi = self.comm.sendrecv(o[:lay.send_lo].copy(), o[lay.n_owned - lay.send_hi:].copy(), lay.halo_lo, lay.halo_hi)
         v[:lay.halo_lo] = lo
@@ -237,6 +251,52 @@ class DistEmulator:
         self.owned(l, e)[:] = self.owned(l, self.ws[l]) * self.owned(l, r)
         return e
 
+    def restrict(self, l, v):
+        """R_l v (ghosts of v) as a level-(l+1) vector, owned part valid; all-gathered whole at the first replicated level"""
+        self.halo(l, v)
+        y = self.R[l] @ v
+        out = self.new_vec(l + 1)
+        if self.pl.layouts[l + 1].distributed or not self.pl.layouts[l].distributed:
+            self.owned(l + 1, out)[:] = y
+        else:
+            self.counts["allgather"] += 1
+            out[:] = self.comm.allgatherv(y, self.pl.all_counts[l + 1])
+        return out
+
+    def sweeps(self, l, f, u, k):
+        """k (L1-)Jacobi sweeps u <- u + s o (f - A_l u) on the owned rows, in place; ghosts refreshed before every sweep"""
+        s = self.owned(l, self.ws[l])
+        for _ in range(k):
+            self.halo(l, u)
+            self.owned(l, u)[:] = self.owned(l, u) + s * (f - self.A[l] @ u)
+
+    def vcycle(self, f, u):
+        """one multiplicative V-cycle (SMEM_Sync_Parfor_Vcycle, src/SMEM_Sync_AMG.cpp:8-145; DMEM_MultCycle with coarse_solve) on
+        f (owned rows of level 0) and u (level-0 layout, updated in place).  The first pre-sweep of levels 1..L-2 starts from
+        zero, the coarsest level's sweeps continue from the previous cycle's iterate.  Mirrors dist_vcycle of csrc/dist.cu."""
+        L = self.pl.num_levels
+        pre, post = self.num_pre, self.num_post
+        fs, us = [np.asarray(f, dtype=np.float64)] + [None] * (L - 1), [u] + self.e[1:]
+        for l in range(L - 1):
+            if l > 0 and pre > 0:
+                self.owned(l, us[l])[:] = self.owned(l, self.ws[l]) * fs[l]
+                self.sweeps(l, fs[l], us[l], pre - 1)
+            else:
+                self.sweeps(l, fs[l], us[l], pre)
+            self.halo(l, us[l])
+            w = self.new_vec(l)
+            self.owned(l, w)[:] = fs[l] - self.A[l] @ us[l]
+            fs[l + 1] = self.owned(l + 1, self.restrict(l, w))
+        c = L - 1
+        if self.coarse_solve:
+            us[c][:] = np.linalg.solve(self.Ac, fs[c])
+        else:
+            self.sweeps(c, fs[c], us[c], pre + post)
+        for l in range(L - 2, -1, -1):
+            self.halo(l + 1, us[l + 1])
+            self.owned(l, us[l])[:] += self.P[l] @ us[l + 1]
+            self.sweeps(l, fs[l], us[l], post)
+
     def cycle(self, r0):
         """one synchronous additive cycle -- Multadd (symmetrised or plain Jacobi), AFACx or BPX, one sweep per level --
         on the residual r0 (level-0 layout, owned part valid); returns the correction in level-0 layout (owned part
@@ -248,15 +308,7 @@ class DistEmulator:
         last_r = L - 1 if afacx else top - 1        # coarsest residual the cycle reads
         r = [r0] + [None] * (L - 1)
         for l in range(last_r):
-            self.halo(l, r[l])
-            nxt = pl.layouts[l + 1]
-            y = self.R[l] @ r[l]
-            v = self.new_vec(l + 1)
-            if nxt.distributed or not pl.layouts[l].distributed:
-                self.owned(l + 1, v)[:] = y
-            else:
-                v[:] = self.comm.allgatherv(y, pl.all_counts[l + 1])
-            r[l + 1] = v
+            r[l + 1] = self.restrict(l, r[l])
         if self.symmetric and L >= 2:
             self.halo(L - 2, r[L - 2])
         if afacx:
@@ -301,13 +353,22 @@ class DistEmulator:
             self.halo(0, u)
             r = self.new_vec(0)
             self.owned(0, r)[:] = f - self.A[0] @ u
+            self.counts["allreduce"] += 1
             return r, np.sqrt(self.comm.allreduce_sum(float(np.dot(self.owned(0, r), self.owned(0, r)))))
         r, r0n = residual()
         hist = [1.0]
+        for v in self.e:
+            v[:] = 0.0
+        self.per_cycle = []
         for _ in range(max_cycles):
-            c = self.cycle(r)
-            self.owned(0, u)[:] += self.owned(0, c)
+            before = sum(self.counts.values())
+            if self.solver == H.MULT:
+                self.vcycle(f, u)
+            else:
+                c = self.cycle(r)
+                self.owned(0, u)[:] += self.owned(0, c)
             r, rn = residual()
+            self.per_cycle.append(sum(self.counts.values()) - before)
             hist.append(rn / r0n)
             if hist[-1] < tol:
                 break

@@ -537,7 +537,9 @@ def dist_unique_id():
 
 class DistSolver:
     """One rank of the row-partitioned synchronous solve -- Multadd, AFACx or BPX with weighted / L1 Jacobi (DMEM_Add /
-    DMEM_SyncAdd replacement).  `plan` is a
+    DMEM_SyncAdd replacement), or solver=MULT: the multiplicative V-cycle of DMEM_Mult (num_pre / num_post sweeps, coarse_solve =
+    direct solve on the replicated coarsest level; hierarchy built with build_transfers(MULT); no acceleration, DMEM_PowerMult or
+    DMEM_Add_async).  `plan` is a
     partition.RankPlan; `uid` the 128-byte id from dist_unique_id() of rank 0."""
 
     def __init__(self, plan, uid, smooth_weight=1.0, num_pre=1, num_post=1, use_sell=True, use_stream=True,

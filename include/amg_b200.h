@@ -290,6 +290,9 @@ int amgb_l2_arena_bytes(amgb_ctx *ctx, long long *used, long long *capacity);
  * Replaces DMEM_Add / DMEM_SyncAdd (src/DMEM_Add.cpp:20-178, src/DMEM_Mult.cpp:263-450) for the synchronous
  * Multadd and BPX cycles, and AFACx with the SMEM meaning (src/SEQ_AMG.cpp:172-208), with weighted or L1 Jacobi, one sweep per level: hypre's ParCSR halo exchange and DMEM_Comm (src/DMEM_Comm.cpp:81-382) become NCCL
  * send/recv between row-neighbours, the residual norm an ncclAllReduce (src/DMEM_Misc.cpp:398-433).
+ * AMGB_SOLVER_MULT runs the multiplicative V-cycle of DMEM_Mult / DMEM_MultCycle (src/DMEM_Mult.cpp:13-261; SMEM_Sync_Parfor_Vcycle's
+ * meaning) on the same kernels: weighted or L1 Jacobi, num_pre / num_post >= 0 sweeps (one of them positive), plain P and R = P^T
+ * (factor_level0 / factor_restriction are refused), no hybrid JGS; coarse_solve = 1 needs a replicated coarsest level.
  * Call order: amgb_create, amgb_dist_init, amgb_set_options, amgb_set_num_levels, amgb_dist_set_level for
  * EVERY level, then the amgb_set_matrix calls (LOCAL row blocks whose column
  * indices are in the rank's extended numbering [ghost_lo | owned | ghost_hi] on distributed levels, full
@@ -307,18 +310,19 @@ int amgb_dist_set_level(amgb_ctx *ctx, int level, int n_global, int row_start, i
 int amgb_dist_setup(amgb_ctx *ctx);
 int amgb_dist_set_rhs(amgb_ctx *ctx, const double *f_owned);        /* this rank's rows of f */
 int amgb_dist_get_solution(amgb_ctx *ctx, double *u_owned);
-/* x0 = 0; cycles until ||r||/||r0|| < tol (global norms) or max_cycles; identical history on every rank */
+/* x0 = 0; cycles until ||r||/||r0|| < tol (global norms) or max_cycles; identical history on every rank.  With MULT one cycle is
+ * the partitioned V-cycle; its coarsest-level iterate starts from zero in every solve. */
 int amgb_dist_solve_sync(amgb_ctx *ctx, double tol, int max_cycles, double *relres_hist, int *n_cycles,
                          double *solve_seconds);
 /* the same with DMEM's acceleration of the accumulated correction (DMEM_ChebyUpdate, src/DMEM_Misc.cpp:612-666, applied in
  * DMEM_SyncAddCorrect src/DMEM_Add.cpp:706-711): accel 0 none, 1 Chebyshev, 2 second-order Richardson; mu, delta from
- * ChebySetup (src/DMEM_Setup.cpp:1901-1914) */
+ * ChebySetup (src/DMEM_Setup.cpp:1901-1914).  MULT: accel != 0 is AMGB_EINVAL (the acceleration applies to the additive correction) */
 int amgb_dist_solve_sync_accel(amgb_ctx *ctx, double tol, int max_cycles, int accel, double mu, double delta,
                                double *relres_hist, int *n_cycles, double *solve_seconds);
 /* DMEM_PowerMult (src/DMEM_Eig.cpp:10-104): extreme eigenvalues of B*A by `iters` steps of power iteration (second, deflated pass
  * for the minimum) on the partitioned path, B = this context's additive cycle from a zero guess; u0_owned = this rank's rows of
  * the start vector (the reference: RandDouble(0,1) - .5 after srand(rank)), NULL = all ones.  Collective: every rank calls it and
- * receives the same bounds; DMEM's ChebySetup takes alpha = eig_min, beta = eig_max (src/DMEM_Setup.cpp:1901-1914). */
+ * receives the same bounds; DMEM's ChebySetup takes alpha = eig_min, beta = eig_max (src/DMEM_Setup.cpp:1901-1914).  AMGB_EINVAL for MULT. */
 int amgb_dist_eigs_power(amgb_ctx *ctx, int iters, const double *u0_owned, double *eig_min, double *eig_max);
 int amgb_dist_stats(amgb_ctx *ctx, long long *halo_bytes_sent, long long *nccl_ops);
 
@@ -330,7 +334,7 @@ int amgb_dist_stats(amgb_ctx *ctx, long long *halo_bytes_sent, long long *nccl_o
  * (CUDA IPC over NVLink; the handles and layouts travel through NCCL all-gathers inside the first call); nobody waits for
  * a peer.  From the resident f and u; LOCAL stop rule: every group of every rank performs num_cycles corrections.
  * Collective.  corrections[num_levels]: this rank's counts; relres = global ||f - A u|| / ||f - A u_start||; solve_seconds =
- * this rank's kernel time (the job's time is the maximum over the ranks). */
+ * this rank's kernel time (the job's time is the maximum over the ranks).  AMGB_EINVAL for MULT (there is no asynchronous MULT). */
 int amgb_dist_solve_async(amgb_ctx *ctx, int num_cycles, int *corrections, double *relres, double *solve_seconds);
 int amgb_dist_async_groups(amgb_ctx *ctx, int *cta_begin /* num_levels + 1 */, double *group_seconds /* num_levels */);
 /* host-only probe (no CUDA call) of the planning behind amgb_dist_solve_async, for the CPU test suite's multi-rank
